@@ -8,6 +8,8 @@ per-chain results are all-gathered once (the "one all-gather of samples per swee
 
   python bench.py [--gpus N] [--steps K] [--warmup W]              our CUDA path
   python bench.py --impl reference [...]                            the reference's CPU path (oracle port)
+  python bench.py --dump-outputs DIR [...]                          also write the last timed step's outputs as DIR/*.npy
+                                                                    (CUDA path only; refused with --impl reference)
 
 Prints ONE JSON line (rank 0).  `value` is timed with the inputs resident in HBM; `e2e` goes through
 the C-ABI host-buffer call (pinned H2D of x/g/theta and D2H of loglik/info inside the timed region).
@@ -46,7 +48,14 @@ def parse():
     ap.add_argument('--no-configs', action='store_true', help='skip the sub-records of the other BASELINE configs / SDS sweeps')
     ap.add_argument('--only-configs', default=None, help='comma list of sub-record names to run (e.g. C3_loglik,C3_sds)')
     ap.add_argument('--gemm-cfg', type=int, default=None, help='experiment: DMMA tile kernel variant (0: 8 warps, 1: 16 warps)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned (loglik, info) as DIR/<name>.npy, for comparing two builds')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
+    return args
 
 
 def workload_config(n, B, world):
@@ -622,6 +631,14 @@ def run_b200(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = world * B * args.steps / (ms * 1e-3)
+    if args.dump_outputs:
+        out = {'loglik': ll, 'info': info}
+        if world > 1:
+            info_all = torch.empty((world * B,), dtype=torch.int32, device='cuda')
+            dist.all_gather_into_tensor(info_all, info)
+            out = {'loglik': gathered, 'info': info_all}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in out.items()})
 
     # ---- end-to-end through the host-buffer C-ABI call (pinned H2D + D2H every step)
     e2e = None
@@ -762,6 +779,24 @@ def run_b200(args):
     emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_LIMIT_BYTES = 60 * 10 ** 6          # data bytes: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write ``arrays`` (name -> 1-D array over chains) as float64 ``out_dir/<name>.npy``.  Above DUMP_LIMIT_BYTES in all, every
+    array keeps the same fixed, seeded sample of chains, whose indices are written beside them as ``sample_index.npy``."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    if 8 * n * len(arrays) > DUMP_LIMIT_BYTES:
+        keep = DUMP_LIMIT_BYTES // (8 * (len(arrays) + 1))
+        idx = np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+        arrays = dict({k: a[idx] for k, a in arrays.items()}, sample_index=idx.astype(np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
 
 
 _REAL_STDOUT = None

@@ -1,8 +1,10 @@
 """Generate ``tests/golden/*.npz`` by running the reference's own ``kcMCMC/sliceSample.py``.
 
-TEST INFRASTRUCTURE (see ``oracle/__init__.py``).  Run in the build container only (needs
-``/root/reference``):  ``python -m oracle.make_golden``.  The fixtures travel to the GPU box;
-this script and the literal reference do not need to.
+TEST INFRASTRUCTURE (see ``oracle/__init__.py``).  Needs a checkout of the original project:
+``GPMC_REFERENCE_ROOT=<checkout> python -m oracle.make_golden``.  The tests read only the
+committed fixtures; neither this script nor the original project is needed to run them.
+``python -m oracle.make_golden literal-cases`` writes ``literal_cases.npz`` alone and runs
+without a checkout; its ``source`` entry then says that the restatement made it.
 
 Each ``sds_N*.npz`` holds the inputs of one ``surrogate_slice_sampling`` call, the explicit
 randomness (tape), and what the UNMODIFIED reference returned for it, plus literal
@@ -19,6 +21,16 @@ from . import kcgp_shim, reference_loader as rl, sds_oracle as so
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN = os.path.join(os.path.dirname(HERE), 'tests', 'golden')
+# OpenBLAS threads the fixtures are made with.  OpenBLAS splits a product by its thread count, and f' of the
+# ill-conditioned SDS fixtures follows that summation order (up to 5e-4 absolute at N = 200 and 512 between 1 and 8
+# threads), so the tests replay the restatement with the same count.
+BLAS_THREADS = 8
+
+
+def pinned_blas():
+    """Context in which OpenBLAS runs BLAS_THREADS threads, whatever the host's cores (needs threadpoolctl)."""
+    import threadpoolctl
+    return threadpoolctl.threadpool_limits(limits=BLAS_THREADS)
 
 
 def _series(n, seed=124, hyp=(5.0, 4.0, 2.5)):
@@ -196,9 +208,62 @@ def ess_case(n, seed, hyp, f_scale):
     return dict(x=x, y=y, hyp=hyp, f=f, z=z, nu=nu, u=tape.u, theta=tape.theta, ref_prop_f=pf, ref_trips=trips, cond_K=cond_K)
 
 
+# the cases of tests/test_oracle_vs_reference.py, stored in literal_cases.npz
+LITERAL_SDS_CASES = [(24, 0, 1), (24, 777, 2), (96, 499, 3), (96, 500, 4)]
+LITERAL_ESS_CASES = [(40, 5), (120, 6)]
+LOG_GAMMA_HYP = [0.7, 3.0, 1.9]
+
+
+def literal_cases():
+    """Inputs, tapes and outputs of the cases of ``tests/test_oracle_vs_reference.py``.  The outputs are computed by the
+    restatement; where the reference is present, its own functions run on the same tapes and must return the same bits.
+    ``source`` records which of the two produced the stored values."""
+    lit = rl.available()
+    mod = rl.load_literal() if lit else None
+    out = {'source': 'restatement, asserted bit-identical to kcMCMC/sliceSample.py' if lit else 'oracle/sds_oracle.py restatement'}
+    for n, it, seed in LITERAL_SDS_CASES:
+        x, y = _series(n)
+        f, hyp, scale = np.zeros(n), np.array([1., 10., 1.2]), np.array([10., 10., 5.])
+        tape = rl.Tape.from_seed(seed, n)
+        tr = so.SweepTrace()
+        of, oh = so.surrogate_slice_sampling(f, x, y, hyp, scale, it, tape, trace=tr)
+        if lit:
+            pf, ph, trips = rl.run_literal_with_tape(f, x, y, hyp, scale, it, tape)
+            assert trips == tr.n_trips and np.array_equal(ph, oh) and np.array_equal(pf, of)
+        k = 'sds_N%d_it%d_s%d_' % (n, it, seed)
+        out.update({k + 'x': x, k + 'y': y, k + 'f': f, k + 'hyp': hyp, k + 'scale': scale, k + 'z': tape.z, k + 'v': tape.v,
+                    k + 'u0': tape.u0, k + 'U': tape.U[:tr.n_trips + 2], k + 'prop_f': of, k + 'prop_hyp': oh,
+                    k + 'trips': tr.n_trips})
+    for n, seed in LITERAL_ESS_CASES:
+        x, y = _series(n)
+        rs = np.random.RandomState(seed)
+        hyp = np.array([4., 5., 1.8])
+        f = 0.7 * (y - y.mean())
+        tape = rl.EssTape(so.ess_nu_from_z(x, hyp, rs.standard_normal(n)), rs.random_sample(), rs.random_sample(64))
+        of, trips = so.elliptical_slice(f, x, y, hyp, tape)
+        if lit:
+            pf, ltrips = rl.run_literal_ess_with_tape(f, x, y, hyp, tape)
+            assert ltrips == trips and np.array_equal(pf, of)
+        k = 'ess_N%d_s%d_' % (n, seed)
+        out.update({k + 'x': x, k + 'y': y, k + 'f': f, k + 'hyp': hyp, k + 'nu': tape.nu, k + 'u': tape.u,
+                    k + 'theta': tape.theta, k + 'prop_f': of, k + 'trips': trips})
+    hyp = np.array(LOG_GAMMA_HYP)
+    a, b = so.log_gamma(hyp, so.PRIOR_K3, so.PRIOR_THETA3, True)
+    if lit:
+        c, d = mod.log_gamma(hyp, so.PRIOR_K3, so.PRIOR_THETA3, True)
+        assert np.array_equal(a, c) and np.array_equal(b, d)
+    out.update(log_gamma_hyp=hyp, log_gamma=a, log_gamma_grad=b)
+    return out
+
+
+def write_literal_cases():
+    np.savez_compressed(os.path.join(GOLDEN, 'literal_cases.npz'), **literal_cases())
+    print('literal_cases written')
+
+
 def main():
     if not rl.available():
-        sys.exit('reference tree not present: fixtures can only be generated in the build container')
+        sys.exit('set GPMC_REFERENCE_ROOT to a checkout of the original project: fixtures are made by running its sliceSample.py')
     os.makedirs(GOLDEN, exist_ok=True)
     cases = [(8, 0, 11, [1., 10., 1.2], 'zero'), (8, 700, 12, [0.35, 2.0, 0.2], 'mid'),
              (64, 0, 21, [1., 10., 1.2], 'zero'), (64, 650, 22, [0.35, 2.0, 0.2], 'mid'), (64, 499, 23, [3., 6., 2.], 'mid'),
@@ -231,7 +296,9 @@ def main():
     ch = chain_case()
     np.savez_compressed(os.path.join(GOLDEN, 'chain_N64.npz'), **ch)
     print('chain_N64: trips mean %.2f max %d; final hyp %s' % (ch['ref_trips'].mean(), ch['ref_trips'].max(), ch['ref_histHyp'][:, -1]))
+    write_literal_cases()
 
 
 if __name__ == '__main__':
-    main()
+    with pinned_blas():
+        write_literal_cases() if sys.argv[1:] == ['literal-cases'] else main()

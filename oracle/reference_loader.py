@@ -1,10 +1,12 @@
 """Load the reference's own ``kcMCMC/sliceSample.py`` UNMODIFIED as the literal oracle.
 
-TEST INFRASTRUCTURE (see ``oracle/__init__.py``).  Works only where
-``/root/reference`` exists (the build container); the GPU box has no copy, so
-nothing here may be reached from ``-m gpu`` tests, ``smoke()`` or ``bench.py``.
-It is used by ``oracle/make_golden.py`` (fixture generation) and by the CPU tests
-that pin :mod:`oracle.sds_oracle` to the literal reference.
+TEST INFRASTRUCTURE (see ``oracle/__init__.py``).  The original project is not
+part of this repository: the loader works only where ``GPMC_REFERENCE_ROOT``
+names a checkout of t-kychen/GaussianProcess-MCMC, so the literal module may not
+be reached from ``-m gpu`` tests, ``smoke()`` or ``bench.py``.  The ``Tape``
+classes below need no checkout.  The loader is used by ``oracle/make_golden.py``
+(fixture generation) and by the CPU tests that pin :mod:`oracle.sds_oracle` to the
+literal reference.
 
 ``kcMCMC/__init__.py:1`` is a Python-2 implicit relative import, so the package
 cannot be imported; the module file is loaded by path instead with the ``kcGP``
@@ -17,18 +19,18 @@ import numpy as np
 
 from . import kcgp_shim
 
-REFERENCE_ROOT = os.environ.get('GPMC_REFERENCE_ROOT', '/root/reference')
+REFERENCE_ROOT = os.environ.get('GPMC_REFERENCE_ROOT', '')
 _SLICE_SAMPLE = os.path.join(REFERENCE_ROOT, 'kcMCMC', 'sliceSample.py')
 
 
 def available():
-    return os.path.isfile(_SLICE_SAMPLE)
+    return bool(REFERENCE_ROOT) and os.path.isfile(_SLICE_SAMPLE)
 
 
 def load_literal(fresh=False):
     """Return the reference ``sliceSample`` module object (executed from its own file)."""
     if not available():
-        raise RuntimeError('reference tree not present at %s' % REFERENCE_ROOT)
+        raise RuntimeError('GPMC_REFERENCE_ROOT does not name a checkout of the original project (%r)' % REFERENCE_ROOT)
     kcgp_shim.install()
     name = 'gpmc_reference_sliceSample' + ('_%d' % id(object()) if fresh else '')
     spec = importlib.util.spec_from_file_location(name, _SLICE_SAMPLE)

@@ -7,6 +7,7 @@ import pytest
 
 from conftest import golden_files, load_rows, GOLDEN
 from oracle import sds_oracle as so
+from oracle.make_golden import pinned_blas
 from oracle.reference_loader import Tape
 
 SDS = golden_files('sds_N*.npz')
@@ -23,9 +24,11 @@ def test_transition_matches_reference_output(path):
     z = np.load(path)
     tape = Tape(z['z'], z['v'], z['u0'], z['U'])
     tr = so.SweepTrace()
-    pf, ph = so.surrogate_slice_sampling(z['f'], z['x'], z['y'], z['hyp'], z['scale'], int(z['it']), tape, trace=tr)
-    # same container, same BLAS: the restatement reproduced the literal run bit for bit when the
-    # fixture was made; across machines allow BLAS-level rounding.
+    # the BLAS summation order of the fixture's run (OpenBLAS sets it by its thread count, whatever the host's cores)
+    with pinned_blas():
+        pf, ph = so.surrogate_slice_sampling(z['f'], z['x'], z['y'], z['hyp'], z['scale'], int(z['it']), tape, trace=tr)
+    # same BLAS order: the restatement reproduced the literal run bit for bit when the
+    # fixture was made; across CPU types allow BLAS-level rounding.
     assert tr.n_trips == int(z['ref_trips'])
     np.testing.assert_allclose(ph, z['ref_prop_hyp'], rtol=1e-13, atol=0)
     np.testing.assert_allclose(pf, z['ref_prop_f'], rtol=1e-6, atol=1e-6)

@@ -1,29 +1,42 @@
-"""Pin the restatement to the reference file itself (build container only: needs /root/reference)."""
+"""Pin the restatement to the reference file itself.  Each case's inputs, tape and outputs are stored in
+``tests/golden/literal_cases.npz`` (``oracle/make_golden.py``), and the restatement must reproduce them bit for bit
+(N <= 120: OpenBLAS does not split these products, so its thread count does not enter).  Where ``GPMC_REFERENCE_ROOT``
+names a checkout of the original project, its own ``sliceSample.py`` runs on the same tapes as well and must return the
+same bits."""
+import os
+
 import numpy as np
 import pytest
 
+from conftest import GOLDEN
 from oracle import reference_loader as rl, sds_oracle as so, make_golden as mg
 
-pytestmark = pytest.mark.skipif(not rl.available(), reason='reference tree not present on this machine')
+CASES = np.load(os.path.join(GOLDEN, 'literal_cases.npz'))
 
 
-@pytest.mark.parametrize('n,it,seed', [(24, 0, 1), (24, 777, 2), (96, 499, 3), (96, 500, 4)])
+def _case(prefix):
+    return {k[len(prefix):]: CASES[k] for k in CASES.files if k.startswith(prefix)}
+
+
+@pytest.mark.parametrize('n,it,seed', mg.LITERAL_SDS_CASES)
 def test_restatement_is_bit_identical_to_literal(n, it, seed):
-    x, y = mg._series(n)
-    f = np.zeros(n); hyp = np.array([1., 10., 1.2]); scale = np.array([10., 10., 5.])
-    tape = rl.Tape.from_seed(seed, n)
-    pf, ph, trips = rl.run_literal_with_tape(f, x, y, hyp, scale, it, tape)
+    c = _case('sds_N%d_it%d_s%d_' % (n, it, seed))
+    tape = rl.Tape(c['z'], c['v'], c['u0'], c['U'])
     tr = so.SweepTrace()
-    of, oh = so.surrogate_slice_sampling(f, x, y, hyp, scale, it, tape, trace=tr)
-    assert trips == tr.n_trips and np.array_equal(ph, oh) and np.array_equal(pf, of)
+    of, oh = so.surrogate_slice_sampling(c['f'], c['x'], c['y'], c['hyp'], c['scale'], it, tape, trace=tr)
+    assert tr.n_trips == int(c['trips']) and np.array_equal(oh, c['prop_hyp']) and np.array_equal(of, c['prop_f'])
+    if rl.available():
+        pf, ph, trips = rl.run_literal_with_tape(c['f'], c['x'], c['y'], c['hyp'], c['scale'], it, tape)
+        assert trips == tr.n_trips and np.array_equal(ph, oh) and np.array_equal(pf, of)
 
 
 def test_literal_module_functions():
-    mod = rl.load_literal()
-    hyp = np.array([0.7, 3.0, 1.9])
-    a, b = mod.log_gamma(hyp, so.PRIOR_K3, so.PRIOR_THETA3, True)
+    hyp = CASES['log_gamma_hyp']
     c, d = so.log_gamma(hyp, so.PRIOR_K3, so.PRIOR_THETA3, True)
-    assert np.array_equal(a, c) and np.array_equal(b, d)
+    assert np.array_equal(c, CASES['log_gamma']) and np.array_equal(d, CASES['log_gamma_grad'])
+    if rl.available():
+        a, b = rl.load_literal().log_gamma(hyp, so.PRIOR_K3, so.PRIOR_THETA3, True)
+        assert np.array_equal(a, c) and np.array_equal(b, d)
 
 
 def test_multivariate_normal_draw_is_f_plus_sd_z():
@@ -37,13 +50,12 @@ def test_multivariate_normal_draw_is_f_plus_sd_z():
     np.testing.assert_allclose(g, f + 1.2 * z, rtol=0, atol=1e-15)
 
 
-@pytest.mark.parametrize('n,seed', [(40, 5), (120, 6)])
+@pytest.mark.parametrize('n,seed', mg.LITERAL_ESS_CASES)
 def test_elliptical_slice_restatement_is_bit_identical_to_literal(n, seed):
-    x, y = mg._series(n)
-    rs = np.random.RandomState(seed)
-    hyp = np.array([4., 5., 1.8])
-    f = 0.7 * (y - y.mean())
-    tape = rl.EssTape(so.ess_nu_from_z(x, hyp, rs.standard_normal(n)), rs.random_sample(), rs.random_sample(64))
-    pf, trips = rl.run_literal_ess_with_tape(f, x, y, hyp, tape)
-    of, otrips = so.elliptical_slice(f, x, y, hyp, tape)
-    assert trips == otrips and np.array_equal(pf, of)
+    c = _case('ess_N%d_s%d_' % (n, seed))
+    tape = rl.EssTape(c['nu'], c['u'], c['theta'])
+    of, otrips = so.elliptical_slice(c['f'], c['x'], c['y'], c['hyp'], tape)
+    assert otrips == int(c['trips']) and np.array_equal(of, c['prop_f'])
+    if rl.available():
+        pf, trips = rl.run_literal_ess_with_tape(c['f'], c['x'], c['y'], c['hyp'], tape)
+        assert trips == otrips and np.array_equal(pf, of)
