@@ -83,19 +83,30 @@ struct LoglikLayout {
     int ld;
     size_t mat_elems;        // per item
     size_t fixed_bytes;      // per-call scratch independent of the wave
-    size_t per_item_bytes;   // matrix + W
+    size_t per_item_bytes;   // matrix + W + envelope
 };
 static LoglikLayout loglik_layout(int N, int B)
 {
     LoglikLayout l;
     l.ld = ld_for(N);
     l.mat_elems = (size_t)(N + 1) * l.ld;            // + the border row that carries g through the factorisation
-    l.per_item_bytes = l.mat_elems * sizeof(double) + (size_t)NB * NB * sizeof(double);
+    l.per_item_bytes = l.mat_elems * sizeof(double) + (size_t)NB * NB * sizeof(double) + (size_t)env_blocks(N) * sizeof(int);
     l.fixed_bytes = align_up((size_t)B * sizeof(double), 256)      // jitter
                     + align_up((size_t)B * sizeof(int), 256)       // map
                     + 256                                          // count
                     + align_up((size_t)32 * l.ld * sizeof(double), 256);   // z scratch of the small-batch solve
     return l;
+}
+
+// Envelope skips (gpmc_set_tuning(14, .)): -1 until set, then the GPMC_ENVELOPE environment variable decides once
+static int g_envelope = -1;
+bool envelope_enabled()
+{
+    if (g_envelope < 0) {
+        const char *e = getenv("GPMC_ENVELOPE");
+        g_envelope = (e && e[0] == '0') ? 0 : 1;
+    }
+    return g_envelope != 0;
 }
 
 // Assemble-and-factor one wave with kcGP.tools.jitchol semantics (pyGPs 1.3.4): one plain attempt for every item, then --
@@ -104,11 +115,11 @@ static LoglikLayout loglik_layout(int N, int B)
 // rows; `diag_value` is the (constant) diagonal of an item's matrix from its hyper-parameter row.
 int factor_wave(const std::function<int(BatchView, int, const double *)> &fill, const std::function<double(const double *)> &diag_value,
                 BatchView A, int N, int nb, const double *hyp_w, int P, int *info_w, double *W, double *jit_dev, int *map_dev,
-                int jitter_policy, int border_rows, cudaStream_t s, int fuse)
+                int jitter_policy, int border_rows, cudaStream_t s, int fuse, Envelope env)
 {
     int rc = fill(A, nb, nullptr);
     if (rc) return rc;
-    if ((rc = potrf_sequence(A, N, nb, info_w, W, NB * NB, 0, 0, s, border_rows, fuse))) return rc;
+    if ((rc = potrf_sequence(A, N, nb, info_w, W, NB * NB, 0, 0, s, border_rows, fuse, env))) return rc;
     if (jitter_policy != GPMC_JITTER_PYGPS) return 0;
     std::vector<int> info(nb);
     GPMC_CUDA_CHECK(cudaMemcpyAsync(info.data(), info_w, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -135,7 +146,7 @@ int factor_wave(const std::function<int(BatchView, int, const double *)> &fill, 
         GPMC_CUDA_CHECK(cudaMemcpyAsync(info_w, info.data(), nb * sizeof(int), cudaMemcpyHostToDevice, s));
         BatchView Am{A.base, A.stride, A.ld, map_dev, nullptr};
         if ((rc = fill(Am, nf, jit_dev))) return rc;
-        if ((rc = potrf_sequence(Am, N, nf, info_w, W, NB * NB, 0, 0, s, border_rows, fuse))) return rc;
+        if ((rc = potrf_sequence(Am, N, nf, info_w, W, NB * NB, 0, 0, s, border_rows, fuse, env))) return rc;
         GPMC_CUDA_CHECK(cudaMemcpyAsync(info.data(), info_w, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
         GPMC_CUDA_CHECK(cudaStreamSynchronize(s));
         std::vector<int> still;
@@ -301,6 +312,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
     const int wave = (int)std::min<size_t>(wave_cap, (size_t)B);
     double *mats = (double *)wp;
     double *W = (double *)(wp + (size_t)wave * l.mat_elems * sizeof(double));
+    const Envelope env_ws{(int *)(W + (size_t)wave * NB * NB), env_blocks(N), N};
 
     { int rc0 = fill_int(info_dev, 0, B, s); if (rc0) return rc0; }
     for (int s0 = 0; s0 < B; s0 += wave) {
@@ -309,14 +321,17 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
         const double *g_w = g_dev + (size_t)s0 * N;
         int *info_w = info_dev + s0;
         BatchView A{mats, (long long)l.mat_elems, l.ld, nullptr, nullptr};
+        const int fuse = potrf_fuse_auto(N, nb, 1);
+        // The fused panel launches (many small matrices) ignore the envelope, and the few short update contractions of
+        // those matrices save less than recording and reading it costs (N=512 x 4096, ARD: 1 % slower): dense there.
+        const Envelope env = (envelope_enabled() && !fuse) ? env_ws : Envelope{};
         auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
-            int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s);
+            int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env);
             if (rc) return rc;
             return border_set(V, N, g_w, N, nitems, s);
         };
         auto diag = [&](const double *h) { return host_diag_value(h, n_ell); };
-        const int fuse = potrf_fuse_auto(N, nb, 1);
-        int rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, W, jit_dev, map_dev, jitter_policy, 1, s, fuse);
+        int rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, W, jit_dev, map_dev, jitter_policy, 1, s, fuse, env);
         if (rc) return rc;
         // z = L^-1 g sits in the border row except for the last column block: finish it, then quad form + log det
         rc = border_finish(A, N, loglik_dev + s0, info_w, nb, s, fuse);
@@ -422,6 +437,7 @@ int gpmc_set_tuning(int key, int value)
     if (key == 10) { set_lookahead_split(value); return 0; }
     if (key == 11) { set_inverse_window(value); return 0; }
     if (key == 13) { set_sds_pin_schedule(value); return 0; }
+    if (key == 14) { g_envelope = value != 0; return 0; }
     return GPMC_EINVAL;
 }
 

@@ -76,11 +76,36 @@ struct BatchView {
 __device__ __forceinline__ int batch_item(const BatchView &v, int b) { return v.map ? v.map[b] : b; }
 
 // ---------------------------------------------------------------------------------------------
+// Envelope of an assembled matrix.  blk[item * ld + r] is the smallest column that holds a nonzero in rows
+// ENV_ROWS*r .. ENV_ROWS*r+ENV_ROWS-1 of the lower triangle, as the assembly wrote it.  Cholesky keeps the envelope
+// (L_ik = 0 exactly for every k left of row i's first nonzero), so a product over k below it adds only zeros and can be
+// skipped without changing a bit.  Rows >= n (right-hand sides carried below the matrix) are not covered and count as
+// dense; blk == nullptr means dense everywhere.
+constexpr int ENV_ROWS = 64;
+struct Envelope {
+    int *blk = nullptr;
+    int ld = 0;            // ints between items
+    int n = 0;             // order of the matrix
+};
+__host__ __device__ inline int env_blocks(int n) { return (n + ENV_ROWS - 1) / ENV_ROWS; }
+
+// first column that may hold a nonzero in rows r0 .. r1-1 of item m (0 when any of them is not covered)
+__device__ __forceinline__ int env_first_col(const Envelope &e, int m, int r0, int r1)
+{
+    if (!e.blk || r1 > e.n || r1 <= r0) return 0;
+    const int *p = e.blk + (size_t)m * e.ld;
+    int k = 0x7fffffff;
+    for (int r = r0 / ENV_ROWS; r <= (r1 - 1) / ENV_ROWS; ++r) k = min(k, p[r]);
+    return k;
+}
+
+// ---------------------------------------------------------------------------------------------
 // launchers (definitions in the .cu files)
 
 // cov_assemble.cu
+// env.blk != nullptr: also writes the envelope of every assembled item (the items A selects)
 int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P, int n_ell, int flags,
-                        const double *jitter, BatchView A, int B, cudaStream_t s);
+                        const double *jitter, BatchView A, int B, cudaStream_t s, Envelope env = {});
 
 // gemm_dmma.cu :  C[i][j] (op)= sum_k A[i][k] * B[j][k]   ("NT": both operands K-contiguous, row-major)
 struct Operand {
@@ -112,6 +137,8 @@ struct GemmArgs {
                            // ROW below the matrix; it receives the same update, C[border_row, cols] -= A[border_row, k] B[cols, k]^T
     const double *svec;    // EPI_R: per-item diagonal of S, [N]
     long long stride_s;
+    Envelope env;          // EPI_SUB Cholesky updates with A = B = C: envelope of the matrix (cfg 4 starts each tile's
+                           // contraction at it; the other variants ignore it)
 };
 int launch_gemm(const GemmArgs &a, int B, int kclass, cudaStream_t s);
 void set_gemm_config(int cfg);
@@ -147,8 +174,9 @@ int launch_trsm_panel(BatchView A, int n, int j0, const double *W, long long str
 // trsm_panel8.cu : the same solve with 8-column sub-blocks, shuffle-based fragment conversion, 2 CTAs per SM (default)
 //   row_start >= 0: solve only rows row_start .. n-1 (border rows of the last block column); n_mat >= 0: order of the matrix
 //   (rows / columns of the diagonal block at or beyond it read as identity)
+//   env: envelope of A -- a 64-row block whose rows have no nonzero left of j0 + NB is zero and stays so (skipped)
 int launch_trsm_panel8(BatchView A, int n, int j0, const double *W, long long strideW, int B, cudaStream_t s,
-                       int row_start = -1, int n_mat = -1);
+                       int row_start = -1, int n_mat = -1, Envelope env = {});
 // trmm_panel8.cu : in place  A[0:rows, c0:c0+width] = -(A[0:rows, c0:c0+128] W^T)  for a lower triangular 128x128 W
 //   (the second product of the triangular inverse, inverse_sequence)
 int launch_trmm_panel8(BatchView A, int rows, int c0, int width, const double *W, long long strideW, int B, cudaStream_t s);

@@ -30,7 +30,7 @@ constexpr int ASM_TPC = 1;      // tiles per CTA (4 was measured: N=4096 x 256 4
 template <int DT, bool PRED>
 __global__ void __launch_bounds__(256)
 cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *__restrict__ hyp, int P, int n_ell,
-                    int flags, const double *__restrict__ jitter, BatchView A)
+                    int flags, const double *__restrict__ jitter, BatchView A, Envelope env)
 {
     const int D = DT > 0 ? DT : Drt;
     const int b = blockIdx.y;
@@ -103,6 +103,8 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
     __syncthreads();
 
     const int gc = c0 + cl;
+    // envelope: this thread's first column holding a nonzero in the tile's lower-triangle rows (NaN counts as nonzero)
+    bool nz0 = false, nz1 = false;
     const bool mirror = (tm != tn) && !(flags & GPMC_ASM_LOWER_ONLY);
 
     const bool interior = (r0 + AT <= N) && (c0 + AT <= N) && (tm != tn);
@@ -128,6 +130,8 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
             if (pred) { k0 = k0 / sn2; k1 = k1 / sn2; }
             if (mirror) *reinterpret_cast<double2 *>(&s_tile[rl][cl]) = make_double2(k0, k1);
             *reinterpret_cast<double2 *>(dst + (size_t)rr * A.ld) = make_double2(k0, k1);
+            nz0 |= (k0 != 0.0);
+            nz1 |= (k1 != 0.0);
         }
     } else {
 #pragma unroll
@@ -152,8 +156,19 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
             double *dst = Ab + (size_t)gr * A.ld + gc;
             if (gc + 1 < N)      *reinterpret_cast<double2 *>(dst) = make_double2(k0, k1);
             else if (gc < N)     dst[0] = k0;
+            nz0 |= (k0 != 0.0 && gc < N && gc <= gr);
+            nz1 |= (k1 != 0.0 && gc + 1 < N && gc + 1 <= gr);
         }
     }
+    }
+    if (env.blk) {
+        __shared__ int s_env;
+        if (tid == 0) s_env = 0x7fffffff;
+        __syncthreads();
+        const int first = __reduce_min_sync(0xffffffffu, nz0 ? gc : (nz1 ? gc + 1 : 0x7fffffff));
+        if (lane == 0 && first != 0x7fffffff) atomicMin(&s_env, first);
+        __syncthreads();
+        if (tid == 0 && s_env != 0x7fffffff) atomicMin(env.blk + (size_t)m * env.ld + tm, s_env);
     }
     if (!mirror) continue;
     __syncthreads();
@@ -174,18 +189,30 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
     }
 }
 
+// every envelope entry of the items A selects starts as "no nonzero"; the assembly lowers it
+__global__ void env_init_kernel(BatchView A, Envelope env)
+{
+    const int b = blockIdx.x;
+    if (A.count && b >= *A.count) return;
+    const int m = batch_item(A, b);
+    for (int r = threadIdx.x; r < env_blocks(env.n); r += blockDim.x) env.blk[(size_t)m * env.ld + r] = 0x7fffffff;
+}
+
 int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P, int n_ell, int flags,
-                        const double *jitter, BatchView A, int B, cudaStream_t s)
+                        const double *jitter, BatchView A, int B, cudaStream_t s, Envelope env)
 {
     if (D > MAX_ELL || n_ell > MAX_ELL) { set_error("D=%d exceeds MAX_ELL=%d", D, MAX_ELL); return GPMC_EINVAL; }
     if (B <= 0) return 0;
+    static_assert(AT == ENV_ROWS, "one tile row block is one envelope block");
+    if (env.blk && (env.n != N || env.ld < env_blocks(N))) { set_error("cov_assemble: envelope n=%d ld=%d for N=%d", env.n, env.ld, N); return GPMC_EINVAL; }
     const int nt = (N + AT - 1) / AT;
     dim3 grid((nt * (nt + 1) / 2 + ASM_TPC - 1) / ASM_TPC, B);
     prof_begin(KC_ASSEMBLE, s);
+    if (env.blk) env_init_kernel<<<B, 128, 0, s>>>(A, env);
 #define GPMC_ASM_LAUNCH(DT_)                                                                                                     \
     do {                                                                                                                          \
-        if (flags & GPMC_ASM_PRED) cov_assemble_kernel<DT_, true><<<grid, 256, 0, s>>>(x, N, D, hyp, P, n_ell, flags, jitter, A);  \
-        else cov_assemble_kernel<DT_, false><<<grid, 256, 0, s>>>(x, N, D, hyp, P, n_ell, flags, jitter, A);                       \
+        if (flags & GPMC_ASM_PRED) cov_assemble_kernel<DT_, true><<<grid, 256, 0, s>>>(x, N, D, hyp, P, n_ell, flags, jitter, A, env);  \
+        else cov_assemble_kernel<DT_, false><<<grid, 256, 0, s>>>(x, N, D, hyp, P, n_ell, flags, jitter, A, env);                       \
     } while (0)
     switch (D) {
         case 1: GPMC_ASM_LAUNCH(1); break;

@@ -86,6 +86,15 @@ gemm_dmma_tma_kernel(GemmArgs p, const __grid_constant__ CUtensorMap tmA, const 
     const int cols_valid = min(TBN, p.cols - tn * TBN);
     int koff = 0;
     if (p.k_follow_row) koff = max(0, (p.ar0 + tm * TBM) - p.k0) & ~(TBK - 1);
+    if (p.env.blk) {
+        // L[r, k] = 0 for k left of row r's envelope: chunks below the later envelope of the A-tile rows and the B-tile
+        // rows add exact zeros (+0 accumulators stay +0, the rest is summed in the same order) -- start after them.  The
+        // border-row warp of a diagonal tile contracts against the B tile, so it may start there too.
+        const int ra = p.ar0 + tm * TBM, rb = p.br0 + tn * TBN;
+        const int kenv = max(env_first_col(p.env, m, ra, ra + rows_valid), env_first_col(p.env, m, rb, rb + cols_valid));
+        koff = max(koff, (kenv & ~(TBK - 1)) - p.k0);
+        if (koff >= p.klen) return;                   // every product of the tile is zero: C stays as it is
+    }
     const int klen = p.klen - koff;
     const int nk = klen > 0 ? (klen + TBK - 1) / TBK : 0;
     const int tid = threadIdx.x;

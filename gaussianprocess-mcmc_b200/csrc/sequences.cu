@@ -264,7 +264,7 @@ int potrf_fuse_auto(int n, int B, int border_rows)
 }
 
 int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long strideW, long long w_step,
-                   int zero_upper_flag, cudaStream_t s, int border_rows, int fuse)
+                   int zero_upper_flag, cudaStream_t s, int border_rows, int fuse, Envelope env)
 {
     if (fuse && (!lite_panels() || (g_potf2_mode != 0 && g_potf2_mode != 3))) { set_error("potrf_sequence: fused panels need the default panel kernels"); return GPMC_EINVAL; }
     if (border_rows < 0) { set_error("potrf_sequence: border_rows < 0"); return GPMC_EINVAL; }
@@ -297,6 +297,7 @@ int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long st
         g.ar0 = j0; g.br0 = j0; g.k0 = k_begin; g.bk0 = k_begin; g.klen = k_end - k_begin;
         g.epi = EPI_SUB;
         g.skip_upper = 1;                               // potf2 reads the lower triangle of the diagonal block only
+        g.env = env;
         return launch_gemm(g, B, KC_GEMM, st);
     };
 
@@ -326,6 +327,7 @@ int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long st
                 g.lower_only = 1;
                 g.epi = EPI_SUB;
                 g.skip_upper = 1;
+                g.env = env;
                 int rc = launch_gemm(g, B, KC_GEMM, sG);
                 if (rc) return rc;
                 if ((rc = extra_rows_update(w1, n - w1, w0 - wlen, wlen, sG))) return rc;
@@ -372,7 +374,7 @@ int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long st
                                          : launch_potf2_reg(A, n, j0, Wj, strideW, info, zero_upper_flag, B, sP)));
             if (rc) return rc;
             if (j0 + NB < n && (rc = (g_trsm_mode == 1 ? launch_trsm_panel(A, nr, j0, Wj, strideW, B, sP)
-                                                        : launch_trsm_panel8(A, nr, j0, Wj, strideW, B, sP)))) return rc;
+                                                        : launch_trsm_panel8(A, nr, j0, Wj, strideW, B, sP, -1, -1, env)))) return rc;
             // several border rows: the last block column is solved for them here too (a single border row is finished by
             // border_finish together with the quadratic form)
             if (j0 + NB >= n && xrows > 0 && (rc = launch_trsm_panel8(A, nr, j0, Wj, strideW, B, sP, n, n))) return rc;
@@ -390,6 +392,7 @@ int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long st
             g.lower_only = split ? 0 : 1;               // split: the next window's columns first (rectangular, the tiles
             g.epi = EPI_SUB;                            // above the diagonal exit at once), the rest at the top of the loop
             g.skip_upper = 1;
+            g.env = env;
             int rc = launch_gemm(g, B, KC_GEMM, sG);
             if (rc) return rc;
             if (!split && (rc = extra_rows_update(w1, n - w1, w0, w1 - w0, sG))) return rc;

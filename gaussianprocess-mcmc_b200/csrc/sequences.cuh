@@ -17,15 +17,20 @@ namespace gpmc {
 // fuse != 0: panel factor and panel solve of every block column in ONE launch (launch_panel_fused); the border rows are
 // then COMPLETE on return, the last block column included (pass the same flag to border_finish).  Callers decide once
 // per batch with potrf_fuse_auto() and use the same flag for every call on those buffers (retries of subsets included).
+// env: envelope of A as launch_cov_assemble wrote it -- the update GEMMs and the panel solves skip the work it shows to
+// be zero (bit-identical results); the fused panel launches ignore it.
 int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long strideW, long long w_step,
-                   int zero_upper, cudaStream_t s, int border_rows = 0, int fuse = 0);
+                   int zero_upper, cudaStream_t s, int border_rows = 0, int fuse = 0, Envelope env = {});
 int potrf_fuse_auto(int n, int B, int border_rows);
 
 // One wave of assemble-and-factor with the pyGPs jitter ladder (capi.cu); shared by the log-lik unit, the predictive
 // path and the elliptical slice sampler's Cholesky draw.
+// env: the envelope `fill` writes for the items it assembles (see potrf_sequence)
 int factor_wave(const std::function<int(BatchView, int, const double *)> &fill, const std::function<double(const double *)> &diag_value,
                 BatchView A, int N, int nb, const double *hyp_w, int P, int *info_w, double *W, double *jit_dev, int *map_dev,
-                int jitter_policy, int border_rows, cudaStream_t s, int fuse = 0);
+                int jitter_policy, int border_rows, cudaStream_t s, int fuse = 0, Envelope env = {});
+// the envelope skips are on unless gpmc_set_tuning(14, 0) or GPMC_ENVELOPE=0 forced the dense path
+bool envelope_enabled();
 
 // Write rhs[item] (length n, row stride ldv) into border row n of every item (zero padded up to ld).
 int border_set(BatchView A, int n, const double *rhs, int ldv, int B, cudaStream_t s);

@@ -44,7 +44,8 @@ __device__ __forceinline__ void dmma884_8(double &c0, double &c1, double a, doub
 }
 
 __global__ void __launch_bounds__(T8_THREADS, 2)
-trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W, long long strideW, int nblk, int row_start, int n_mat)
+trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W, long long strideW, int nblk, int row_start, int n_mat,
+                   Envelope env)
 {
     extern __shared__ __align__(16) double sm[];
     double *Lb = sm;                              // 10 lower 32x32 blocks of L11
@@ -52,6 +53,18 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
     const int b = blockIdx.y;
     if (A.count && b >= *A.count) return;
     const int m = batch_item(A, b);
+    // a row block with no nonzero left of column j0 + NB is zero in this block column, and so is its solution: skip it,
+    // and leave at once when that holds for every row block of this CTA (border rows are never skipped)
+    auto empty_block = [&](int rb) {
+        const int row0 = row_start + rb * T8_ROWS;
+        const int rows_valid = (rb == nblk - 1) ? min(T8_ROWS + 8, n_rows - row0) : T8_ROWS;
+        return env_first_col(env, m, row0, row0 + rows_valid) >= j0 + NB;
+    };
+    if (env.blk) {
+        bool any = false;
+        for (int rb = blockIdx.x; rb < nblk && !any; rb += gridDim.x) any = !empty_block(rb);
+        if (!any) return;
+    }
     double *Ab = A.base + (size_t)m * A.stride;
     const int ld = A.ld;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -118,6 +131,7 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
     const int row0 = row_start + rb * T8_ROWS;
     const int rows_valid = (rb == nblk - 1) ? min(T8_ROWS + 8, n_rows - row0) : T8_ROWS;
     if (warp * 8 >= rows_valid) continue;         // nothing to solve (no border row, or a ragged last block)
+    if (env.blk && empty_block(rb)) continue;
     double *grow = Ab + (size_t)(row0 + min(r_loc, max(rows_valid, 1) - 1)) * ld + j0 + 2 * fk;
     if (rb != rb_first) {
 #pragma unroll
@@ -277,7 +291,8 @@ int launch_inv_blocks8(BatchView A, int n, double *W, long long strideW, int B, 
 static int g_trsm_blocks_per_cta = 0;
 void set_trsm_blocks_per_cta(int v) { g_trsm_blocks_per_cta = v; }
 
-int launch_trsm_panel8(BatchView A, int n_rows, int j0, const double *W, long long strideW, int B, cudaStream_t s, int row_start, int n_mat)
+int launch_trsm_panel8(BatchView A, int n_rows, int j0, const double *W, long long strideW, int B, cudaStream_t s, int row_start, int n_mat,
+                       Envelope env)
 {
     // default: every row below the diagonal block; row_start / n_mat: only the rows from row_start on (the border rows
     // of the LAST block column, whose diagonal block may be ragged: L11 rows / columns >= n_mat read as identity)
@@ -301,7 +316,7 @@ int launch_trsm_panel8(BatchView A, int n_rows, int j0, const double *W, long lo
     }
     dim3 grid((nblk + per_cta - 1) / per_cta, B);
     prof_begin(KC_TRSM, s);
-    trsm_panel8_kernel<<<grid, T8_THREADS, T8_SMEM, s>>>(A, n_rows, j0, W, strideW, nblk, row_start, n_mat);
+    trsm_panel8_kernel<<<grid, T8_THREADS, T8_SMEM, s>>>(A, n_rows, j0, W, strideW, nblk, row_start, n_mat, env);
     prof_end(KC_TRSM, s);
     GPMC_LAUNCH_CHECK();
     return 0;

@@ -233,8 +233,8 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
                    void *ws_dev, size_t ws_bytes, void *stream);
 
 /* Kernel tuning knobs for experiments.
- * (Environment, read once: GPMC_GEMM_CFG=<key 0 value> preselects the tile kernel variant; GPMC_DEBUG=1 makes the SDS loops
- *  print their round counters to stderr.)
+ * (Environment, read once: GPMC_GEMM_CFG=<key 0 value> preselects the tile kernel variant; GPMC_ENVELOPE=0 presets key 14
+ *  to 0; GPMC_DEBUG=1 makes the SDS loops print their round counters to stderr.)
  * key 0: DMMA tile kernel variant (0/1/2 cp.async staged, 3 TMA lock-step, 4 TMA free-running = default, 5 = 4 with
  *        persistent CTAs drawing tiles in order from a global counter: measured slower, kept for A/B).
  * key 1: panel factor kernel (0 = the register-resident kernel potf2_reg.cu (default), 3 = the same fragments as a dataflow
@@ -262,7 +262,11 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
  *        few matrices are in flight), 0 = none (one long-K product per block column), else forced.
  * key 13: 1 = the resident SDS loop chooses its factorisation schedules from a constant (min(slots, chains)) instead of the
  *        launch sizes: with a run-ahead deeper than 1 (key 7) those follow polled status words, and this keeps results
- *        repeatable bit for bit beyond N = 512 (1-4 % of the sweep time).  0 = default (not needed at run-ahead 1). */
+ *        repeatable bit for bit beyond N = 512 (1-4 % of the sweep time).  0 = default (not needed at run-ahead 1).
+ * key 14: envelope skips in gpmc_loglik_batched / gpmc_loglik_host: 1 = on (default): the assembly records, per 64-row block,
+ *        the first column that holds a nonzero, and the update GEMM and the panel solve skip the products it shows to be
+ *        exact zeros (K of a stationary kernel underflows to 0 far from the diagonal; results are bit-identical); 0 = dense.
+ *        Waves factored with fused panel launches (key 9) are always dense. */
 int gpmc_set_tuning(int key, int value);
 
 /* FP64 micro-benchmarks used by bench.py to put a measured peak beside the roofline:
