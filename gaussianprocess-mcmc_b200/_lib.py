@@ -15,7 +15,8 @@ ASM_ADD_S, ASM_LOWER_ONLY = 1, 2
 JITTER_NONE, JITTER_PYGPS = 0, 1
 INFO_NOT_PD = -1
 OP_POTRF, OP_LOGLIK, OP_SDS = 1, 2, 3
-KC_NAMES = ('assemble', 'gemm_update', 'potf2', 'panel_trsm', 'solve_reduce', 'tri_inverse', 'syrk_R', 'vector_control')
+KC_NAMES = ('assemble', 'gemm_update', 'potf2', 'panel_trsm', 'solve_reduce', 'tri_inverse', 'syrk_R', 'vector_control',
+            'band_clear')
 
 _c_double_p = ctypes.c_void_p     # raw addresses (torch data_ptr() / numpy ctypes.data)
 _vp = ctypes.c_void_p

@@ -83,14 +83,14 @@ struct LoglikLayout {
     int ld;
     size_t mat_elems;        // per item
     size_t fixed_bytes;      // per-call scratch independent of the wave
-    size_t per_item_bytes;   // matrix + W + envelope
+    size_t per_item_bytes;   // matrix + W + envelope + band
 };
 static LoglikLayout loglik_layout(int N, int B)
 {
     LoglikLayout l;
     l.ld = ld_for(N);
     l.mat_elems = (size_t)(N + 1) * l.ld;            // + the border row that carries g through the factorisation
-    l.per_item_bytes = l.mat_elems * sizeof(double) + (size_t)NB * NB * sizeof(double) + (size_t)env_blocks(N) * sizeof(int);
+    l.per_item_bytes = l.mat_elems * sizeof(double) + (size_t)NB * NB * sizeof(double) + 2 * (size_t)env_blocks(N) * sizeof(int);
     l.fixed_bytes = align_up((size_t)B * sizeof(double), 256)      // jitter
                     + align_up((size_t)B * sizeof(int), 256)       // map
                     + 256                                          // count
@@ -108,6 +108,62 @@ bool envelope_enabled()
     }
     return g_envelope != 0;
 }
+
+// Band-only assembly and launches (gpmc_set_tuning(15, .), GPMC_BAND), and where the region left of the band is cleared
+// (gpmc_set_tuning(16, .), GPMC_BAND_CLEAR): 2 = inline in the assembly (default: measured faster on the bench workload,
+// profiles/r03b_band_ab.json), 1 = side stream, 0 = not at all
+static int g_band = -1, g_band_clear = -1;
+static bool band_enabled()
+{
+    if (g_band < 0) {
+        const char *e = getenv("GPMC_BAND");
+        g_band = (e && e[0] == '0') ? 0 : 1;
+    }
+    // a band leaves the matrix unwritten left of it: only the update and solve kernels that start at the envelope keep
+    // their reads inside it (the other tile-kernel variants and the 32-column panel solve read whole rows)
+    return g_band != 0 && gemm_honours_envelope() && trsm_honours_envelope();
+}
+static int band_clear_mode()
+{
+    if (g_band_clear < 0) {
+        const char *e = getenv("GPMC_BAND_CLEAR");
+        g_band_clear = (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 2;
+    }
+    return g_band_clear;
+}
+
+// The band clear runs on a low-priority side stream per device: it starts after the band bound of its wave and the
+// caller's stream waits for it before the next wave's bound and before gpmc_loglik_batched returns.
+struct ClearStream {
+    cudaStream_t s = nullptr;
+    cudaEvent_t start = nullptr, done = nullptr;
+    bool ok = false;
+};
+static ClearStream *clear_stream()
+{
+    static ClearStream cs[64];
+    static bool tried[64] = {};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
+    if (!tried[dev]) {
+        tried[dev] = true;
+        int lo = 0, hi = 0;
+        ClearStream &c = cs[dev];
+        bool ok = cudaDeviceGetStreamPriorityRange(&lo, &hi) == cudaSuccess;
+        ok = ok && cudaStreamCreateWithPriority(&c.s, cudaStreamNonBlocking, lo) == cudaSuccess;
+        ok = ok && cudaEventCreateWithFlags(&c.start, cudaEventDisableTiming) == cudaSuccess;
+        ok = ok && cudaEventCreateWithFlags(&c.done, cudaEventDisableTiming) == cudaSuccess;
+        c.ok = ok;
+    }
+    return cs[dev].ok ? &cs[dev] : nullptr;
+}
+// the caller's stream waits for an issued clear on every way out of gpmc_loglik_batched (errors included)
+struct ClearJoin {
+    cudaStream_t s;
+    ClearStream *cs = nullptr;
+    bool pending = false;
+    ~ClearJoin() { if (pending) cudaStreamWaitEvent(s, cs->done, 0); }
+};
 
 // Assemble-and-factor one wave with kcGP.tools.jitchol semantics (pyGPs 1.3.4): one plain attempt for every item, then --
 // for the items that failed only -- any(diag <= 0) -> GPMC_INFO_NOT_PD, else the ladder mean(diag) * 1e-6 * 10^k, k < 5,
@@ -306,13 +362,16 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
     char *wp = (char *)ws_dev;
     double *jit_dev = (double *)wp; wp += align_up((size_t)B * sizeof(double), 256);
     int *map_dev = (int *)wp; wp += align_up((size_t)B * sizeof(int), 256);
-    wp += 256;
-    wp += align_up((size_t)32 * l.ld * sizeof(double), 256);      // (reserved: vector scratch)
+    int *band_dev = (int *)wp; wp += 256;                          // band bound: max r - lo[r], max r - w[r]
+    double *xbox = (double *)wp;                                    // band bound: boxes of x (2 D env_blocks(N) <= 32 ld doubles)
+    wp += align_up((size_t)32 * l.ld * sizeof(double), 256);
     const size_t wave_cap = std::min<size_t>((ws_bytes - l.fixed_bytes) / l.per_item_bytes, (size_t)MAX_BATCH_ITEMS);   // items ride in grid.y
     const int wave = (int)std::min<size_t>(wave_cap, (size_t)B);
     double *mats = (double *)wp;
     double *W = (double *)(wp + (size_t)wave * l.mat_elems * sizeof(double));
     const Envelope env_ws{(int *)(W + (size_t)wave * NB * NB), env_blocks(N), N};
+    int *band_w = env_ws.blk + (size_t)wave * env_blocks(N);
+    ClearJoin clear{s};
 
     { int rc0 = fill_int(info_dev, 0, B, s); if (rc0) return rc0; }
     for (int s0 = 0; s0 < B; s0 += wave) {
@@ -324,14 +383,49 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
         const int fuse = potrf_fuse_auto(N, nb, 1);
         // The fused panel launches (many small matrices) ignore the envelope, and the few short update contractions of
         // those matrices save less than recording and reading it costs (N=512 x 4096, ARD: 1 % slower): dense there.
-        const Envelope env = (envelope_enabled() && !fuse) ? env_ws : Envelope{};
+        Envelope env = (envelope_enabled() && !fuse) ? env_ws : Envelope{};
+        // Band: a bound taken before the assembly says which tiles can hold a nonzero; only those (widened, see Band) are
+        // assembled, and the update GEMM and the panel solve launch only the rows of the widest band of the wave.  The
+        // zeros left of the band are stored by a clear that nothing on the factorisation path waits for.
+        Band band{};
+        int rc = 0;
+        if (env.blk && band_enabled()) {
+            const int mode = band_clear_mode();
+            if (clear.pending) {                        // the previous wave's clear still writes these buffers
+                GPMC_CUDA_CHECK(cudaStreamWaitEvent(s, clear.cs->done, 0));
+                clear.pending = false;
+            }
+            GPMC_CUDA_CHECK(cudaMemsetAsync(band_dev, 0, 2 * sizeof(int), s));
+            rc = launch_band_bound(x_dev, N, D, hyp_w, P, n_ell, nb, band_w, env_blocks(N), band_dev, xbox, s);
+            if (rc) return rc;
+            // The launch sizes need the band on the host: one synchronisation.  The inline clear's assembly grid does not,
+            // and with few matrices in flight the update and solve launches are small anyway (N=16384 x 1 measured 0.3 %
+            // slower with the read-back), so such waves keep full launch grids.
+            int bh[2] = {-1, 0};
+            if (mode != 2 || (long long)nb * ((N + NB - 1) / NB) >= 1024) {
+                GPMC_CUDA_CHECK(cudaMemcpyAsync(bh, band_dev, sizeof(bh), cudaMemcpyDeviceToHost, s));
+                GPMC_CUDA_CHECK(cudaStreamSynchronize(s));
+            }
+            env.band = bh[0];
+            band = Band{band_w, env_blocks(N), bh[1], mode == 2};
+            if (mode == 1) {
+                ClearStream *cs = clear.cs ? clear.cs : (clear.cs = clear_stream());
+                if (!cs) { set_error("loglik: the band clear stream could not be created"); return GPMC_EINVAL; }
+                GPMC_CUDA_CHECK(cudaEventRecord(cs->start, s));
+                GPMC_CUDA_CHECK(cudaStreamWaitEvent(cs->s, cs->start, 0));
+                BatchView Aw{mats, (long long)l.mat_elems, l.ld, nullptr, nullptr};
+                if ((rc = launch_band_clear(Aw, N, band, nb, cs->s))) return rc;
+                GPMC_CUDA_CHECK(cudaEventRecord(cs->done, cs->s));
+                clear.pending = true;
+            }
+        }
         auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
-            int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env);
+            int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
             if (rc) return rc;
             return border_set(V, N, g_w, N, nitems, s);
         };
         auto diag = [&](const double *h) { return host_diag_value(h, n_ell); };
-        int rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, W, jit_dev, map_dev, jitter_policy, 1, s, fuse, env);
+        rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, W, jit_dev, map_dev, jitter_policy, 1, s, fuse, env);
         if (rc) return rc;
         // z = L^-1 g sits in the border row except for the last column block: finish it, then quad form + log det
         rc = border_finish(A, N, loglik_dev + s0, info_w, nb, s, fuse);
@@ -438,6 +532,8 @@ int gpmc_set_tuning(int key, int value)
     if (key == 11) { set_inverse_window(value); return 0; }
     if (key == 13) { set_sds_pin_schedule(value); return 0; }
     if (key == 14) { g_envelope = value != 0; return 0; }
+    if (key == 15) { g_band = value != 0; return 0; }
+    if (key == 16) { if (value < 0 || value > 2) return GPMC_EINVAL; g_band_clear = value; return 0; }
     return GPMC_EINVAL;
 }
 

@@ -16,7 +16,8 @@ constexpr int MAX_ELL = 8;         // max number of length-scales (ARD input dim
 constexpr int MAX_BATCH_ITEMS = 32768;   // batch items of one launch ride in grid.y / grid.z (limit 65535)
 
 // kernel classes for the profiling hooks (gpmc_profile_read)
-enum KernelClass { KC_ASSEMBLE = 0, KC_GEMM = 1, KC_POTF2 = 2, KC_TRSM = 3, KC_SOLVE = 4, KC_INV = 5, KC_SYRK_R = 6, KC_VEC = 7, KC_COUNT = 8 };
+enum KernelClass { KC_ASSEMBLE = 0, KC_GEMM = 1, KC_POTF2 = 2, KC_TRSM = 3, KC_SOLVE = 4, KC_INV = 5, KC_SYRK_R = 6, KC_VEC = 7,
+                   KC_CLEAR = 8, KC_COUNT = 9 };
 
 void set_error(const char *fmt, ...);
 // Every computing entry point of the C ABI takes this (recursive) lock: the library keeps per-process state (side streams,
@@ -86,6 +87,31 @@ struct Envelope {
     int *blk = nullptr;
     int ld = 0;            // ints between items
     int n = 0;             // order of the matrix
+    int band = -1;         // >= 0: no row block r of any item holds a nonzero left of 64-column tile r - band (so rows more
+                           // than `band` blocks below a block column's last tile are zero in it: the update GEMM and the
+                           // panel solve launch no CTA for them); -1: unknown
+};
+
+// Band of an assembled matrix (gpmc_loglik_batched with the band on).  A conservative bound taken from bounding boxes of
+// x / ell gives, per item and 64-row block r, lo[r]: the leftmost 64-column tile that can hold a nonzero.  The assembly
+// writes only tiles w[r] .. r of row block r, with
+//     w[r] = min(lo[r-1], lo[r], lo[r+1]) rounded down to a multiple of NB / 64.
+// Nothing on the factorisation path reads a row left of its w, which is why the stored band may stay unwritten (or be
+// cleared off the critical path):
+//   * the update GEMM's 128-row A tile (two row blocks) starts at the later envelope of its rows, >= the min of their lo,
+//     floor 16; B rows start at their own envelope; its C tile (columns of the block column) is only read by a tile whose
+//     contraction is not empty, i.e. when one of its row blocks has a nonzero left of the block column -- so both row
+//     blocks have w left of the block column;
+//   * the panel factor reads the diagonal NB x NB block (w rounded down to NB / 64 tiles keeps its lower part written);
+//   * the panel solve reads a row block's whole NB-wide block column only when the block has a nonzero in it (lo <= the
+//     block column's last tile, so the rounded-down w is at or left of its first tile);
+//   * the last-block solve, the quadratic form and the log-determinant read the diagonal and the diagonal blocks;
+//   * the jitter ladder re-assembles the same band (the bound does not depend on the jitter).
+struct Band {
+    const int *w = nullptr;  // w[item * ld + r]; nullptr: the whole lower triangle is assembled
+    int ld = 0;
+    int width = 0;           // max over the wave of r - w[r] (tiles left of the diagonal tile the assembly writes)
+    int clear = 0;           // cov_assemble also writes +0 left of w[r] (band clear done inline)
 };
 __host__ __device__ inline int env_blocks(int n) { return (n + ENV_ROWS - 1) / ENV_ROWS; }
 
@@ -104,8 +130,16 @@ __device__ __forceinline__ int env_first_col(const Envelope &e, int m, int r0, i
 
 // cov_assemble.cu
 // env.blk != nullptr: also writes the envelope of every assembled item (the items A selects)
+// band.w != nullptr: only the tiles of the band (see Band) are written
 int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P, int n_ell, int flags,
-                        const double *jitter, BatchView A, int B, cudaStream_t s, Envelope env = {});
+                        const double *jitter, BatchView A, int B, cudaStream_t s, Envelope env = {}, Band band = {});
+// Band bound of items 0 .. B-1 (hyp rows, as launch_cov_assemble reads them): w[item * ldw + r] (see Band), and
+// band_out[0] = max over items and r of r - lo[r], band_out[1] = max of r - w[r] (band_out must start at 0).
+// xbox: scratch of 2 * D * env_blocks(N) doubles.
+int launch_band_bound(const double *x, int N, int D, const double *hyp, int P, int n_ell, int B, int *w, int ldw,
+                      int *band_out, double *xbox, cudaStream_t s);
+// +0 into every element of rows 0 .. N-1 of items 0 .. B-1 left of their row block's w (store only, small grid)
+int launch_band_clear(BatchView A, int N, Band band, int B, cudaStream_t s);
 
 // gemm_dmma.cu :  C[i][j] (op)= sum_k A[i][k] * B[j][k]   ("NT": both operands K-contiguous, row-major)
 struct Operand {
@@ -142,6 +176,7 @@ struct GemmArgs {
 };
 int launch_gemm(const GemmArgs &a, int B, int kclass, cudaStream_t s);
 void set_gemm_config(int cfg);
+bool gemm_honours_envelope();      // the selected tile kernel starts its contractions at the envelope (cfg 4)
 
 // potf2.cu : factor the NB x NB diagonal block at (j0, j0) in place, write its inverse to W
 int launch_potf2(BatchView A, int n, int j0, double *W, long long strideW, int *info, int zero_upper,
@@ -174,7 +209,8 @@ int launch_trsm_panel(BatchView A, int n, int j0, const double *W, long long str
 // trsm_panel8.cu : the same solve with 8-column sub-blocks, shuffle-based fragment conversion, 2 CTAs per SM (default)
 //   row_start >= 0: solve only rows row_start .. n-1 (border rows of the last block column); n_mat >= 0: order of the matrix
 //   (rows / columns of the diagonal block at or beyond it read as identity)
-//   env: envelope of A -- a 64-row block whose rows have no nonzero left of j0 + NB is zero and stays so (skipped)
+//   env: envelope of A -- a 64-row block whose rows have no nonzero left of j0 + NB is zero and stays so (skipped); with
+//   env.band >= 0 and rows below the matrix only the band's row blocks and those rows are launched
 int launch_trsm_panel8(BatchView A, int n, int j0, const double *W, long long strideW, int B, cudaStream_t s,
                        int row_start = -1, int n_mat = -1, Envelope env = {});
 // trmm_panel8.cu : in place  A[0:rows, c0:c0+width] = -(A[0:rows, c0:c0+128] W^T)  for a lower triangular 128x128 W
@@ -184,6 +220,7 @@ int launch_trmm_panel8(BatchView A, int rows, int c0, int width, const double *W
 //   (W: nt blocks of NB x NB per item, item stride strideW)
 int launch_inv_blocks8(BatchView A, int n, double *W, long long strideW, int B, cudaStream_t s);
 void set_trsm_mode(int mode);      // 0: trsm_panel8 (default), 1: trsm_panel (32-column sub-blocks)
+bool trsm_honours_envelope();      // the selected panel solve skips the row blocks the envelope shows to be zero (mode 0)
 void set_trsm_blocks_per_cta(int v);   // 0: auto (1, 2 or 4 by launch size), else forced
 
 // solve_reduce.cu : z = L^-1 (a - b), optional outputs: z, loglik = -(0.5 z.z + sum log L_ii + 0.5 n log 2pi)

@@ -141,6 +141,20 @@ int launch_gemm_tma(const GemmArgs &a, int B, int kclass, bool free_running, cud
 // the next tile's first chunks during the current tile's tail (used for short contractions when 4 is selected: see below)
 static int g_gemm_cfg = 4;
 void set_gemm_config(int cfg) { g_gemm_cfg = cfg; }
+static void read_gemm_env()
+{
+    static bool env_read = false;
+    if (!env_read) {            // GPMC_GEMM_CFG=0..3 selects the tile-kernel variant (experiments / A-B tests)
+        const char *e = getenv("GPMC_GEMM_CFG");
+        if (e && e[0] >= '0' && e[0] <= '5') g_gemm_cfg = e[0] - '0';
+        env_read = true;
+    }
+}
+bool gemm_honours_envelope()
+{
+    read_gemm_env();
+    return g_gemm_cfg == 4;
+}
 
 template <typename K>
 static int launch_variant(K kernel, const GemmArgs &a, int B, int bn, int threads, int smem, int kclass, cudaStream_t s, DeviceOnce &attr_set)
@@ -166,18 +180,15 @@ int launch_gemm(const GemmArgs &a, int B, int kclass, cudaStream_t s)
         return GPMC_EALIGN;
     }
     static DeviceOnce set0, set1, set2;
-    static bool env_read = false;
-    if (!env_read) {            // GPMC_GEMM_CFG=0..3 selects the tile-kernel variant (experiments / A-B tests)
-        const char *e = getenv("GPMC_GEMM_CFG");
-        if (e && e[0] >= '0' && e[0] <= '5') g_gemm_cfg = e[0] - '0';
-        env_read = true;
-    }
+    read_gemm_env();
     const bool border_fusable = a.border_row == 0 || (a.skip_upper && a.epi == EPI_SUB && a.cr0 == a.cc0 && a.A.base == a.C.base);
     // persistent form: every tile needs at least one chunk, and the tile count must fit the scheduler's 32-bit words
     const bool persist_ok = !a.k_follow_row && a.klen >= 1 &&
                             (long long)((a.rows + 127) / 128 + 1) * ((a.cols + 63) / 64 + 1) * B < 0x70000000LL;
     if (g_gemm_cfg == 5 && persist_ok && gemm_tma_supported(a) && border_fusable) return launch_gemm_tma(a, B, kclass, true, s, true);
     if (g_gemm_cfg == 4 && gemm_tma_supported(a) && border_fusable) return launch_gemm_tma(a, B, kclass, true, s);   // border row fused in-kernel
+    // a band (env.band >= 0) leaves the matrix unwritten left of it: only the kernel above keeps its reads inside
+    if (a.env.band >= 0) { set_error("gemm: a banded update needs the envelope-aware TMA tile kernel (tuning key 0 = 4)"); return GPMC_EINVAL; }
     if (a.border_row > 0) {
         // the other variants have no border duty: take the row along as one more output row (it follows the matrix)
         if (a.cr0 + a.rows != a.border_row || a.ar0 != a.cr0) { set_error("gemm: border row %d is not adjacent to the output rows", a.border_row); return GPMC_EINVAL; }

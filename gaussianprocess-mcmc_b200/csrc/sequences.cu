@@ -197,6 +197,7 @@ static int potrf_window_for(int n, int B)
 
 static int g_trsm_mode = 0;
 void set_trsm_mode(int mode) { g_trsm_mode = mode; }
+bool trsm_honours_envelope() { return g_trsm_mode == 0; }
 static int g_potf2_mode = 0;
 void set_potf2_mode(int mode) { g_potf2_mode = mode; }
 static bool lite_panels() { return g_trsm_mode == 0 && g_potf2_mode != 1; }
@@ -293,6 +294,10 @@ int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long st
         GemmArgs g{};
         g.C = A; g.A = self; g.B = self;
         g.cr0 = j0; g.cc0 = j0; g.rows = n - j0 + xrows; g.cols = width;
+        // band: rows more than env.band row blocks below the block column are zero left of it (their tiles would leave at
+        // once).  The diagonal tile, which carries the border row, is always launched.  The right-looking trailing updates
+        // of the windowed schedule keep their full grids.
+        if (env.band >= 0 && xrows == 0) g.rows = std::min(g.rows, NB + env.band * ENV_ROWS);
         g.border_row = brow;
         g.ar0 = j0; g.br0 = j0; g.k0 = k_begin; g.bk0 = k_begin; g.klen = k_end - k_begin;
         g.epi = EPI_SUB;

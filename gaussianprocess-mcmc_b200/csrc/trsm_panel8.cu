@@ -45,7 +45,7 @@ __device__ __forceinline__ void dmma884_8(double &c0, double &c1, double a, doub
 
 __global__ void __launch_bounds__(T8_THREADS, 2)
 trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W, long long strideW, int nblk, int row_start, int n_mat,
-                   Envelope env)
+                   Envelope env, int nband)
 {
     extern __shared__ __align__(16) double sm[];
     double *Lb = sm;                              // 10 lower 32x32 blocks of L11
@@ -53,6 +53,17 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
     const int b = blockIdx.y;
     if (A.count && b >= *A.count) return;
     const int m = batch_item(A, b);
+    // nband >= 0: the launch takes row blocks 0 .. nband-1 (the band) and then the last row block for its border rows only
+    // (its matrix rows lie below the band: zero in this block column, and not necessarily written)
+    const int nlaunch = nband >= 0 ? nband + 1 : nblk;
+    auto blk_of = [&](int i) { return (nband >= 0 && i == nband) ? nblk - 1 : i; };
+    // the last row block solves its matrix rows only when the envelope shows a nonzero in them: zero rows stay zero, and
+    // left of a band they may not have been written (a failed factorisation would otherwise leave NaN there for good)
+    auto border_only = [&](int rb) {
+        if (rb != nblk - 1) return false;
+        const int row0 = row_start + rb * T8_ROWS;
+        return nband >= 0 || (env.blk && row0 < env.n && env_first_col(env, m, row0, env.n) >= j0 + NB);
+    };
     // a row block with no nonzero left of column j0 + NB is zero in this block column, and so is its solution: skip it,
     // and leave at once when that holds for every row block of this CTA (border rows are never skipped)
     auto empty_block = [&](int rb) {
@@ -62,7 +73,7 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
     };
     if (env.blk) {
         bool any = false;
-        for (int rb = blockIdx.x; rb < nblk && !any; rb += gridDim.x) any = !empty_block(rb);
+        for (int i = blockIdx.x; i < nlaunch && !any; i += gridDim.x) any = !empty_block(blk_of(i));
         if (!any) return;
     }
     double *Ab = A.base + (size_t)m * A.stride;
@@ -98,18 +109,21 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
     // matrices in flight a CTA solves several row blocks against the L11 it staged once (the 108 KB prologue is what
     // kept the DMMA pipe at 75 % when every CTA took a single block).
     // n_rows counts a border row too; the last row block takes every row that is left (at most 64 + 1)
-    const int rb_first = blockIdx.x;
+    const int rb_first = blk_of(blockIdx.x);
     const int row0_first = row_start + rb_first * T8_ROWS;
     const int rv_first = (rb_first == nblk - 1) ? min(T8_ROWS + 8, n_rows - row0_first) : T8_ROWS;
     // this warp's 8 rows as accumulator fragments: acc[b8] = row warp*8 + fr, cols b8*8 + 2fk, +1
     double acc[T8_NB8][2];
     const int r_loc = warp * 8 + fr;
+    // rows this lane solves in row block rb
+    auto row_ok = [&](int rb, int row0, int rows_valid) { return r_loc < rows_valid && (!border_only(rb) || row0 + r_loc >= env.n); };
     {
         const double *grow0 = Ab + (size_t)(row0_first + min(r_loc, max(rv_first, 1) - 1)) * ld + j0 + 2 * fk;
+        const bool ok = row_ok(rb_first, row0_first, rv_first);
 #pragma unroll
         for (int b8 = 0; b8 < T8_NB8; ++b8) {
             double2 v = make_double2(0.0, 0.0);
-            if (r_loc < rv_first && b8 * 8 + 2 * fk < ncv) v = *reinterpret_cast<const double2 *>(grow0 + b8 * 8);
+            if (ok && b8 * 8 + 2 * fk < ncv) v = *reinterpret_cast<const double2 *>(grow0 + b8 * 8);
             acc[b8][0] = v.x;
             acc[b8][1] = v.y;
         }
@@ -127,17 +141,20 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
     }
     __syncthreads();
 
-    for (int rb = rb_first; rb < nblk; rb += gridDim.x) {
+    for (int li = blockIdx.x; li < nlaunch; li += gridDim.x) {
+    const int rb = blk_of(li);
     const int row0 = row_start + rb * T8_ROWS;
     const int rows_valid = (rb == nblk - 1) ? min(T8_ROWS + 8, n_rows - row0) : T8_ROWS;
     if (warp * 8 >= rows_valid) continue;         // nothing to solve (no border row, or a ragged last block)
+    if (border_only(rb) && row0 + warp * 8 + 7 < env.n) continue;
     if (env.blk && empty_block(rb)) continue;
+    const bool ok = row_ok(rb, row0, rows_valid);
     double *grow = Ab + (size_t)(row0 + min(r_loc, max(rows_valid, 1) - 1)) * ld + j0 + 2 * fk;
     if (rb != rb_first) {
 #pragma unroll
         for (int b8 = 0; b8 < T8_NB8; ++b8) {
             double2 v = make_double2(0.0, 0.0);
-            if (r_loc < rows_valid && b8 * 8 + 2 * fk < ncv) v = *reinterpret_cast<const double2 *>(grow + b8 * 8);
+            if (ok && b8 * 8 + 2 * fk < ncv) v = *reinterpret_cast<const double2 *>(grow + b8 * 8);
             acc[b8][0] = v.x;
             acc[b8][1] = v.y;
         }
@@ -169,7 +186,7 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
             dmma884_8(acc[bp][0], acc[bp][1], nx1, lp.y);
         }
         // ---- the finished 8 columns leave from the accumulator registers (4 lanes x 16 bytes per row)
-        if (r_loc < rows_valid) {
+        if (ok) {
             const int c = b8 * 8 + 2 * fk;
             if (c + 1 < ncv) *reinterpret_cast<double2 *>(grow + b8 * 8) = make_double2(x0, x1);
             else if (c < ncv) grow[b8 * 8] = x0;
@@ -307,16 +324,21 @@ int launch_trsm_panel8(BatchView A, int n_rows, int j0, const double *W, long lo
         GPMC_CUDA_CHECK(cudaFuncSetAttribute(trsm_panel8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, T8_SMEM));
     }
     const int nblk = (rows + T8_ROWS - 1) / T8_ROWS;
+    // band (env.band >= 0, rows below the matrix present): the row blocks that can hold a nonzero left of j0 + NB are the
+    // first env.band ones; the others would leave at once -- launch those and the last block (its border rows)
+    int nband = -1;
+    if (env.blk && env.band >= 0 && n_rows > env.n && row_start == j0 + NB && env.band < nblk - 1) nband = env.band;
+    const int nlaunch = nband >= 0 ? nband + 1 : nblk;
     // CTAs per matrix: one per row block while the launch would not fill the chip several times over, else up to
     // four row blocks per CTA (g_trsm_blocks_per_cta overrides: experiments)
     int per_cta = g_trsm_blocks_per_cta;
     if (per_cta <= 0) {
-        const long long ctas = (long long)nblk * B;
+        const long long ctas = (long long)nlaunch * B;
         per_cta = ctas >= 16 * 296 ? 4 : (ctas >= 8 * 296 ? 2 : 1);
     }
-    dim3 grid((nblk + per_cta - 1) / per_cta, B);
+    dim3 grid((nlaunch + per_cta - 1) / per_cta, B);
     prof_begin(KC_TRSM, s);
-    trsm_panel8_kernel<<<grid, T8_THREADS, T8_SMEM, s>>>(A, n_rows, j0, W, strideW, nblk, row_start, n_mat, env);
+    trsm_panel8_kernel<<<grid, T8_THREADS, T8_SMEM, s>>>(A, n_rows, j0, W, strideW, nblk, row_start, n_mat, env, nband);
     prof_end(KC_TRSM, s);
     GPMC_LAUNCH_CHECK();
     return 0;

@@ -266,7 +266,16 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
  * key 14: envelope skips in gpmc_loglik_batched / gpmc_loglik_host: 1 = on (default): the assembly records, per 64-row block,
  *        the first column that holds a nonzero, and the update GEMM and the panel solve skip the products it shows to be
  *        exact zeros (K of a stationary kernel underflows to 0 far from the diagonal; results are bit-identical); 0 = dense.
- *        Waves factored with fused panel launches (key 9) are always dense. */
+ *        Waves factored with fused panel launches (key 9) are always dense.
+ * key 15: band (with key 14 on): 1 = on (default): a bound from bounding boxes of x / ell gives, per 64-row block, the first
+ *        64-column tile that can hold a nonzero; only the band right of it is assembled, and the update GEMM and the panel
+ *        solve launch only the rows of the widest band of the wave (bit-identical results); 0 = envelope skips only.
+ *        GPMC_BAND=0 presets it to 0.
+ *        The band is used only with the envelope-aware kernels (key 0 = 4, key 4 = 0); with the others key 15 acts as 0.
+ * key 16: where the band's key 15 stores the +0 left of the band, which nothing on the factorisation path reads: 2 = inline
+ *        in the assembly (default), 1 = on a low-priority side stream beside the factorisation (measured slower on the
+ *        bench workload: the stores compete with the band's assembly), 0 = not at all (the workspace keeps what it held
+ *        there; results are unchanged).  GPMC_BAND_CLEAR=<value> presets it. */
 int gpmc_set_tuning(int key, int value);
 
 /* FP64 micro-benchmarks used by bench.py to put a measured peak beside the roofline:
