@@ -52,6 +52,7 @@ SIGNATURES = {
     'gpmc_ess_sweep': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, ctypes.c_double, ctypes.c_double, ctypes.c_double,
                             ctypes.c_ulonglong, ctypes.c_uint, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     'gpmc_set_tuning': (_i, [_i, _i]),
+    'gpmc_loglik_layout': (_i, [ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)]),
     'gpmc_bench_fp64_peak': (_i, [_i, _i, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]),
     'gpmc_bench_dmma_ilp': (_i, [_i, _i, _i, ctypes.POINTER(ctypes.c_double)]),
     'gpmc_sds_loop_stats': (_i, [ctypes.POINTER(ctypes.c_longlong)] * 3),

@@ -112,7 +112,7 @@ bool envelope_enabled()
 // Band-only assembly and launches (gpmc_set_tuning(15, .), GPMC_BAND), and where the region left of the band is cleared
 // (gpmc_set_tuning(16, .), GPMC_BAND_CLEAR): 2 = inline in the assembly (default: measured faster on the bench workload,
 // profiles/r03b_band_ab.json), 1 = side stream, 0 = not at all
-static int g_band = -1, g_band_clear = -1;
+static int g_band = -1, g_band_clear = -1, g_band_compact = -1;
 static bool band_enabled()
 {
     if (g_band < 0) {
@@ -123,6 +123,18 @@ static bool band_enabled()
     // their reads inside it (the other tile-kernel variants and the 32-column panel solve read whole rows)
     return g_band != 0 && gemm_honours_envelope() && trsm_honours_envelope();
 }
+// Compact band storage (gpmc_set_tuning(17, .), GPMC_BAND_COMPACT): 1 = automatic (default), 0 = always the dense layout
+static bool band_compact_allowed()
+{
+    if (g_band_compact < 0) {
+        const char *e = getenv("GPMC_BAND_COMPACT");
+        g_band_compact = (e && e[0] == '0') ? 0 : 1;
+    }
+    return g_band_compact != 0;
+}
+// layout of the last gpmc_loglik_batched call (gpmc_loglik_layout)
+static int g_last_W = 0, g_last_waves = 0;
+
 static int band_clear_mode()
 {
     if (g_band_clear < 0) {
@@ -200,7 +212,9 @@ int factor_wave(const std::function<int(BatchView, int, const double *)> &fill, 
         GPMC_CUDA_CHECK(cudaMemcpyAsync(jit_dev, jit.data(), nb * sizeof(double), cudaMemcpyHostToDevice, s));
         for (int i : todo) info[i] = 0;
         GPMC_CUDA_CHECK(cudaMemcpyAsync(info_w, info.data(), nb * sizeof(int), cudaMemcpyHostToDevice, s));
-        BatchView Am{A.base, A.stride, A.ld, map_dev, nullptr};
+        BatchView Am = A;                               // the failed items, re-assembled in place
+        Am.map = map_dev;
+        Am.count = nullptr;
         if ((rc = fill(Am, nf, jit_dev))) return rc;
         if ((rc = potrf_sequence(Am, N, nf, info_w, W, NB * NB, 0, 0, s, border_rows, fuse, env))) return rc;
         GPMC_CUDA_CHECK(cudaMemcpyAsync(info.data(), info_w, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -367,13 +381,70 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
     wp += align_up((size_t)32 * l.ld * sizeof(double), 256);
     const size_t wave_cap = std::min<size_t>((ws_bytes - l.fixed_bytes) / l.per_item_bytes, (size_t)MAX_BATCH_ITEMS);   // items ride in grid.y
     const int wave = (int)std::min<size_t>(wave_cap, (size_t)B);
+    g_last_W = 0;
+    g_last_waves = (B + wave - 1) / wave;
+    { int rc0 = fill_int(info_dev, 0, B, s); if (rc0) return rc0; }
+
+    // Compact band layout: when the dense layout needs several waves, bound the band of every item of the call first.
+    // Rows W = 128 + 64 * (widest band) columns wide hold every element the factorisation reads (see BatchView, Band); it
+    // is used when it needs fewer waves and those waves run the plain left-looking schedule (the kernels that know it).
+    if (wave < B && band_compact_allowed() && envelope_enabled() && band_enabled()) {
+        const int nblk = env_blocks(N);
+        const size_t wenv = align_up((size_t)B * nblk * sizeof(int), 256);
+        char *cp = wp;
+        int *w_all = (int *)cp; cp += wenv;              // band starts of every item of the call
+        int *env_all = (int *)cp; cp += wenv;            // envelopes of every item of the call
+        const size_t room = ws_bytes - l.fixed_bytes;
+        if (2 * wenv + 256 < room) {
+            GPMC_CUDA_CHECK(cudaMemsetAsync(band_dev, 0, 2 * sizeof(int), s));
+            int rc = launch_band_bound(x_dev, N, D, hyp_dev, P, n_ell, B, w_all, nblk, band_dev, xbox, s);
+            if (rc) return rc;
+            int bh[2] = {0, 0};
+            GPMC_CUDA_CHECK(cudaMemcpyAsync(bh, band_dev, sizeof(bh), cudaMemcpyDeviceToHost, s));
+            GPMC_CUDA_CHECK(cudaStreamSynchronize(s));
+            const int Wc = (int)align_up((size_t)BAND_ROWS + (size_t)ENV_ROWS * bh[1], 16);
+            // per item: the rows, the border row and the panel factor's scratch
+            const size_t per_item = (size_t)N * Wc * sizeof(double) + (size_t)l.ld * sizeof(double) + (size_t)NB * NB * sizeof(double);
+            const size_t wave_c = std::min<size_t>((room - 2 * wenv - 256) / per_item, (size_t)MAX_BATCH_ITEMS);   // 256: the border rows' alignment
+            const int waves_c = wave_c > 0 ? (int)((B + wave_c - 1) / wave_c) : 0;
+            // equal waves (sizes differ by one at most), so that every wave runs the same schedule
+            const int nb_lo = waves_c > 0 ? B / waves_c : 0, nb_hi = waves_c > 0 ? (B + waves_c - 1) / waves_c : 0;
+            if (Wc < l.ld && waves_c > 0 && waves_c < g_last_waves && potrf_compact_ok(N, nb_lo, 1) && potrf_compact_ok(N, nb_hi, 1)) {
+                double *border = (double *)cp; cp += align_up((size_t)nb_hi * l.ld * sizeof(double), 256);
+                double *Wsc = (double *)cp; cp += (size_t)nb_hi * NB * NB * sizeof(double);
+                double *mats_c = (double *)cp;
+                g_last_W = Wc;
+                g_last_waves = waves_c;
+                for (int wi = 0, s0 = 0; wi < waves_c; ++wi) {
+                    const int nb = nb_lo + (wi < B % waves_c ? 1 : 0);
+                    BatchView A{mats_c, (long long)N * Wc, Wc, nullptr, nullptr, Wc, N, border, l.ld};
+                    const Envelope env{env_all + (size_t)s0 * nblk, nblk, N, bh[0]};
+                    const Band band{w_all + (size_t)s0 * nblk, nblk, bh[1], 0};
+                    const double *hyp_w = hyp_dev + (size_t)s0 * P;
+                    const double *g_w = g_dev + (size_t)s0 * N;
+                    int *info_w = info_dev + s0;
+                    auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
+                        int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
+                        if (rc) return rc;
+                        return border_set(V, N, g_w, N, nitems, s);
+                    };
+                    auto diag = [&](const double *h) { return host_diag_value(h, n_ell); };
+                    rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, Wsc, jit_dev, map_dev, jitter_policy, 1, s, 0, env);
+                    if (rc) return rc;
+                    if ((rc = border_finish(A, N, loglik_dev + s0, info_w, nb, s, 0))) return rc;
+                    s0 += nb;
+                }
+                return 0;
+            }
+        }
+    }
+
     double *mats = (double *)wp;
     double *W = (double *)(wp + (size_t)wave * l.mat_elems * sizeof(double));
     const Envelope env_ws{(int *)(W + (size_t)wave * NB * NB), env_blocks(N), N};
     int *band_w = env_ws.blk + (size_t)wave * env_blocks(N);
     ClearJoin clear{s};
 
-    { int rc0 = fill_int(info_dev, 0, B, s); if (rc0) return rc0; }
     for (int s0 = 0; s0 < B; s0 += wave) {
         const int nb = std::min(wave, B - s0);
         const double *hyp_w = hyp_dev + (size_t)s0 * P;
@@ -534,7 +605,16 @@ int gpmc_set_tuning(int key, int value)
     if (key == 14) { g_envelope = value != 0; return 0; }
     if (key == 15) { g_band = value != 0; return 0; }
     if (key == 16) { if (value < 0 || value > 2) return GPMC_EINVAL; g_band_clear = value; return 0; }
+    if (key == 17) { g_band_compact = value != 0; return 0; }
     return GPMC_EINVAL;
+}
+
+int gpmc_loglik_layout(int *band_W, int *waves)
+{
+    GPMC_API_LOCK();
+    if (band_W) *band_W = g_last_W;
+    if (waves) *waves = g_last_waves;
+    return 0;
 }
 
 int gpmc_sds_loop_stats(long long *rounds, long long *idle_rounds, long long *ladders)

@@ -66,15 +66,38 @@ struct DeviceOnce {
 // ---------------------------------------------------------------------------------------------
 // Batched matrix view.  Item b of a launch is matrix `map ? map[b] : b` of the allocation, so a
 // compacted list of active chains / failed items can be processed without moving data.
+// Compact band layout (W > 0, gpmc_loglik_batched when its band is narrow): row r keeps only the W columns
+// band_col0(r, W) .. band_col0(r, W) + W - 1, stored at base + item * stride + r * W.  The shift is constant over each
+// 128-row block (the update tile's height and the panel width), so every tile the kernels touch is still a rectangle with
+// row stride W, and it ends at the diagonal block.  band_col0 may be negative for the first blocks.  W is a multiple of 16,
+// so the 16-column contraction chunks line up with the dense ones.  The border row (row n, the right-hand side carried
+// through the factorisation) is dense and lives in its own array.  Nothing outside the band may be read (see Band).
+constexpr int BAND_ROWS = 128;
 struct BatchView {
     double *base;          // first matrix
     long long stride;      // elements between matrices
-    int ld;                // leading dimension (even; multiple of 16 for internal buffers)
+    int ld;                // leading dimension (even; multiple of 16 for internal buffers); == W in the compact layout
     const int *map;        // optional indirection (device), may be nullptr
     const int *count;      // optional device-side item count; CTAs with blockIdx.y >= *count exit
+    int W = 0;             // 0: dense; > 0: compact band layout of width W
+    int n = 0;             // compact layout: order of the matrix; row n is the border row
+    double *border = nullptr;        // compact layout: border rows, item m's at border + m * border_stride
+    long long border_stride = 0;
 };
 
 __device__ __forceinline__ int batch_item(const BatchView &v, int b) { return v.map ? v.map[b] : b; }
+
+__host__ __device__ __forceinline__ int band_col0(int r, int W) { return (r / BAND_ROWS) * BAND_ROWS + BAND_ROWS - W; }
+
+// element (r, c) of item m -- every kernel that may see the compact layout addresses the matrix through this
+__host__ __device__ __forceinline__ double *view_elem(const BatchView &v, int m, int r, int c)
+{
+    if (!v.W) return v.base + (size_t)m * v.stride + (size_t)r * v.ld + c;
+    if (r >= v.n) return v.border + (size_t)m * v.border_stride + c;
+    return v.base + ((long long)m * v.stride + (long long)r * v.W + (c - band_col0(r, v.W)));
+}
+// elements between the border rows of consecutive items
+__host__ __device__ __forceinline__ long long view_border_stride(const BatchView &v) { return v.W ? v.border_stride : v.stride; }
 
 // ---------------------------------------------------------------------------------------------
 // Envelope of an assembled matrix.  blk[item * ld + r] is the smallest column that holds a nonzero in rows
@@ -107,6 +130,8 @@ struct Envelope {
 //     block column's last tile, so the rounded-down w is at or left of its first tile);
 //   * the last-block solve, the quadratic form and the log-determinant read the diagonal and the diagonal blocks;
 //   * the jitter ladder re-assembles the same band (the bound does not depend on the jitter).
+// The compact layout (see BatchView) stores exactly that much: with width = max over items of r - w[r], W >= 128 +
+// 64 width puts band_col0 of every 128-row block at or left of 64 w[r] of both its 64-row blocks.
 struct Band {
     const int *w = nullptr;  // w[item * ld + r]; nullptr: the whole lower triangle is assembled
     int ld = 0;

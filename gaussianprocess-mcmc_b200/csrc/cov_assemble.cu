@@ -111,7 +111,6 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
     const double diag_add = s_scal[1], jit = s_scal[2], sn2 = s_scal[3];
     constexpr bool pred = PRED;
     const bool has_jit = (jitter != nullptr);
-    double *Ab = A.base + (size_t)m * A.stride;
     const int cl = 2 * lane;
     const int ntiles = band.w && !band.clear ? nt1 * (band.width + 1) : nt1 * (nt1 + 1) / 2;
     // A CTA takes ASM_TPC consecutive tiles of its matrix (experiment: amortise the per-item scalars above -- two
@@ -148,7 +147,7 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
         double uj0[DT > 0 ? DT : 1], uj1[DT > 0 ? DT : 1];
 #pragma unroll
         for (int d = 0; d < DT; ++d) { uj0[d] = s_uj[d][cl]; uj1[d] = s_uj[d][cl + 1]; }
-        double *dst = Ab + (size_t)(r0 + warp * 8) * A.ld + gc;
+        double *dst = view_elem(A, m, r0 + warp * 8, gc);     // 8 rows of one 64-row block: row stride A.ld
 #pragma unroll
         for (int rr = 0; rr < 8; ++rr) {
             const int rl = warp * 8 + rr;
@@ -188,7 +187,7 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
         if (gr == gc + 1) { k1 = k1 + diag_add; if (has_jit) k1 = k1 + jit; }
         if (mirror) *reinterpret_cast<double2 *>(&s_tile[rl][cl]) = make_double2(k0, k1);
         if (gr < N) {
-            double *dst = Ab + (size_t)gr * A.ld + gc;
+            double *dst = view_elem(A, m, gr, gc);
             if (gc + 1 < N)      *reinterpret_cast<double2 *>(dst) = make_double2(k0, k1);
             else if (gc < N)     dst[0] = k0;
             nz0 |= (k0 != 0.0 && gc < N && gc <= gr);
@@ -216,7 +215,7 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
         const double k0 = s_tile[cl][cm];
         const double k1 = s_tile[cl + 1][cm];
         if (gr < N) {
-            double *dst = Ab + (size_t)gr * A.ld + gcol;
+            double *dst = view_elem(A, m, gr, gcol);
             if (gcol + 1 < N)    *reinterpret_cast<double2 *>(dst) = make_double2(k0, k1);
             else if (gcol < N)   dst[0] = k0;
         }
@@ -356,6 +355,7 @@ __global__ void __launch_bounds__(256) band_clear_kernel(BatchView A, int N, Ban
 int launch_band_clear(BatchView A, int N, Band band, int B, cudaStream_t s)
 {
     if (B <= 0 || !band.w) return 0;
+    if (A.W) { set_error("band clear: the compact layout has no storage left of the band"); return GPMC_EINVAL; }
     static int sms = 0;
     if (sms == 0) {
         int dev = 0;
@@ -376,6 +376,8 @@ int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P,
     static_assert(AT == ENV_ROWS, "one tile row block is one envelope block");
     if (env.blk && (env.n != N || env.ld < env_blocks(N))) { set_error("cov_assemble: envelope n=%d ld=%d for N=%d", env.n, env.ld, N); return GPMC_EINVAL; }
     if (band.w && (!(flags & GPMC_ASM_LOWER_ONLY) || band.width < 0)) { set_error("cov_assemble: band needs the lower-only assembly"); return GPMC_EINVAL; }
+    // the compact layout stores the band only: its tiles are all the assembly may write
+    if (A.W && (!band.w || band.clear || A.n != N)) { set_error("cov_assemble: the compact layout needs the band grid without a clear"); return GPMC_EINVAL; }
     const int nt = (N + AT - 1) / AT;
     dim3 grid(band.w && !band.clear ? nt * (std::min(band.width, nt - 1) + 1) : (nt * (nt + 1) / 2 + ASM_TPC - 1) / ASM_TPC, B);
     prof_begin(KC_ASSEMBLE, s);

@@ -16,7 +16,8 @@ template <int FM, int FN, int BM_, int BN_>
 __device__ __forceinline__ void gemm_epilogue(const GemmArgs &p, int m, int tm, int tn, int wm, int wn, int frow, int fk,
                                               int rows_valid, int cols_valid, double (&acc)[FM][FN][2])
 {
-    double *Cb = p.C.base + (size_t)m * p.C.stride;
+    // the C tile's rows lie in one 128-row block: one row stride p.C.ld in either layout of BatchView
+    double *Cb = view_elem(p.C, m, p.cr0 + tm * BM_, p.cc0 + tn * BN_);
     const int ldc = p.C.ld;
     const double *sv = (p.epi == EPI_R) ? p.svec + (size_t)m * p.stride_s : nullptr;
 #pragma unroll
@@ -24,7 +25,7 @@ __device__ __forceinline__ void gemm_epilogue(const GemmArgs &p, int m, int tm, 
         const int rl = wm * FM * 8 + i * 8 + frow;
         if (rl >= rows_valid) continue;
         const int gr = p.cr0 + tm * BM_ + rl;
-        double *crow = Cb + (size_t)gr * ldc + p.cc0 + tn * BN_;
+        double *crow = Cb + (size_t)rl * ldc;
         const double s_r = sv ? sv[gr] : 0.0;
 #pragma unroll
         for (int j = 0; j < FN; ++j) {

@@ -109,12 +109,15 @@ gemm_dmma_tma_kernel(GemmArgs p, const __grid_constant__ CUtensorMap tmA, const 
 
     const int arow = p.ar0 + tm * TBM, brow = p.br0 + tn * TBN;
     const int ak = p.k0 + koff, bk = p.bk0 + koff;
+    // compact layout (A = B = C): a box's rows lie in one 128-row block, its column coordinate is relative to that block's
+    // first stored column
+    const int acol = p.C.W ? ak - band_col0(arow, p.C.W) : ak, bcol = p.C.W ? bk - band_col0(brow, p.C.W) : bk;
     auto issue = [&](int chunk) {
         const int s = chunk % TSTAGES;
         unsigned char *st = smem + s * STAGE_BYTES;
         mbar_expect_tx(&full[s], STAGE_BYTES);
-        tma_load_3d(st, &tmA, &full[s], ak + chunk * TBK, arow, m);
-        tma_load_3d(st + A_BYTES, &tmB, &full[s], bk + chunk * TBK, brow, m);
+        tma_load_3d(st, &tmA, &full[s], acol + chunk * TBK, arow, m);
+        tma_load_3d(st + A_BYTES, &tmB, &full[s], bcol + chunk * TBK, brow, m);
     };
     if (tid == 0)      // lock step: one stage stays free for the refill; free running: all stages start full
         for (int s = 0; s < (FREE_RUNNING ? TSTAGES : TSTAGES - 1) && s < nk; ++s) issue(s);
@@ -123,7 +126,7 @@ gemm_dmma_tma_kernel(GemmArgs p, const __grid_constant__ CUtensorMap tmA, const 
     // end of the K loop do not wait for HBM -- matters for the short contractions only (K = 128 parts of the look-ahead,
     // N = 512 matrices: +1 ... 1.5 %; long contractions hide the epilogue behind the co-resident CTA anyway)
     if ((p.epi == EPI_SUB || p.epi == EPI_ADD) && klen <= 512) {
-        const double *Cb = p.C.base + (size_t)m * p.C.stride + (size_t)(p.cr0 + tm * TBM) * p.C.ld + p.cc0 + tn * TBN;
+        const double *Cb = view_elem(p.C, m, p.cr0 + tm * TBM, p.cc0 + tn * TBN);
 #pragma unroll
         for (int e = tid; e < TBM * (TBN / 16); e += TTHREADS) {
             const int r = e / (TBN / 16), c = (e % (TBN / 16)) * 16;
@@ -158,7 +161,7 @@ gemm_dmma_tma_kernel(GemmArgs p, const __grid_constant__ CUtensorMap tmA, const 
         // one real row in the 8-row A fragment (read straight from global memory, one chunk ahead), B fragments
         // from the staged tile -- 8 DMMAs per k step instead of none.
         const bool duty = p.border_row > 0 && wm == 0 && wn == 1 && (p.cr0 + tm * TBM == p.cc0 + (tn * TBN) / TBM * TBM);
-        const double *zrow = p.A.base + (size_t)m * p.A.stride + (size_t)p.border_row * p.A.ld + ak;
+        const double *zrow = view_elem(p.C, m, p.border_row, ak);      // (A == C: the launcher checks)
         const int kq = (fk >> 1) * 8 + (fk & 1);        // this lane's k inside a chunk at step ks: kq + 2 ks (the permuted order)
         double bacc[8][2];
 #pragma unroll
@@ -197,7 +200,7 @@ gemm_dmma_tma_kernel(GemmArgs p, const __grid_constant__ CUtensorMap tmA, const 
             }
         }
         if (duty && frow == 0) {
-            double *crow = p.C.base + (size_t)m * p.C.stride + (size_t)p.border_row * p.C.ld + p.cc0 + tn * TBN;
+            double *crow = view_elem(p.C, m, p.border_row, p.cc0 + tn * TBN);
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 const int cl = j * 8 + fk * 2;
@@ -566,6 +569,16 @@ int launch_gemm_tma(const GemmArgs &a, int B, int kclass, bool free_running, cud
     }
     CUtensorMap tmA, tmB;
     // rows at or beyond (origin + extent) are out of bounds for the TMA unit -> zero fill
+    if (a.C.W) {
+        // compact layout: only the one-tile kernel of the Cholesky updates knows it (A = B = C, envelope exits before any
+        // access outside the band, boxes and C tiles inside one 128-row block)
+        if (persistent || !free_running || a.A.base != a.C.base || a.B.base != a.C.base || !a.env.blk ||
+            a.k_follow_row || a.epi != EPI_SUB || a.A.ld != a.C.W || a.B.ld != a.C.W || a.ar0 % BAND_ROWS || a.br0 % BAND_ROWS ||
+            a.cr0 % BAND_ROWS) {
+            set_error("gemm: the compact band layout is supported by the Cholesky updates of the one-tile kernel only");
+            return GPMC_EINVAL;
+        }
+    }
     if ((rc = make_map(&tmA, a.A, a.ar0 + a.rows, TBM))) return rc;
     if ((rc = make_map(&tmB, a.B, a.br0 + a.cols, TBN))) return rc;
     const int tiles_m = (a.rows + TBM - 1) / TBM;

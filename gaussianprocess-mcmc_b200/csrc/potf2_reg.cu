@@ -129,7 +129,7 @@ potf2_reg_kernel(BatchView A, int n, int j0, double *__restrict__ W, long long s
     const int item = blockIdx.x;
     if (A.count && item >= *A.count) return;
     const int m = batch_item(A, item);
-    double *Ab = A.base + (size_t)m * A.stride + (size_t)j0 * A.ld + j0;
+    double *Ab = view_elem(A, m, j0, j0);        // the diagonal block: one 128-row block, row stride A.ld in either layout
     double *Wb = W + (size_t)m * strideW;
     const int ld = A.ld;
     const int nv = min(NB, n - j0);
@@ -351,6 +351,7 @@ int launch_panel_fused(BatchView A, int n, int n_rows, int j0, double *W, long l
 {
     if (B <= 0) return 0;
     if ((A.ld & 1) || (j0 & 1)) { set_error("panel: ld=%d j0=%d must be even", A.ld, j0); return GPMC_EALIGN; }
+    if (A.W) { set_error("panel: the fused panel kernel does not take the compact band layout"); return GPMC_EINVAL; }
     static DeviceOnce attr_set;
     if (attr_set.first()) GPMC_CUDA_CHECK(cudaFuncSetAttribute(potf2_reg_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM));
     prof_begin(KC_POTF2, s);

@@ -264,9 +264,24 @@ int potrf_fuse_auto(int n, int B, int border_rows)
     return (B >= 4 * sm_count() && n + border_rows <= 1664) ? 1 : 0;
 }
 
+// The compact band layout (BatchView::W) is known to the envelope-aware update tile kernel, the register-resident panel
+// factor and the 8-column panel solve, not to the fused panel kernels.  The layout is chosen for waves that run the plain
+// left-looking schedule; the jitter ladder's retries of a few items may run windows and look-ahead on it (every update
+// tile there also starts at the envelope and leaves before touching C when its contraction is empty).
+static bool compact_kernels() { return NB == BAND_ROWS && g_trsm_mode == 0 && g_potf2_mode == 0; }
+bool potrf_compact_ok(int n, int B, int border_rows)
+{
+    const int Bs = schedule_batch(B);
+    return compact_kernels() && potrf_window_for(n, Bs) == 0 && g_lookahead_mode != 2 && !potrf_fuse_auto(n, B, border_rows);
+}
+
 int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long strideW, long long w_step,
                    int zero_upper_flag, cudaStream_t s, int border_rows, int fuse, Envelope env)
 {
+    if (A.W && (fuse || border_rows != 1 || w_step || zero_upper_flag || !env.blk || !compact_kernels())) {
+        set_error("potrf_sequence: the compact band layout needs the envelope-aware kernels and one border row");
+        return GPMC_EINVAL;
+    }
     if (fuse && (!lite_panels() || (g_potf2_mode != 0 && g_potf2_mode != 3))) { set_error("potrf_sequence: fused panels need the default panel kernels"); return GPMC_EINVAL; }
     if (border_rows < 0) { set_error("potrf_sequence: border_rows < 0"); return GPMC_EINVAL; }
     const int nr = n + border_rows;                     // rows that take part in the panel solves
@@ -408,20 +423,21 @@ int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long st
 }
 
 // ------------------------------------------------------------------ border row (right-hand side carried as row n)
-__global__ void border_set_kernel(BatchView A, int n, const double *__restrict__ rhs, int ldv)
+__global__ void border_set_kernel(BatchView A, int n, const double *__restrict__ rhs, int ldv, int len)
 {
     const int b = blockIdx.y;
     if (A.count && b >= *A.count) return;
     const int m = batch_item(A, b);
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < A.ld) A.base[(size_t)m * A.stride + (size_t)n * A.ld + i] = (i < n) ? rhs[(size_t)m * ldv + i] : 0.0;
+    if (i < len) *view_elem(A, m, n, i) = (i < n) ? rhs[(size_t)m * ldv + i] : 0.0;
 }
 
 int border_set(BatchView A, int n, const double *rhs, int ldv, int B, cudaStream_t s)
 {
     if (B <= 0) return 0;
+    const int len = A.W ? (int)A.border_stride : A.ld;     // the row padded to the dense leading dimension
     prof_begin(KC_VEC, s);
-    border_set_kernel<<<dim3((A.ld + 255) / 256, B), 256, 0, s>>>(A, n, rhs, ldv);
+    border_set_kernel<<<dim3((len + 255) / 256, B), 256, 0, s>>>(A, n, rhs, ldv, len);
     prof_end(KC_VEC, s);
     GPMC_LAUNCH_CHECK();
     return 0;
@@ -433,7 +449,7 @@ __global__ void border_get_kernel(BatchView A, int n, double *__restrict__ z, in
     if (A.count && b >= *A.count) return;
     const int m = batch_item(A, b);
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) z[(size_t)m * ldv + i] = (info && info[m] != 0) ? nan("") : A.base[(size_t)m * A.stride + (size_t)n * A.ld + i];
+    if (i < n) z[(size_t)m * ldv + i] = (info && info[m] != 0) ? nan("") : *view_elem(A, m, n, i);
 }
 
 int border_get(BatchView A, int n, double *z, int ldv, const int *info, int B, cudaStream_t s)
@@ -449,19 +465,18 @@ int border_get(BatchView A, int n, double *z, int ldv, const int *info, int B, c
 int border_finish(BatchView A, int n, double *loglik, const int *info, int B, cudaStream_t s, int solved)
 {
     if (B <= 0) return 0;
-    if (solved) {
-        // the fused panel launches solved the border row through the last block column as well
-        if (A.stride > 0x7fffffffLL) { set_error("border_finish: item stride %lld does not fit the vector stride", A.stride); return GPMC_EINVAL; }
-        return loglik ? launch_quad_logdet(A, n, A.base + (size_t)n * A.ld, (int)A.stride, loglik, info, B, s) : 0;
-    }
-    if (A.stride > 0x7fffffffLL) { set_error("border_finish: item stride %lld does not fit the vector stride", A.stride); return GPMC_EINVAL; }
+    const long long bstride = view_border_stride(A);
+    if (bstride > 0x7fffffffLL) { set_error("border_finish: item stride %lld does not fit the vector stride", bstride); return GPMC_EINVAL; }
+    double *row = view_elem(A, 0, n, 0);                // item m's border row = row + m * bstride
+    // the fused panel launches solved the border row through the last block column as well
+    if (solved) return loglik ? launch_quad_logdet(A, n, row, (int)bstride, loglik, info, B, s) : 0;
     const int j0 = (n - 1) / NB * NB;                   // last block column: its part of the row is updated, not solved
     const int nv = n - j0;
-    double *row = A.base + (size_t)n * A.ld;            // item m's border row = row + m * stride
-    BatchView D{A.base + (size_t)j0 * A.ld + j0, A.stride, A.ld, A.map, A.count};
-    int rc = launch_solve_reduce(D, nv, row + j0, nullptr, (int)A.stride, row + j0, nullptr, info, B, s);
+    // the last diagonal block as a dense view (its rows share one row stride in either layout)
+    BatchView D{view_elem(A, 0, j0, j0), A.stride, A.ld, A.map, A.count};
+    int rc = launch_solve_reduce(D, nv, row + j0, nullptr, (int)bstride, row + j0, nullptr, info, B, s);
     if (rc || !loglik) return rc;
-    return launch_quad_logdet(A, n, row, (int)A.stride, loglik, info, B, s);
+    return launch_quad_logdet(A, n, row, (int)bstride, loglik, info, B, s);
 }
 
 // U = L^-T, built block column by block column in the upper triangle of the same buffer:

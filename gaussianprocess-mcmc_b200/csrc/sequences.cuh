@@ -22,6 +22,9 @@ namespace gpmc {
 int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long strideW, long long w_step,
                    int zero_upper, cudaStream_t s, int border_rows = 0, int fuse = 0, Envelope env = {});
 int potrf_fuse_auto(int n, int B, int border_rows);
+// potrf_sequence of B matrices of order n would run the plain left-looking schedule with the kernels that know the compact
+// band layout (BatchView::W)
+bool potrf_compact_ok(int n, int B, int border_rows);
 
 // One wave of assemble-and-factor with the pyGPs jitter ladder (capi.cu); shared by the log-lik unit, the predictive
 // path and the elliptical slice sampler's Cholesky draw.

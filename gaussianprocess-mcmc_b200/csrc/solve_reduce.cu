@@ -185,12 +185,11 @@ quad_logdet_kernel(BatchView L, int n, const double *__restrict__ z, int ldv, do
     const int m = batch_item(L, b);
     __shared__ double rq[8], rl[8];
     if (info && info[m] != 0) { if (threadIdx.x == 0) loglik[m] = nan(""); return; }
-    const double *Lb = L.base + (size_t)m * L.stride;
     double q = 0.0, ld = 0.0;
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
         const double zi = z[(size_t)m * ldv + i];
         q = fma(zi, zi, q);
-        ld += log(Lb[(size_t)i * L.ld + i]);
+        ld += log(*view_elem(L, m, i, i));
     }
     q = warp_sum(q); ld = warp_sum(ld);
     if ((threadIdx.x & 31) == 0) { rq[threadIdx.x >> 5] = q; rl[threadIdx.x >> 5] = ld; }

@@ -76,11 +76,10 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
         for (int i = blockIdx.x; i < nlaunch && !any; i += gridDim.x) any = !empty_block(blk_of(i));
         if (!any) return;
     }
-    double *Ab = A.base + (size_t)m * A.stride;
-    const int ld = A.ld;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int fr = lane >> 2, fk = lane & 3;
     const int ncv = min(NB, n_mat - j0);          // columns of this block column that exist (ragged last block: < NB)
+    const double *L11 = view_elem(A, m, j0, j0);  // the diagonal block: one 128-row block, row stride A.ld in either layout
 
     for (int e = tid; e < T8_NLB * 32 * 16; e += T8_THREADS) {        // 16 16-byte pieces per block row
         const int blk = e / (32 * 16), rem = e - blk * 32 * 16;
@@ -92,7 +91,7 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
         const int gr = j0 + bi * 32 + r, gc = j0 + bj * 32 + c2;
         if (gr < n_mat && gc < n_mat) {
             const unsigned dst = (unsigned)__cvta_generic_to_shared(dstp);
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(dst), "l"(Ab + (size_t)gr * ld + gc));
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(dst), "l"(L11 + (size_t)(gr - j0) * A.ld + (gc - j0)));
         } else {                                  // beyond the matrix (ragged last block solved for border rows): identity
             dstp[0] = (gr == gc) ? 1.0 : 0.0;
             dstp[1] = (gr == gc + 1) ? 1.0 : 0.0;
@@ -118,7 +117,7 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
     // rows this lane solves in row block rb
     auto row_ok = [&](int rb, int row0, int rows_valid) { return r_loc < rows_valid && (!border_only(rb) || row0 + r_loc >= env.n); };
     {
-        const double *grow0 = Ab + (size_t)(row0_first + min(r_loc, max(rv_first, 1) - 1)) * ld + j0 + 2 * fk;
+        const double *grow0 = view_elem(A, m, row0_first + min(r_loc, max(rv_first, 1) - 1), j0 + 2 * fk);
         const bool ok = row_ok(rb_first, row0_first, rv_first);
 #pragma unroll
         for (int b8 = 0; b8 < T8_NB8; ++b8) {
@@ -149,7 +148,7 @@ trsm_panel8_kernel(BatchView A, int n_rows, int j0, const double *__restrict__ W
     if (border_only(rb) && row0 + warp * 8 + 7 < env.n) continue;
     if (env.blk && empty_block(rb)) continue;
     const bool ok = row_ok(rb, row0, rows_valid);
-    double *grow = Ab + (size_t)(row0 + min(r_loc, max(rows_valid, 1) - 1)) * ld + j0 + 2 * fk;
+    double *grow = view_elem(A, m, row0 + min(r_loc, max(rows_valid, 1) - 1), j0 + 2 * fk);
     if (rb != rb_first) {
 #pragma unroll
         for (int b8 = 0; b8 < T8_NB8; ++b8) {

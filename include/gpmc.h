@@ -275,8 +275,17 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
  * key 16: where the band's key 15 stores the +0 left of the band, which nothing on the factorisation path reads: 2 = inline
  *        in the assembly (default), 1 = on a low-priority side stream beside the factorisation (measured slower on the
  *        bench workload: the stores compete with the band's assembly), 0 = not at all (the workspace keeps what it held
- *        there; results are unchanged).  GPMC_BAND_CLEAR=<value> presets it. */
+ *        there; results are unchanged).  GPMC_BAND_CLEAR=<value> presets it.
+ * key 17: compact band storage (with key 15 on): 1 = automatic (default): when the dense layout would need several waves,
+ *        the band of every item of the call is bounded first and, if rows of W = 128 + 64 * (widest band) columns need
+ *        fewer waves that run the plain left-looking schedule, each row keeps only those W columns (nothing left of the
+ *        band is written or cleared; results are bit-identical); 0 = always the dense layout.  GPMC_BAND_COMPACT=0
+ *        presets it to 0.  One item with a wide band (non-finite input, a huge length-scale) makes the whole call dense. */
 int gpmc_set_tuning(int key, int value);
+
+/* Layout the last gpmc_loglik_batched / gpmc_loglik_host call used: *band_W = 0 for the dense layout, else the row width
+ * of the compact band layout (key 17); *waves = the number of waves the call's items were factored in. */
+int gpmc_loglik_layout(int *band_W, int *waves);
 
 /* FP64 micro-benchmarks used by bench.py to put a measured peak beside the roofline:
  * register-resident DMMA (mma.sync m8n8k4 f64) and DFMA loops over the whole chip. */

@@ -1,7 +1,8 @@
-"""Band-only assembly and launches on vs. off (gpmc_set_tuning(15, .)) on the bench.py workload, with the region left of
-the band cleared inline in the assembly (gpmc_set_tuning(16, 2), default) or on a side stream (16, 1): ms per step, per
-class kernel ms per step, launched vs. working CTAs of the assembly, the update GEMM and the panel solve, and a bitwise
-comparison of loglik and info with the envelope-only run.
+"""Band-only assembly and launches on vs. off (gpmc_set_tuning(15, .)) on the bench.py workload, in the dense layout with
+the region left of the band cleared inline in the assembly (gpmc_set_tuning(16, 2)) or on a side stream (16, 1), and in
+the compact band layout (gpmc_set_tuning(17, 1), default: only the band's columns are stored, all chains in fewer waves):
+ms per step, per class kernel ms per step, waves and row width W of each arm, launched vs. working CTAs of the assembly,
+the update GEMM and the panel solve, and a bitwise comparison of loglik and info with the envelope-only run.
 
 The CTA counts replay the plain left-looking schedule of sequences.cu (the one the bench workload runs) on the envelopes,
 band starts w and wave bands the device wrote (read back from gpmc_loglik_batched's workspace, wave by wave).  A CTA
@@ -96,9 +97,18 @@ def work_counts(waves, n, band_on):
     return c
 
 
-def per_step_ms(x, G, H, band, clear, steps):
+def layout():
+    """(row width W of the compact layout or 0 for dense, waves) of the last call"""
+    import ctypes
+    W, waves = ctypes.c_int(-1), ctypes.c_int(-1)
+    gp._lib.load().gpmc_loglik_layout(ctypes.byref(W), ctypes.byref(waves))
+    return W.value, waves.value
+
+
+def per_step_ms(x, G, H, band, clear, compact, steps):
     gp.ops.set_tuning(15, band)
     gp.ops.set_tuning(16, clear)
+    gp.ops.set_tuning(17, compact)
     try:
         for _ in range(2):
             ll, info = gp.ops.loglik_batched(x, G, H)
@@ -110,15 +120,17 @@ def per_step_ms(x, G, H, band, clear, steps):
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / steps
+        lay = layout()
         gp.ops.profile(True)                    # per-class times in a run of their own (the events slow the host)
         for _ in range(steps):
             gp.ops.loglik_batched(x, G, H)
         prof = gp.ops.profile_read()
         gp.ops.profile(False)
-        return ms, {k: v[0] / steps for k, v in prof.items() if v[1] > 0}, ll.cpu().numpy(), info.cpu().numpy()
+        return ms, {k: v[0] / steps for k, v in prof.items() if v[1] > 0}, ll.cpu().numpy(), info.cpu().numpy(), lay
     finally:
         gp.ops.set_tuning(15, 1)
         gp.ops.set_tuning(16, 2)
+        gp.ops.set_tuning(17, 1)
 
 
 def main():
@@ -136,14 +148,22 @@ def main():
     ws_bytes = lib.gpmc_workspace_bytes(gp._lib.OP_LOGLIK, n, 1, B)
     per_item = lib.gpmc_workspace_bytes(gp._lib.OP_LOGLIK, n, 1, 2) - lib.gpmc_workspace_bytes(gp._lib.OP_LOGLIK, n, 1, 1)
     wave = min(B, ws_bytes // per_item)
-    waves = band_data(x, G, H, wave)
-    arms = (('band_off', 0, 1), ('band_on_side_clear', 1, 1), ('band_on_inline_clear', 1, 2))
-    res = {k: [] for k, _, _ in arms}
+    gp.ops.set_tuning(17, 0)                    # the dense layout's workspace contents, wave by wave
+    try:
+        waves = band_data(x, G, H, wave)
+    finally:
+        gp.ops.set_tuning(17, 1)
+    # the compact layout factors every chain in one wave (when it fits) with the call's widest band
+    one = [(np.concatenate([w[0] for w in waves]), np.concatenate([w[1] for w in waves]),
+            max(w[2] for w in waves), max(w[3] for w in waves))]
+    arms = (('band_off', 0, 1, 0), ('band_on_side_clear', 1, 1, 0), ('band_on_inline_clear', 1, 2, 0),
+            ('band_compact', 1, 2, 1))
+    res = {k: [] for k, _, _, _ in arms}
     outs = {}
     for _ in range(a.rounds):
-        for label, band, clear in arms:
-            ms, cls, ll, info = per_step_ms(x, G, H, band, clear, a.steps)
-            res[label].append({'ms_per_step': ms, 'kernel_ms_per_step': cls})
+        for label, band, clear, compact in arms:
+            ms, cls, ll, info, lay = per_step_ms(x, G, H, band, clear, compact, a.steps)
+            res[label].append({'ms_per_step': ms, 'kernel_ms_per_step': cls, 'band_W': lay[0], 'waves': lay[1]})
             outs[label] = (ll, info)
     gp.ops.set_tuning(14, 0)
     try:
@@ -155,7 +175,8 @@ def main():
     row = {'n': n, 'chains': B, 'wave': int(wave), 'steps': a.steps,
            'wave_bands': [{'launch_band_blocks': w[2], 'assembly_band_tiles': w[3]} for w in waves],
            'work_band_off': work_counts(waves, n, False), 'work_band_on': work_counts(waves, n, True),
-           'outputs_bitwise_equal_to_band_off': {k: same(outs[k], outs['band_off']) for k, _, _ in arms},
+           'work_band_compact': work_counts(one, n, True),
+           'outputs_bitwise_equal_to_band_off': {k: same(outs[k], outs['band_off']) for k, _, _, _ in arms},
            'band_off_bitwise_equal_to_dense': same(outs['band_off'], dense),
            'arms': res}
     print(json.dumps(row))
