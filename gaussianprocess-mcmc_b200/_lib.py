@@ -14,9 +14,9 @@ KIND_SE_ISO, KIND_SE_ARD = 0, 1
 ASM_ADD_S, ASM_LOWER_ONLY = 1, 2
 JITTER_NONE, JITTER_PYGPS = 0, 1
 INFO_NOT_PD = -1
-OP_POTRF, OP_LOGLIK, OP_SDS = 1, 2, 3
+OP_POTRF, OP_LOGLIK, OP_SDS, OP_LOGLIK_GRAD = 1, 2, 3, 4
 KC_NAMES = ('assemble', 'gemm_update', 'potf2', 'panel_trsm', 'solve_reduce', 'tri_inverse', 'syrk_R', 'vector_control',
-            'band_clear')
+            'band_clear', 'grad_contract')
 
 _c_double_p = ctypes.c_void_p     # raw addresses (torch data_ptr() / numpy ctypes.data)
 _vp = ctypes.c_void_p
@@ -33,6 +33,7 @@ SIGNATURES = {
     'gpmc_cov_assemble': (_i, [_vp, _i, _i, _vp, _i, _i, _i, _i, _vp, _vp, _i, _vp]),
     'gpmc_potrf_batched': (_i, [_vp, _i, _i, _i, _vp, _i, _i, _vp, _sz, _vp]),
     'gpmc_loglik_batched': (_i, [_vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
+    'gpmc_loglik_grad_batched': (_i, [_vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     'gpmc_loglik_host': (_i, [_vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _vp, _vp]),
     'gpmc_sds_workspace_bytes': (_sz, [_i, _i, _i]),
     'gpmc_sds_sweep': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _i,

@@ -113,7 +113,7 @@ bool envelope_enabled()
 // (gpmc_set_tuning(16, .), GPMC_BAND_CLEAR): 2 = inline in the assembly (default: measured faster on the bench workload,
 // profiles/r03b_band_ab.json), 1 = side stream, 0 = not at all
 static int g_band = -1, g_band_clear = -1, g_band_compact = -1;
-static bool band_enabled()
+bool band_enabled()
 {
     if (g_band < 0) {
         const char *e = getenv("GPMC_BAND");
@@ -183,11 +183,13 @@ struct ClearJoin {
 // rows; `diag_value` is the (constant) diagonal of an item's matrix from its hyper-parameter row.
 int factor_wave(const std::function<int(BatchView, int, const double *)> &fill, const std::function<double(const double *)> &diag_value,
                 BatchView A, int N, int nb, const double *hyp_w, int P, int *info_w, double *W, double *jit_dev, int *map_dev,
-                int jitter_policy, int border_rows, cudaStream_t s, int fuse, Envelope env)
+                int jitter_policy, int border_rows, cudaStream_t s, int fuse, Envelope env, long long w_step)
 {
+    // w_step = NB*NB keeps every diagonal-block inverse (item stride: all block columns' worth), as inverse_sequence needs
+    const long long strideW = w_step ? (long long)((N + NB - 1) / NB) * w_step : NB * NB;
     int rc = fill(A, nb, nullptr);
     if (rc) return rc;
-    if ((rc = potrf_sequence(A, N, nb, info_w, W, NB * NB, 0, 0, s, border_rows, fuse, env))) return rc;
+    if ((rc = potrf_sequence(A, N, nb, info_w, W, strideW, w_step, 0, s, border_rows, fuse, env))) return rc;
     if (jitter_policy != GPMC_JITTER_PYGPS) return 0;
     std::vector<int> info(nb);
     GPMC_CUDA_CHECK(cudaMemcpyAsync(info.data(), info_w, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -216,7 +218,7 @@ int factor_wave(const std::function<int(BatchView, int, const double *)> &fill, 
         Am.map = map_dev;
         Am.count = nullptr;
         if ((rc = fill(Am, nf, jit_dev))) return rc;
-        if ((rc = potrf_sequence(Am, N, nf, info_w, W, NB * NB, 0, 0, s, border_rows, fuse, env))) return rc;
+        if ((rc = potrf_sequence(Am, N, nf, info_w, W, strideW, w_step, 0, s, border_rows, fuse, env))) return rc;
         GPMC_CUDA_CHECK(cudaMemcpyAsync(info.data(), info_w, nb * sizeof(int), cudaMemcpyDeviceToHost, s));
         GPMC_CUDA_CHECK(cudaStreamSynchronize(s));
         std::vector<int> still;
@@ -254,7 +256,6 @@ int gpmc_device_info(int *sm_count, int *cc_major, int *cc_minor, size_t *hbm_by
 
 size_t gpmc_workspace_bytes(int op, int N, int D, int B)
 {
-    (void)D;
     if (N <= 0 || B <= 0) return 0;
     const size_t w = (size_t)NB * NB * sizeof(double);
     if (op == GPMC_OP_POTRF) {
@@ -271,6 +272,7 @@ size_t gpmc_workspace_bytes(int op, int N, int D, int B)
         size_t wave = std::min<size_t>(std::min<size_t>(B, 8192), std::max<size_t>(1, cap / l.per_item_bytes));
         return l.fixed_bytes + wave * l.per_item_bytes;
     }
+    if (op == GPMC_OP_LOGLIK_GRAD) return loglik_grad_workspace_bytes(N, D, B);
     return 0;
 }
 

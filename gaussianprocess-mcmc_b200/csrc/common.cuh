@@ -17,7 +17,7 @@ constexpr int MAX_BATCH_ITEMS = 32768;   // batch items of one launch ride in gr
 
 // kernel classes for the profiling hooks (gpmc_profile_read)
 enum KernelClass { KC_ASSEMBLE = 0, KC_GEMM = 1, KC_POTF2 = 2, KC_TRSM = 3, KC_SOLVE = 4, KC_INV = 5, KC_SYRK_R = 6, KC_VEC = 7,
-                   KC_CLEAR = 8, KC_COUNT = 9 };
+                   KC_CLEAR = 8, KC_GRAD = 9, KC_COUNT = 10 };
 
 void set_error(const char *fmt, ...);
 // Every computing entry point of the C ABI takes this (recursive) lock: the library keeps per-process state (side streams,
@@ -165,6 +165,15 @@ int launch_band_bound(const double *x, int N, int D, const double *hyp, int P, i
                       int *band_out, double *xbox, cudaStream_t s);
 // +0 into every element of rows 0 .. N-1 of items 0 .. B-1 left of their row block's w (store only, small grid)
 int launch_band_clear(BatchView A, int N, Band band, int B, cudaStream_t s);
+
+// grad_contract.cu : the contraction of gpmc_loglik_grad_batched for items 0 .. B-1 (item stride strideW / ldv / ldw):
+//   grad[b][p] = 0.5 sum_ij (alpha_i alpha_j - W_ij) dA_ij/dtheta_p  from the lower triangle of W (row stride ldW),
+//   K_ij recomputed from x and hyp with cov_assemble's expression.  band_w != nullptr: row block r of item b reads only the
+//   64-column tiles from band_w[b * ldw + r] on (left of them K_ij is +0).  partial: scratch of B * env_blocks(N) * P
+//   doubles.  Items with info != 0, or a parameter that is not a positive finite number, get a NaN row.
+int launch_grad_contract(const double *x, int N, int D, const double *hyp, int P, int n_ell, const double *alpha, int ldv,
+                         const double *W, int ldW, long long strideW, const int *band_w, int ldw, const int *info,
+                         double *partial, double *grad, int B, cudaStream_t s);
 
 // gemm_dmma.cu :  C[i][j] (op)= sum_k A[i][k] * B[j][k]   ("NT": both operands K-contiguous, row-major)
 struct Operand {

@@ -29,11 +29,15 @@ bool potrf_compact_ok(int n, int B, int border_rows);
 // One wave of assemble-and-factor with the pyGPs jitter ladder (capi.cu); shared by the log-lik unit, the predictive
 // path and the elliptical slice sampler's Cholesky draw.
 // env: the envelope `fill` writes for the items it assembles (see potrf_sequence)
+// w_step: as potrf_sequence's (0: one scratch block per item; NB*NB: every diagonal-block inverse kept, W holds
+// (N+NB-1)/NB blocks per item)
 int factor_wave(const std::function<int(BatchView, int, const double *)> &fill, const std::function<double(const double *)> &diag_value,
                 BatchView A, int N, int nb, const double *hyp_w, int P, int *info_w, double *W, double *jit_dev, int *map_dev,
-                int jitter_policy, int border_rows, cudaStream_t s, int fuse = 0, Envelope env = {});
+                int jitter_policy, int border_rows, cudaStream_t s, int fuse = 0, Envelope env = {}, long long w_step = 0);
 // the envelope skips are on unless gpmc_set_tuning(14, 0) or GPMC_ENVELOPE=0 forced the dense path
 bool envelope_enabled();
+// the band (with the envelope) is on unless gpmc_set_tuning(15, 0) or GPMC_BAND=0, and the selected kernels honour it
+bool band_enabled();
 
 // Write rhs[item] (length n, row stride ldv) into border row n of every item (zero padded up to ld).
 int border_set(BatchView A, int n, const double *rhs, int ldv, int B, cudaStream_t s);
@@ -52,6 +56,9 @@ void set_schedule_batch(int B);
 
 // R = S - S (U U^T) S + 1e-11 I, lower tiles only, from U (upper, in A) into Rm.  svec = diag(S) per item.
 int r_sequence(BatchView Rm, BatchView U, int n, int B, const double *svec, long long stride_s, cudaStream_t s);
+
+// gpmc_workspace_bytes(GPMC_OP_LOGLIK_GRAD, ...) (loglik_grad.cu)
+size_t loglik_grad_workspace_bytes(int N, int D, int B);
 
 // small helpers
 int fill_int(int *p, int v, int n, cudaStream_t s);

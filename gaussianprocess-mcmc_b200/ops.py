@@ -6,7 +6,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (KIND_SE_ISO, KIND_SE_ARD, ASM_ADD_S, ASM_LOWER_ONLY, JITTER_NONE, JITTER_PYGPS,
-                   OP_POTRF, OP_LOGLIK, GpmcError)
+                   OP_POTRF, OP_LOGLIK, OP_LOGLIK_GRAD, GpmcError)
 
 
 def _stream_ptr(torch):
@@ -136,6 +136,47 @@ def loglik_batched(x, g, hyp, jitter_policy=JITTER_PYGPS, workspace=None, max_wa
                                  out.data_ptr(), info.data_ptr(), ws.data_ptr(), use_bytes, _stream_ptr(torch))
     _lib.check(rc, 'gpmc_loglik_batched')
     return out, info
+
+
+def loglik_grad_batched(x, g, hyp, jitter_policy=JITTER_PYGPS, workspace=None, max_wave=None):
+    """``log N(g_b; 0, K(hyp_b) + sn_b^2 I)`` and its gradient with respect to the natural-scale row ``hyp[b] = (ell..,
+    sf, sn)``; returns ``(loglik[B], grad[B,P], info[B])`` CUDA tensors (``gpmc_loglik_grad_batched``, include/gpmc.h).
+
+    ``max_wave`` limits the items factored at once (the workspace is sized for that many)."""
+    torch = _lib.require_cuda()
+    lib = _lib.load()
+    x = _f64_cuda(torch, x, 'x')
+    if x.dim() == 1:
+        x = x.reshape(-1, 1)
+    g = _f64_cuda(torch, g, 'g')
+    hyp = _f64_cuda(torch, hyp, 'hyp')
+    if g.dim() == 1:
+        g = g.reshape(1, -1)
+    if hyp.dim() == 1:
+        hyp = hyp.reshape(1, -1)
+    N, D = x.shape
+    B, P = hyp.shape
+    if g.shape != (B, N):
+        raise ValueError('g must be [B=%d, N=%d], got %s' % (B, N, tuple(g.shape)))
+    out = torch.empty((B,), dtype=torch.float64, device='cuda')
+    grad = torch.empty((B, P), dtype=torch.float64, device='cuda')
+    info = torch.empty((B,), dtype=torch.int32, device='cuda')
+    if B == 0:
+        return out, grad, info
+    wsobj = workspace or _default_ws
+    need = lib.gpmc_workspace_bytes(OP_LOGLIK_GRAD, N, D, B if max_wave is None else min(B, max_wave))
+    have = 0 if wsobj.buf is None else wsobj.buf.numel()
+    if max_wave is None and have < need:
+        free, _ = torch.cuda.mem_get_info()
+        one = lib.gpmc_workspace_bytes(OP_LOGLIK_GRAD, N, D, 1)
+        need = max(one, min(need, (free + have) * 6 // 10))
+    ws = wsobj.get(torch, need)
+    use_bytes = need if max_wave is not None else ws.numel()
+    rc = lib.gpmc_loglik_grad_batched(x.data_ptr(), N, D, g.data_ptr(), hyp.data_ptr(), B, P, kind_of(D, P), jitter_policy,
+                                      out.data_ptr(), grad.data_ptr(), info.data_ptr(), ws.data_ptr(), use_bytes,
+                                      _stream_ptr(torch))
+    _lib.check(rc, 'gpmc_loglik_grad_batched')
+    return out, grad, info
 
 
 def loglik_host(x, g, hyp, jitter_policy=JITTER_PYGPS):

@@ -72,6 +72,7 @@ extern "C" {
 #define GPMC_OP_POTRF   1
 #define GPMC_OP_LOGLIK  2
 #define GPMC_OP_SDS     3
+#define GPMC_OP_LOGLIK_GRAD 4
 
 int gpmc_version(void);
 /* panel width (block-column width) of the blocked Cholesky this build was compiled with: 64 or 128 */
@@ -118,6 +119,32 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
                         int B, int P, int kind, int jitter_policy,
                         double *loglik_dev, int *info_dev,
                         void *ws_dev, size_t ws_bytes, void *stream);
+
+/*
+ * The log-lik unit above and its gradient with respect to the hyper-parameters, for B (theta, g) pairs -- what a type-II
+ * maximum-likelihood fit of theta (pyGPs 1.3.4 GPR.optimize, the reference's gpK.GPR at framework.py:158,208 and
+ * demoRegression.py:110-115) and any gradient-based sampler need.  With A = K(ell, sf) + sn^2 I (the S_ii of
+ * sliceSample.py:184-187 is differentiated as the sn^2 it equals):
+ *   loglik(theta)       = -(0.5 g^T A^-1 g + 0.5 log|A| + 0.5 N log 2 pi)      (loglik_dev[b], as gpmc_loglik_batched)
+ *   d loglik / d th_p   = 0.5 sum_ij (alpha_i alpha_j - W_ij) dA_ij/d th_p,   alpha = A^-1 g,  W = A^-1
+ *     dA_ij / d ell     = K_ij r2_ij / ell^3              (GPMC_KIND_SE_ISO, r2 = |x_i - x_j|^2)
+ *     dA_ij / d ell_d   = K_ij (x_id - x_jd)^2 / ell_d^3  (GPMC_KIND_SE_ARD)
+ *     dA_ij / d sf      = 2 K_ij / sf
+ *     dA / d sn         = 2 sn I              ->  sn (alpha.alpha - tr W)
+ * grad_dev[B,P] is taken with respect to the NATURAL-scale row hyp[b] = (ell.., sf, sn).  An item the jitter ladder
+ * rescued gets loglik and gradient of A + jitter I, the jitter held constant.  An item whose info != 0 after the ladder
+ * gets loglik = NaN and a row of NaN; so does the gradient of a row with a parameter that is not a positive finite
+ * number.  Arguments are checked as in gpmc_loglik_batched; B = 0 returns 0.  Items are processed in waves sized to the
+ * workspace (gpmc_workspace_bytes(GPMC_OP_LOGLIK_GRAD, N, D, B)): per item two N x N matrices (the factor with g as its
+ * border row, and W), the saved diagonal-block inverses of the factorisation and a few vectors.
+ * Pipeline per wave: assemble and factor (jitter ladder), z = L^-1 g and loglik, U = L^-T, alpha = U z, W = U U^T on the
+ * lower tiles that can meet K_ij != 0 (the band of tuning keys 14/15; outside it dA/dtheta is an exact zero), then one
+ * pass over those tiles that recomputes K_ij and contracts.  Repeated calls are bitwise identical.
+ */
+int gpmc_loglik_grad_batched(const double *x_dev, int N, int D, const double *g_dev, const double *hyp_dev,
+                             int B, int P, int kind, int jitter_policy,
+                             double *loglik_dev, double *grad_dev, int *info_dev,
+                             void *ws_dev, size_t ws_bytes, void *stream);
 
 /*
  * Same unit with HOST buffers (what a numpy caller holds): pinned staging, H2D of (x, g, hyp),
@@ -296,7 +323,8 @@ int gpmc_bench_dmma_ilp(int nacc, int warps_per_sm, int iters, double *tflops_ou
 
 /* Timing hooks: the library records CUDA-event durations of its own kernels per class
  * (0 assemble, 1 Cholesky update GEMM, 2 panel potf2, 3 panel trsm, 4 solve+reduce, 5 triangular inverse,
- *  6 posterior-covariance SYRK, 7 vector/control kernels)
+ *  6 posterior-covariance SYRK (and W = U U^T of gpmc_loglik_grad_batched), 7 vector/control kernels, 8 band clear,
+ *  9 gradient contraction of gpmc_loglik_grad_batched)
  * when enabled; used by bench.py for roofline.achieved. */
 /* Diagnostics of the last gpmc_sds_sweep on this thread: rounds queued, rounds that found nothing to do (queued past the
  * end), times the host-side jitter ladder had to run. */
