@@ -411,7 +411,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
             const int waves_c = wave_c > 0 ? (int)((B + wave_c - 1) / wave_c) : 0;
             // equal waves (sizes differ by one at most), so that every wave runs the same schedule
             const int nb_lo = waves_c > 0 ? B / waves_c : 0, nb_hi = waves_c > 0 ? (B + waves_c - 1) / waves_c : 0;
-            if (Wc < l.ld && waves_c > 0 && waves_c < g_last_waves && potrf_compact_ok(N, nb_lo, 1) && potrf_compact_ok(N, nb_hi, 1)) {
+            if (Wc < l.ld && waves_c > 0 && waves_c < g_last_waves && potrf_compact_ok(N, nb_lo) && potrf_compact_ok(N, nb_hi)) {
                 double *border = (double *)cp; cp += align_up((size_t)nb_hi * l.ld * sizeof(double), 256);
                 double *Wsc = (double *)cp; cp += (size_t)nb_hi * NB * NB * sizeof(double);
                 double *mats_c = (double *)cp;
@@ -431,7 +431,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
                         return border_set(V, N, g_w, N, nitems, s);
                     };
                     auto diag = [&](const double *h) { return host_diag_value(h, n_ell); };
-                    rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, Wsc, jit_dev, map_dev, jitter_policy, 1, s, 0, env);
+                    rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, Wsc, jit_dev, map_dev, jitter_policy, 1, s, potrf_fuse_compact(), env);
                     if (rc) return rc;
                     if ((rc = border_finish(A, N, loglik_dev + s0, info_w, nb, s, 0))) return rc;
                     s0 += nb;

@@ -230,9 +230,10 @@ int launch_potf2_flow(BatchView A, int n, int j0, double *W, long long strideW, 
 int launch_panel_fused_flow(BatchView A, int n, int n_rows, int j0, double *W, long long strideW, int *info, int zero_upper,
                             int B, cudaStream_t s);
 // potf2_reg.cu : panel factor AND panel solve of block column j0 in one launch (n_rows = n + border rows; in the last block
-// column the border rows are solved too) -- for many small matrices in flight
+// column the border rows are solved too) -- for many small matrices in flight.  Compact band layout (A.W > 0): one border
+// row, env required; only the rows trsm_panel8 would solve for env are solved, and the last block column solves none.
 int launch_panel_fused(BatchView A, int n, int n_rows, int j0, double *W, long long strideW, int *info, int zero_upper,
-                       int B, cudaStream_t s);
+                       int B, cudaStream_t s, Envelope env = {});
 void set_lookahead_mode(int mode); // potrf_sequence: 0 auto (few matrices in flight), 1 off, 2 on
 void set_potrf_window(int w);      // override the window of the windowed schedule (multiple of NB; 0 = default)
 void set_potf2_mode(int mode);     // 0: register-resident kernel (default), 3: the same as a dataflow program (no block barriers),

@@ -111,13 +111,58 @@ __device__ __forceinline__ void pick_slot(const double (&acc)[PR_SLOTS][2], int 
 // bytes per warp: conflict free), and after the 16 factor steps every warp takes 8 rows at a time through the same
 // inverse-multiply + refinement chain as trsm_panel8.cu.  With one CTA per matrix and two CTAs per SM, one matrix's
 // latency-bound factor steps overlap the other's DMMA-bound solve -- which separate launches cannot do: every CTA of a
-// launch is in the same phase.  Used when many small matrices are in flight (potrf_sequence decides).
+// launch is in the same phase.  Used when many small matrices are in flight (potrf_sequence decides), and for the compact
+// band layout, where every block column has only the band's few rows below its diagonal block.
 constexpr int PF_LC_ELEMS = (PR_NF * (PR_NF + 1) / 2) * 64;      // lower 8x8 blocks of L11: block (R, C) at R (R + 1) / 2 + C
 constexpr int PF_SMEM = (PF_LC_ELEMS + PR_NF * 64) * (int)sizeof(double);
 
+// Panel solve of one warp's 8 rows,  X L11^T = A21,  from L11 (Lc) and the 8x8 diagonal inverses (W8c) in shared memory:
+// the lane's row starts at grow (column j0 + 2 fk; rv: the row exists, else nothing is read or written), nv columns exist.
+// Sub-blocks b8 < b8s (warp-uniform) hold exact +0: their X is +0 and their updates of later sub-blocks add +-0, so the
+// chain starts at b8s and leaves them as stored.
+__device__ __forceinline__ void fused_solve8(double *grow, bool rv, int nv, int b8s, const double *Lc, const double *W8c,
+                                             int frag_off, int fk)
+{
+    double t[PR_NF][2];
+#pragma unroll
+    for (int b8 = 0; b8 < PR_NF; ++b8) {
+        double2 v = make_double2(0.0, 0.0);
+        if (rv && b8 >= b8s && b8 * 8 + 2 * fk < nv) v = *reinterpret_cast<const double2 *>(grow + b8 * 8);
+        t[b8][0] = v.x;
+        t[b8][1] = v.y;
+    }
+#pragma unroll
+    for (int b8 = 0; b8 < PR_NF; ++b8) {
+        if (b8 < b8s) continue;
+        const double2 wv = *reinterpret_cast<const double2 *>(&W8c[b8 * 64 + frag_off]);
+        const double2 lv = *reinterpret_cast<const double2 *>(&Lc[(b8 * (b8 + 1) / 2 + b8) * 64 + frag_off]);
+        double x0 = 0.0, x1 = 0.0;
+        dmma884_r(x0, x1, t[b8][0], wv.x);                                  // X0 = A W8^T
+        dmma884_r(x0, x1, t[b8][1], wv.y);
+        double r0 = t[b8][0], r1 = t[b8][1];
+        dmma884_r(r0, r1, -x0, lv.x);                                       // r = A - X0 L8^T
+        dmma884_r(r0, r1, -x1, lv.y);
+        dmma884_r(x0, x1, r0, wv.x);                                        // X = X0 + r W8^T
+        dmma884_r(x0, x1, r1, wv.y);
+        const double nx0 = -x0, nx1 = -x1;
+#pragma unroll
+        for (int bp = b8 + 1; bp < PR_NF; ++bp) {
+            const double2 lp = *reinterpret_cast<const double2 *>(&Lc[(bp * (bp + 1) / 2 + b8) * 64 + frag_off]);
+            dmma884_r(t[bp][0], t[bp][1], nx0, lp.x);
+            dmma884_r(t[bp][0], t[bp][1], nx1, lp.y);
+        }
+        if (rv) {
+            const int c = b8 * 8 + 2 * fk;
+            if (c + 1 < nv) *reinterpret_cast<double2 *>(grow + b8 * 8) = make_double2(x0, x1);
+            else if (c < nv) grow[b8 * 8] = x0;
+        }
+    }
+}
+
 template <bool FUSED>
 __global__ void __launch_bounds__(PR_THREADS, 2)
-potf2_reg_kernel(BatchView A, int n, int j0, double *__restrict__ W, long long strideW, int *__restrict__ info, int zero_upper, int n_rows)
+potf2_reg_kernel(BatchView A, int n, int j0, double *__restrict__ W, long long strideW, int *__restrict__ info, int zero_upper, int n_rows,
+                 Envelope env)
 {
     extern __shared__ __align__(16) double pf_dyn[];
     double *Lc = pf_dyn;                                 // FUSED only
@@ -281,7 +326,7 @@ potf2_reg_kernel(BatchView A, int n, int j0, double *__restrict__ W, long long s
     if (tid == 0 && s_fail != 0) {
         if (info[m] == 0) info[m] = s_fail;
     }
-    if (FUSED) {
+    if (FUSED && !A.W) {
         // ---------------------------------------------------------------- panel solve: X L11^T = A21 for the rows below
         // (trsm_panel8.cu's chain; a warp owns 8 rows x 128 columns as accumulator fragments, 64 rows per pass of the CTA)
         const int row_start = (j0 + NB < n) ? NB : n - j0;            // relative to the block's first row; last column: border rows only
@@ -290,40 +335,28 @@ potf2_reg_kernel(BatchView A, int n, int j0, double *__restrict__ W, long long s
         for (int row0 = row_start; row0 < rows_end; row0 += 8 * PR_WARPS) {
             if (row0 + w * 8 >= rows_end) continue;                     // warp-uniform
             const int r = row0 + w * 8 + fr;
-            const bool rv = r < rows_end;
-            double *grow = Ab + (size_t)min(r, rows_end - 1) * ld + 2 * fk;
-            double t[PR_NF][2];
-#pragma unroll
-            for (int b8 = 0; b8 < PR_NF; ++b8) {
-                double2 v = make_double2(0.0, 0.0);
-                if (rv && b8 * 8 + 2 * fk < nv) v = *reinterpret_cast<const double2 *>(grow + b8 * 8);
-                t[b8][0] = v.x;
-                t[b8][1] = v.y;
-            }
-#pragma unroll
-            for (int b8 = 0; b8 < PR_NF; ++b8) {
-                const double2 wv = *reinterpret_cast<const double2 *>(&W8c[b8 * 64 + frag_off]);
-                const double2 lv = *reinterpret_cast<const double2 *>(&Lc[(b8 * (b8 + 1) / 2 + b8) * 64 + frag_off]);
-                double x0 = 0.0, x1 = 0.0;
-                dmma884_r(x0, x1, t[b8][0], wv.x);                                  // X0 = A W8^T
-                dmma884_r(x0, x1, t[b8][1], wv.y);
-                double r0 = t[b8][0], r1 = t[b8][1];
-                dmma884_r(r0, r1, -x0, lv.x);                                       // r = A - X0 L8^T
-                dmma884_r(r0, r1, -x1, lv.y);
-                dmma884_r(x0, x1, r0, wv.x);                                        // X = X0 + r W8^T
-                dmma884_r(x0, x1, r1, wv.y);
-                const double nx0 = -x0, nx1 = -x1;
-#pragma unroll
-                for (int bp = b8 + 1; bp < PR_NF; ++bp) {
-                    const double2 lp = *reinterpret_cast<const double2 *>(&Lc[(bp * (bp + 1) / 2 + b8) * 64 + frag_off]);
-                    dmma884_r(t[bp][0], t[bp][1], nx0, lp.x);
-                    dmma884_r(t[bp][0], t[bp][1], nx1, lp.y);
-                }
-                if (rv) {
-                    const int c = b8 * 8 + 2 * fk;
-                    if (c + 1 < nv) *reinterpret_cast<double2 *>(grow + b8 * 8) = make_double2(x0, x1);
-                    else if (c < nv) grow[b8 * 8] = x0;
-                }
+            fused_solve8(Ab + (size_t)min(r, rows_end - 1) * ld + 2 * fk, r < rows_end, nv, 0, Lc, W8c, frag_off, fk);
+        }
+    }
+    if (FUSED && A.W && j0 + NB < n) {
+        // ---------------------------------------------------------------- the same solve in the compact band layout
+        // Exactly the rows trsm_panel8 solves for this envelope: the band's 64-row blocks below the diagonal block (all of
+        // them when the band reaches the last one) that hold a nonzero left of j0 + NB, then the border row (row n) alone.
+        // Other rows are not stored.  The last block column solves nothing: border_finish solves the border row's last
+        // block, as after separate launches, so the result is the same to the bit.
+        const int r_first = j0 + NB;
+        const int nmb = (n - r_first + 63) / 64;
+        const int nbl = (env.band >= 0 && env.band < nmb - 1) ? env.band : nmb;
+#pragma unroll 1
+        for (int rb = 0; rb <= nbl; ++rb) {
+            const int row0 = r_first + rb * 64;
+            if (rb < nbl) {
+                const int e = env_first_col(env, m, row0, min(row0 + 64, n));
+                if (e >= j0 + NB || row0 + w * 8 >= n) continue;        // block- / warp-uniform
+                const int r = min(row0 + w * 8 + fr, n - 1);
+                fused_solve8(view_elem(A, m, r, j0 + 2 * fk), row0 + w * 8 + fr < n, nv, max(e - j0, 0) / 8, Lc, W8c, frag_off, fk);
+            } else if (w == 0) {
+                fused_solve8(view_elem(A, m, n, j0 + 2 * fk), fr == 0, nv, 0, Lc, W8c, frag_off, fk);
             }
         }
     }
@@ -340,22 +373,23 @@ int launch_potf2_reg(BatchView A, int n, int j0, double *W, long long strideW, i
     if (B <= 0) return 0;
     if ((A.ld & 1) || (j0 & 1)) { set_error("potf2: ld=%d j0=%d must be even", A.ld, j0); return GPMC_EALIGN; }
     prof_begin(KC_POTF2, s);
-    potf2_reg_kernel<false><<<B, PR_THREADS, 0, s>>>(A, n, j0, W, strideW, info, zero_upper, n);
+    potf2_reg_kernel<false><<<B, PR_THREADS, 0, s>>>(A, n, j0, W, strideW, info, zero_upper, n, Envelope{});
     prof_end(KC_POTF2, s);
     GPMC_LAUNCH_CHECK();
     return 0;
 }
 
 // panel factor + panel solve of block column j0 in one launch; n_rows = n + border rows
-int launch_panel_fused(BatchView A, int n, int n_rows, int j0, double *W, long long strideW, int *info, int zero_upper, int B, cudaStream_t s)
+int launch_panel_fused(BatchView A, int n, int n_rows, int j0, double *W, long long strideW, int *info, int zero_upper, int B, cudaStream_t s,
+                       Envelope env)
 {
     if (B <= 0) return 0;
     if ((A.ld & 1) || (j0 & 1)) { set_error("panel: ld=%d j0=%d must be even", A.ld, j0); return GPMC_EALIGN; }
-    if (A.W) { set_error("panel: the fused panel kernel does not take the compact band layout"); return GPMC_EINVAL; }
+    if (A.W && (!env.blk || n_rows != n + 1)) { set_error("panel: the compact band layout needs its envelope and one border row"); return GPMC_EINVAL; }
     static DeviceOnce attr_set;
     if (attr_set.first()) GPMC_CUDA_CHECK(cudaFuncSetAttribute(potf2_reg_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM));
     prof_begin(KC_POTF2, s);
-    potf2_reg_kernel<true><<<B, PR_THREADS, PF_SMEM, s>>>(A, n, j0, W, strideW, info, zero_upper, n_rows);
+    potf2_reg_kernel<true><<<B, PR_THREADS, PF_SMEM, s>>>(A, n, j0, W, strideW, info, zero_upper, n_rows, env);
     prof_end(KC_POTF2, s);
     GPMC_LAUNCH_CHECK();
     return 0;

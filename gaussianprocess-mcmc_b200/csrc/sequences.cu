@@ -265,20 +265,23 @@ int potrf_fuse_auto(int n, int B, int border_rows)
 }
 
 // The compact band layout (BatchView::W) is known to the envelope-aware update tile kernel, the register-resident panel
-// factor and the 8-column panel solve, not to the fused panel kernels.  The layout is chosen for waves that run the plain
-// left-looking schedule; the jitter ladder's retries of a few items may run windows and look-ahead on it (every update
-// tile there also starts at the envelope and leaves before touching C when its contraction is empty).
+// factor (alone or fused with the panel solve) and the 8-column panel solve.  The layout is chosen for waves that run the
+// plain left-looking schedule; the jitter ladder's retries of a few items may run windows and look-ahead on it (every
+// update tile there also starts at the envelope and leaves before touching C when its contraction is empty).
 static bool compact_kernels() { return NB == BAND_ROWS && g_trsm_mode == 0 && g_potf2_mode == 0; }
-bool potrf_compact_ok(int n, int B, int border_rows)
+bool potrf_compact_ok(int n, int B)
 {
     const int Bs = schedule_batch(B);
-    return compact_kernels() && potrf_window_for(n, Bs) == 0 && g_lookahead_mode != 2 && !potrf_fuse_auto(n, B, border_rows);
+    return compact_kernels() && potrf_window_for(n, Bs) == 0 && g_lookahead_mode != 2;
 }
+// Every block column of a banded matrix has only the band's few rows below its diagonal block, which is what the fused
+// panel launches are for: the compact layout fuses them unless gpmc_set_tuning(9, 1) forbids it.
+int potrf_fuse_compact() { return g_panel_fuse == 1 ? 0 : 1; }
 
 int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long strideW, long long w_step,
                    int zero_upper_flag, cudaStream_t s, int border_rows, int fuse, Envelope env)
 {
-    if (A.W && (fuse || border_rows != 1 || w_step || zero_upper_flag || !env.blk || !compact_kernels())) {
+    if (A.W && (border_rows != 1 || w_step || zero_upper_flag || !env.blk || !compact_kernels())) {
         set_error("potrf_sequence: the compact band layout needs the envelope-aware kernels and one border row");
         return GPMC_EINVAL;
     }
@@ -384,7 +387,7 @@ int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long st
             }
             if (fuse) {
                 if ((rc = (g_potf2_mode == 3 ? launch_panel_fused_flow(A, n, nr, j0, Wj, strideW, info, zero_upper_flag, B, sP)
-                                             : launch_panel_fused(A, n, nr, j0, Wj, strideW, info, zero_upper_flag, B, sP)))) return rc;
+                                             : launch_panel_fused(A, n, nr, j0, Wj, strideW, info, zero_upper_flag, B, sP, A.W ? env : Envelope{})))) return rc;
                 if (la) GPMC_CUDA_CHECK(cudaEventRecord(la->ev_p, sP));
                 continue;
             }

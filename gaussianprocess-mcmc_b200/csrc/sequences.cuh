@@ -17,14 +17,17 @@ namespace gpmc {
 // fuse != 0: panel factor and panel solve of every block column in ONE launch (launch_panel_fused); the border rows are
 // then COMPLETE on return, the last block column included (pass the same flag to border_finish).  Callers decide once
 // per batch with potrf_fuse_auto() and use the same flag for every call on those buffers (retries of subsets included).
+// In the compact band layout (A.W > 0) the fused launches leave the border row's last block to border_finish (solved = 0).
 // env: envelope of A as launch_cov_assemble wrote it -- the update GEMMs and the panel solves skip the work it shows to
-// be zero (bit-identical results); the fused panel launches ignore it.
+// be zero (bit-identical results); the fused panel launches use it in the compact band layout only.
 int potrf_sequence(BatchView A, int n, int B, int *info, double *W, long long strideW, long long w_step,
                    int zero_upper, cudaStream_t s, int border_rows = 0, int fuse = 0, Envelope env = {});
 int potrf_fuse_auto(int n, int B, int border_rows);
 // potrf_sequence of B matrices of order n would run the plain left-looking schedule with the kernels that know the compact
 // band layout (BatchView::W)
-bool potrf_compact_ok(int n, int B, int border_rows);
+bool potrf_compact_ok(int n, int B);
+// the fuse flag of potrf_sequence for the compact band layout (1 unless gpmc_set_tuning(9, 1))
+int potrf_fuse_compact();
 
 // One wave of assemble-and-factor with the pyGPs jitter ladder (capi.cu); shared by the log-lik unit, the predictive
 // path and the elliptical slice sampler's Cholesky draw.

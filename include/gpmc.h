@@ -281,7 +281,8 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
  *        sliceSample.py:197-198,204 write it (8/3 N^3; twice the workspace per chain -- query gpmc_sds_workspace_bytes
  *        after setting it).  Used for parity with the reference, not for speed.
  * key 9: panel factor + panel solve of a block column in ONE launch (one CTA per matrix): 0 = auto (many small matrices in
- *        flight), 1 = never, 2 = whenever the default panel kernels are selected.
+ *        flight, and every wave of the compact band layout, key 17), 1 = never, 2 = whenever the default panel kernels are
+ *        selected.
  * key 10: in-window update of a look-ahead column: 0 = auto (split in a long and a K = 128 short part when a trailing update
  *        runs beside the window or the launches are small; one launch otherwise), 1 = always split, 2 = one launch in every
  *        window that runs alone.
@@ -293,7 +294,7 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
  * key 14: envelope skips in gpmc_loglik_batched / gpmc_loglik_host: 1 = on (default): the assembly records, per 64-row block,
  *        the first column that holds a nonzero, and the update GEMM and the panel solve skip the products it shows to be
  *        exact zeros (K of a stationary kernel underflows to 0 far from the diagonal; results are bit-identical); 0 = dense.
- *        Waves factored with fused panel launches (key 9) are always dense.
+ *        Dense-layout waves factored with fused panel launches (key 9) do not record or use it.
  * key 15: band (with key 14 on): 1 = on (default): a bound from bounding boxes of x / ell gives, per 64-row block, the first
  *        64-column tile that can hold a nonzero; only the band right of it is assembled, and the update GEMM and the panel
  *        solve launch only the rows of the widest band of the wave (bit-identical results); 0 = envelope skips only.

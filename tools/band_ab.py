@@ -1,8 +1,10 @@
 """Band-only assembly and launches on vs. off (gpmc_set_tuning(15, .)) on the bench.py workload, in the dense layout with
 the region left of the band cleared inline in the assembly (gpmc_set_tuning(16, 2)) or on a side stream (16, 1), and in
-the compact band layout (gpmc_set_tuning(17, 1), default: only the band's columns are stored, all chains in fewer waves):
-ms per step, per class kernel ms per step, waves and row width W of each arm, launched vs. working CTAs of the assembly,
-the update GEMM and the panel solve, and a bitwise comparison of loglik and info with the envelope-only run.
+the compact band layout (gpmc_set_tuning(17, 1), default: only the band's columns are stored, all chains in fewer waves)
+with the panel factor and solve of a block column in one launch (default) or in two (gpmc_set_tuning(9, 1)):
+ms per step, per class kernel ms and launches per step, waves and row width W of each arm, launched vs. working CTAs of
+the assembly, the update GEMM and the panel solve, a bitwise comparison of loglik and info with the envelope-only run and
+between the two compact arms, and the name and power limit of the card.
 
 The CTA counts replay the plain left-looking schedule of sequences.cu (the one the bench workload runs) on the envelopes,
 band starts w and wave bands the device wrote (read back from gpmc_loglik_batched's workspace, wave by wave).  A CTA
@@ -105,10 +107,11 @@ def layout():
     return W.value, waves.value
 
 
-def per_step_ms(x, G, H, band, clear, compact, steps):
+def per_step_ms(x, G, H, band, clear, compact, fuse_off, steps):
     gp.ops.set_tuning(15, band)
     gp.ops.set_tuning(16, clear)
     gp.ops.set_tuning(17, compact)
+    gp.ops.set_tuning(9, fuse_off)
     try:
         for _ in range(2):
             ll, info = gp.ops.loglik_batched(x, G, H)
@@ -126,11 +129,24 @@ def per_step_ms(x, G, H, band, clear, compact, steps):
             gp.ops.loglik_batched(x, G, H)
         prof = gp.ops.profile_read()
         gp.ops.profile(False)
-        return ms, {k: v[0] / steps for k, v in prof.items() if v[1] > 0}, ll.cpu().numpy(), info.cpu().numpy(), lay
+        return (ms, {k: v[0] / steps for k, v in prof.items() if v[1] > 0}, {k: v[1] / steps for k, v in prof.items() if v[1] > 0},
+                ll.cpu().numpy(), info.cpu().numpy(), lay)
     finally:
         gp.ops.set_tuning(15, 1)
         gp.ops.set_tuning(16, 2)
         gp.ops.set_tuning(17, 1)
+        gp.ops.set_tuning(9, 0)
+
+
+def card():
+    """name and power limit of the card, read next to the measurement"""
+    import subprocess
+    try:
+        q = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit', '--format=csv,noheader', '-i', str(torch.cuda.current_device())],
+                           capture_output=True, text=True, timeout=60).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        q = ''
+    return q or torch.cuda.get_device_name()
 
 
 def main():
@@ -156,14 +172,16 @@ def main():
     # the compact layout factors every chain in one wave (when it fits) with the call's widest band
     one = [(np.concatenate([w[0] for w in waves]), np.concatenate([w[1] for w in waves]),
             max(w[2] for w in waves), max(w[3] for w in waves))]
-    arms = (('band_off', 0, 1, 0), ('band_on_side_clear', 1, 1, 0), ('band_on_inline_clear', 1, 2, 0),
-            ('band_compact', 1, 2, 1))
-    res = {k: [] for k, _, _, _ in arms}
+    # (label, band, clear, compact, fused panels forbidden)
+    arms = (('band_off', 0, 1, 0, 1), ('band_on_side_clear', 1, 1, 0, 1), ('band_on_inline_clear', 1, 2, 0, 1),
+            ('band_compact', 1, 2, 1, 1), ('band_compact_fused', 1, 2, 1, 0))
+    res = {k[0]: [] for k in arms}
     outs = {}
     for _ in range(a.rounds):
-        for label, band, clear, compact in arms:
-            ms, cls, ll, info, lay = per_step_ms(x, G, H, band, clear, compact, a.steps)
-            res[label].append({'ms_per_step': ms, 'kernel_ms_per_step': cls, 'band_W': lay[0], 'waves': lay[1]})
+        for label, band, clear, compact, fuse_off in arms:
+            ms, cls, nl, ll, info, lay = per_step_ms(x, G, H, band, clear, compact, fuse_off, a.steps)
+            res[label].append({'ms_per_step': ms, 'kernel_ms_per_step': cls, 'launches_per_step': nl, 'band_W': lay[0],
+                               'waves': lay[1]})
             outs[label] = (ll, info)
     gp.ops.set_tuning(14, 0)
     try:
@@ -172,11 +190,12 @@ def main():
     finally:
         gp.ops.set_tuning(14, 1)
     same = lambda p, q: bool(np.array_equal(p[0].view(np.int64), q[0].view(np.int64)) and np.array_equal(p[1], q[1]))
-    row = {'n': n, 'chains': B, 'wave': int(wave), 'steps': a.steps,
+    row = {'card': card(), 'n': n, 'chains': B, 'wave': int(wave), 'steps': a.steps,
            'wave_bands': [{'launch_band_blocks': w[2], 'assembly_band_tiles': w[3]} for w in waves],
            'work_band_off': work_counts(waves, n, False), 'work_band_on': work_counts(waves, n, True),
            'work_band_compact': work_counts(one, n, True),
-           'outputs_bitwise_equal_to_band_off': {k: same(outs[k], outs['band_off']) for k, _, _, _ in arms},
+           'outputs_bitwise_equal_to_band_off': {k[0]: same(outs[k[0]], outs['band_off']) for k in arms},
+           'compact_fused_bitwise_equal_to_compact': same(outs['band_compact_fused'], outs['band_compact']),
            'band_off_bitwise_equal_to_dense': same(outs['band_off'], dense),
            'arms': res}
     print(json.dumps(row))
