@@ -11,6 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libgpmc.so')
 
 KIND_SE_ISO, KIND_SE_ARD = 0, 1
+KIND_MATERN1, KIND_MATERN3, KIND_MATERN5 = 2, 3, 4
 ASM_ADD_S, ASM_LOWER_ONLY = 1, 2
 JITTER_NONE, JITTER_PYGPS = 0, 1
 INFO_NOT_PD = -1

@@ -28,7 +28,7 @@ class ChainEnsemble(object):
     ``(Hyp[B,P], loglik[B], ntrips[B])`` as numpy arrays on every rank."""
 
     def __init__(self, x, y, F0, Hyp0, scale, seed=0, max_trips=64, sweeper=None, gather_f=False, sharded_input=False,
-                 distributed=True, strict=False):
+                 distributed=True, strict=False, kind=None):
         self.x = np.asarray(x, dtype=np.float64)
         if self.x.ndim == 1:
             self.x = self.x.reshape(-1, 1)
@@ -36,6 +36,7 @@ class ChainEnsemble(object):
         self.my = float(np.mean(self.y))                       # sliceSample.py:102
         self.scale = np.asarray(scale, dtype=np.float64).reshape(-1)
         self.seed, self.max_trips, self.gather_f = int(seed), int(max_trips), gather_f
+        self.kind = kind                   # covariance kind (ops.KIND_*); None: SE iso / ARD from the width of Hyp0
         # A chain whose slice does not close within ``max_trips`` proposals keeps its state and is reported with
         # status 1 (the reference's ``while True`` would loop on, or raise LinAlgError out of jitchol when the
         # factorisation at the current state is the reason).  ``strict`` turns that into an exception; otherwise the
@@ -234,7 +235,7 @@ class _DeviceSweeper(object):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         nt, ll, status = ops.sds_sweep(self.x, self.y, self.F, self.H, self.scale, it, my=e.my, seed=e.seed,
-                                       chain0=e.lo, max_trips=e.max_trips)
+                                       chain0=e.lo, max_trips=e.max_trips, kind=e.kind)
         e1.record()
         e1.synchronize()
         self.last_busy_ms = e0.elapsed_time(e1)
@@ -252,7 +253,7 @@ class _DeviceSweeper(object):
             # blocks that do not start on a kept iteration: run up to the next kept one first
             raise ValueError('gather_every must be a multiple of thin_f')
         hh, ll, nt, hf, n_exh = ops.sds_run(self.x, self.y, self.F, self.H, self.scale, it0, n_iters, my=e.my, seed=e.seed,
-                                            chain0=e.lo, max_trips=e.max_trips, keep_f_every=thin_f)
+                                            chain0=e.lo, max_trips=e.max_trips, keep_f_every=thin_f, kind=e.kind)
         e1.record()
         e1.synchronize()
         self.last_busy_ms = e0.elapsed_time(e1)

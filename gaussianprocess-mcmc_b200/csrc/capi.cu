@@ -280,11 +280,11 @@ int gpmc_cov_assemble(const double *x_dev, int N, int D, const double *hyp_dev, 
                       const double *jitter_dev, double *A_dev, int ld, void *stream)
 {
     GPMC_API_LOCK();
-    const int n_ell = (kind == GPMC_KIND_SE_ARD) ? D : 1;
-    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2) { set_error("cov_assemble: bad shape N=%d D=%d B=%d P=%d kind=%d", N, D, B, P, kind); return GPMC_EINVAL; }
+    const int n_ell = kind_n_ell(kind, D);
+    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2 || kind_cf(kind) < 0) { set_error("cov_assemble: bad shape N=%d D=%d B=%d P=%d kind=%d", N, D, B, P, kind); return GPMC_EINVAL; }
     if (ld < N || (ld & 1)) { set_error("cov_assemble: ld=%d must be even and >= N=%d", ld, N); return GPMC_EALIGN; }
     BatchView A{A_dev, (long long)N * ld, ld, nullptr, nullptr};
-    return launch_cov_assemble(x_dev, N, D, hyp_dev, P, n_ell, flags, jitter_dev, A, B, (cudaStream_t)stream);
+    return launch_cov_assemble(x_dev, N, D, hyp_dev, P, kind, flags, jitter_dev, A, B, (cudaStream_t)stream);
 }
 
 int gpmc_potrf_batched(double *A_dev, int N, int ld, int B, int *info_dev, int jitter_policy, int zero_upper,
@@ -367,8 +367,8 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
 {
     GPMC_API_LOCK();
     cudaStream_t s = (cudaStream_t)stream;
-    const int n_ell = (kind == GPMC_KIND_SE_ARD) ? D : 1;
-    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2) { set_error("loglik: bad shape N=%d D=%d B=%d P=%d kind=%d", N, D, B, P, kind); return GPMC_EINVAL; }
+    const int n_ell = kind_n_ell(kind, D);
+    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2 || kind_cf(kind) < 0) { set_error("loglik: bad shape N=%d D=%d B=%d P=%d kind=%d", N, D, B, P, kind); return GPMC_EINVAL; }
     if (B == 0) return 0;
     const LoglikLayout l = loglik_layout(N, B);
     if (!ws_dev || ws_bytes < l.fixed_bytes + l.per_item_bytes) {
@@ -399,7 +399,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
         const size_t room = ws_bytes - l.fixed_bytes;
         if (2 * wenv + 256 < room) {
             GPMC_CUDA_CHECK(cudaMemsetAsync(band_dev, 0, 2 * sizeof(int), s));
-            int rc = launch_band_bound(x_dev, N, D, hyp_dev, P, n_ell, B, w_all, nblk, band_dev, xbox, s);
+            int rc = launch_band_bound(x_dev, N, D, hyp_dev, P, kind, B, w_all, nblk, band_dev, xbox, s);
             if (rc) return rc;
             int bh[2] = {0, 0};
             GPMC_CUDA_CHECK(cudaMemcpyAsync(bh, band_dev, sizeof(bh), cudaMemcpyDeviceToHost, s));
@@ -426,7 +426,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
                     const double *g_w = g_dev + (size_t)s0 * N;
                     int *info_w = info_dev + s0;
                     auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
-                        int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
+                        int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, kind, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
                         if (rc) return rc;
                         return border_set(V, N, g_w, N, nitems, s);
                     };
@@ -469,7 +469,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
                 clear.pending = false;
             }
             GPMC_CUDA_CHECK(cudaMemsetAsync(band_dev, 0, 2 * sizeof(int), s));
-            rc = launch_band_bound(x_dev, N, D, hyp_w, P, n_ell, nb, band_w, env_blocks(N), band_dev, xbox, s);
+            rc = launch_band_bound(x_dev, N, D, hyp_w, P, kind, nb, band_w, env_blocks(N), band_dev, xbox, s);
             if (rc) return rc;
             // The launch sizes need the band on the host: one synchronisation.  The inline clear's assembly grid does not,
             // and with few matrices in flight the update and solve launches are small anyway (N=16384 x 1 measured 0.3 %
@@ -493,7 +493,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
             }
         }
         auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
-            int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
+            int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, kind, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
             if (rc) return rc;
             return border_set(V, N, g_w, N, nitems, s);
         };

@@ -64,6 +64,49 @@ struct DeviceOnce {
 };
 
 // ---------------------------------------------------------------------------------------------
+// Covariance functions.  Every kernel that evaluates K off the diagonal takes the family as a template parameter CF (a
+// uniform run-time branch in cov_assemble_kernel's fast path cost the hot instantiation 20 %) and forms K with these two
+// helpers, from s = sum_d (u_id - u_jd)^2 summed in cdist's order without FMA:
+//   CF = 0        squared exponential (GPMC_KIND_SE_ISO / _ARD; pyGPs 1.3.4 cov.RBF / RBFard):
+//                 u = x / ell,             K = sf2 * exp(-0.5 * s)
+//   CF = 1, 3, 5  Matern with d = 2 nu = CF (GPMC_KIND_MATERN1/3/5; pyGPs 1.3.4 cov.Matern as restated in oracle/matern_oracle.py):
+//                 u = sqrt(d) * x / ell,   t = sqrt(s),   K = sf2 * (f_d(t) * exp(-t)),
+//                 f_1 = 1,  f_3 = 1 + t,  f_5 = 1 + t * (1 + t / 3)
+// f_d(0) = 1, so K_ii = sf2 for every family.  The SE expressions are the ones the kernels evaluated before Matern existed.
+// Host side: the kind of an entry point maps to (CF, number of length-scales) through kind_cf / kind_n_ell.
+template <int CF> __device__ __forceinline__ double cov_u(double x, double ell)
+{
+    static_assert(CF == 0 || CF == 1 || CF == 3 || CF == 5, "SE (0) or Matern d = 1, 3, 5");
+    if (CF == 0) return x / ell;
+    // np.sqrt(d) * x / ell, left to right; sqrt(1) * x == x exactly.  The constants are the doubles np.sqrt(3), np.sqrt(5).
+    return (CF == 1 ? x : (CF == 3 ? 1.7320508075688772 : 2.23606797749979) * x) / ell;
+}
+template <int CF> __device__ __forceinline__ double cov_k(double sf2, double s)
+{
+    if (CF == 0) return sf2 * exp(-0.5 * s);
+    const double t = sqrt(s);
+    const double e = exp(-t);
+    if (CF == 1) return sf2 * e;                                    // f_1 * e == e exactly
+    if (CF == 3) return sf2 * (__dadd_rn(1.0, t) * e);
+    return sf2 * (__dadd_rn(1.0, __dmul_rn(t, __dadd_rn(1.0, t / 3.0))) * e);     // no FMA: numpy rounds every step
+}
+// d K / d ell * ell (Matern; the gradient contraction): sf2 * (g_d(t) * exp(-t)), g_1 = t, g_3 = t^2, g_5 = t^2 (1 + t) / 3
+template <int CF> __device__ __forceinline__ double matern_dk_dell_ell(double sf2, double s)
+{
+    static_assert(CF == 1 || CF == 3 || CF == 5, "Matern only");
+    const double t = sqrt(s);
+    const double e = exp(-t);
+    const double g = CF == 1 ? t : (CF == 3 ? __dmul_rn(t, t) : __dmul_rn(__dmul_rn(t, t), __dadd_rn(1.0, t)) / 3.0);
+    return sf2 * (g * e);
+}
+// Kind of an entry point -> covariance family (-1: not a kind) and number of length-scales in a hyper-parameter row
+__host__ __device__ inline int kind_cf(int kind)
+{
+    return kind == 0 || kind == 1 ? 0 : kind == 2 ? 1 : kind == 3 ? 3 : kind == 4 ? 5 : -1;
+}
+__host__ __device__ inline int kind_n_ell(int kind, int D) { return kind == 1 ? D : 1; }
+
+// ---------------------------------------------------------------------------------------------
 // Batched matrix view.  Item b of a launch is matrix `map ? map[b] : b` of the allocation, so a
 // compacted list of active chains / failed items can be processed without moving data.
 // Compact band layout (W > 0, gpmc_loglik_batched when its band is narrow): row r keeps only the W columns
@@ -132,6 +175,14 @@ struct Envelope {
 //   * the jitter ladder re-assembles the same band (the bound does not depend on the jitter).
 // The compact layout (see BatchView) stores exactly that much: with width = max over items of r - w[r], W >= 128 +
 // 64 width puts band_col0 of every 128-row block at or left of 64 w[r] of both its 64-row blocks.
+// Why a tile is +0 (band_bound_kernel): the boxes of u (cov_u is monotone in x under round-to-nearest) give a lower bound
+// s_lo of every element's s in the tile (each difference, square and sum rounds monotonically), then
+//   SE:     0.5 s_lo > 760 + max(0, ln sf2): exp(-0.5 s) underflows to +0, so sf2 * exp(-0.5 s) is +0;
+//   Matern: sqrt(s_lo) > 745.14 (both with relative slack 1e-9): the device exp returns +0 for arguments <= -745 (the
+//           IEEE result is +0 below -745.133), f_d(t) >= 1 is finite, so f_d * exp(-t) is +0, and sf2 * (+0) = +0 for a
+//           finite sf2.  f_d is finite as long as s is; an item whose largest possible s overflows is dense (t = inf
+//           would make K = inf * 0 = NaN there).
+// Non-finite x, ell or sf2, and sf2 <= 0, make the item dense in both families.
 struct Band {
     const int *w = nullptr;  // w[item * ld + r]; nullptr: the whole lower triangle is assembled
     int ld = 0;
@@ -156,22 +207,23 @@ __device__ __forceinline__ int env_first_col(const Envelope &e, int m, int r0, i
 // cov_assemble.cu
 // env.blk != nullptr: also writes the envelope of every assembled item (the items A selects)
 // band.w != nullptr: only the tiles of the band (see Band) are written
-int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P, int n_ell, int flags,
+// kind: GPMC_KIND_* (validated by the entry point; the length-scales of a row are kind_n_ell(kind, D))
+int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P, int kind, int flags,
                         const double *jitter, BatchView A, int B, cudaStream_t s, Envelope env = {}, Band band = {});
 // Band bound of items 0 .. B-1 (hyp rows, as launch_cov_assemble reads them): w[item * ldw + r] (see Band), and
 // band_out[0] = max over items and r of r - lo[r], band_out[1] = max of r - w[r] (band_out must start at 0).
 // xbox: scratch of 2 * D * env_blocks(N) doubles.
-int launch_band_bound(const double *x, int N, int D, const double *hyp, int P, int n_ell, int B, int *w, int ldw,
+int launch_band_bound(const double *x, int N, int D, const double *hyp, int P, int kind, int B, int *w, int ldw,
                       int *band_out, double *xbox, cudaStream_t s);
 // +0 into every element of rows 0 .. N-1 of items 0 .. B-1 left of their row block's w (store only, small grid)
 int launch_band_clear(BatchView A, int N, Band band, int B, cudaStream_t s);
 
 // grad_contract.cu : the contraction of gpmc_loglik_grad_batched for items 0 .. B-1 (item stride strideW / ldv / ldw):
 //   grad[b][p] = 0.5 sum_ij (alpha_i alpha_j - W_ij) dA_ij/dtheta_p  from the lower triangle of W (row stride ldW),
-//   K_ij recomputed from x and hyp with cov_assemble's expression.  band_w != nullptr: row block r of item b reads only the
+//   K_ij recomputed from x and hyp with cov_assemble's expression (cov_u / cov_k).  band_w != nullptr: row block r of item b reads only the
 //   64-column tiles from band_w[b * ldw + r] on (left of them K_ij is +0).  partial: scratch of B * env_blocks(N) * P
 //   doubles.  Items with info != 0, or a parameter that is not a positive finite number, get a NaN row.
-int launch_grad_contract(const double *x, int N, int D, const double *hyp, int P, int n_ell, const double *alpha, int ldv,
+int launch_grad_contract(const double *x, int N, int D, const double *hyp, int P, int kind, const double *alpha, int ldv,
                          const double *W, int ldW, long long strideW, const int *band_w, int ldw, const int *info,
                          double *partial, double *grad, int B, cudaStream_t s);
 

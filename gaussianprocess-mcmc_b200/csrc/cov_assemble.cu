@@ -1,11 +1,11 @@
-// Fused covariance assembly: SE (iso / ARD) kernel + S diagonal + jitter + symmetric fill.
+// Fused covariance assembly: SE (iso / ARD) or Matern (d = 1, 3, 5) kernel + S diagonal + jitter + symmetric fill.
 //
 // Replaces, per batch item, the reference's
 //   Kc = covK.RBF(np.log(hyp[0]), np.log(hyp[1])); K = Kc.getCovMatrix(x=x, mode='train')   sliceSample.py:104-105,136-137
 //   S_ii = 1/((1/sn^2 + 1/K_ii) - 1/K_ii); S = max(S, 0); K+S                               sliceSample.py:183-190,196
 // (pyGPs 1.3.4 cov.RBF: K = sf2 * exp(-0.5 * cdist(x/ell, x/ell, 'sqeuclidean')), ell = exp(log_ell),
 //  sf2 = exp(2 log_sigma)); the operation order of those expressions is kept so the matrix matches
-//  numpy's to the last bits of exp().
+//  numpy's to the last bits of exp().  The Matern kinds replace the kernel expression only (cov_u / cov_k, common.cuh).
 //
 // Layout: one CTA = one 64x64 tile on or below the diagonal.  Each lane owns two adjacent columns
 // (double2, 16 B stores; a warp writes 512 contiguous bytes of one row), the tile is mirrored
@@ -38,7 +38,8 @@ __device__ __forceinline__ void tile_decode(int t, int &tm, int &tn)
 // the diagonal.
 // PRED: the K / sn^2 + I variant of inf_mcmc (GPMC_ASM_PRED) -- a template parameter, not a run-time test: a uniform
 // `if (pred)` in the fast path cost the hot (non-PRED) instantiation 20 % (3.5 vs 4.2 TB/s at N=4096, round 2).
-template <int DT, bool PRED>
+// CF: covariance family (cov_u / cov_k, common.cuh), a template parameter for the same reason.
+template <int DT, bool PRED, int CF>
 __global__ void __launch_bounds__(256)
 cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *__restrict__ hyp, int P, int n_ell,
                     int flags, const double *__restrict__ jitter, BatchView A, Envelope env, Band band)
@@ -124,14 +125,14 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
     else tile_decode(t, tm, tn);
     const int r0 = tm * AT, c0 = tn * AT;
     if (tt > 0) __syncthreads();                 // the previous tile's u vectors / mirrored tile are still being read
-    // u = x / ell for the tile's rows and columns
+    // u = x / ell (SE) or sqrt(d) x / ell (Matern) for the tile's rows and columns
     for (int e = tid; e < 2 * AT * D; e += 256) {
         const int which = e / (AT * D);
         const int rem = e - which * AT * D;
         const int i = rem / D, d = rem - i * D;
         const int gi = (which ? c0 : r0) + i;
         const double ell = s_ell[n_ell == 1 ? 0 : d];
-        const double v = (gi < N) ? x[(size_t)gi * D + d] / ell : 0.0;
+        const double v = (gi < N) ? cov_u<CF>(x[(size_t)gi * D + d], ell) : 0.0;
         if (which) s_uj[d][i] = v; else s_ui[d][i] = v;
     }
     __syncthreads();
@@ -159,8 +160,8 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
                 s0 = __dadd_rn(s0, __dmul_rn(d0, d0));
                 s1 = __dadd_rn(s1, __dmul_rn(d1, d1));
             }
-            double k0 = sf2 * exp(-0.5 * s0);
-            double k1 = sf2 * exp(-0.5 * s1);
+            double k0 = cov_k<CF>(sf2, s0);
+            double k1 = cov_k<CF>(sf2, s1);
             if (pred) { k0 = k0 / sn2; k1 = k1 / sn2; }
             if (mirror) *reinterpret_cast<double2 *>(&s_tile[rl][cl]) = make_double2(k0, k1);
             *reinterpret_cast<double2 *>(dst + (size_t)rr * A.ld) = make_double2(k0, k1);
@@ -180,8 +181,8 @@ cov_assemble_kernel(const double *__restrict__ x, int N, int Drt, const double *
             s0 = __dadd_rn(s0, __dmul_rn(d0, d0));            // cdist 'sqeuclidean': s += d*d, no FMA
             s1 = __dadd_rn(s1, __dmul_rn(d1, d1));
         }
-        double k0 = sf2 * exp(-0.5 * s0);
-        double k1 = sf2 * exp(-0.5 * s1);
+        double k0 = cov_k<CF>(sf2, s0);
+        double k1 = cov_k<CF>(sf2, s1);
         if (pred) { k0 = k0 / sn2; k1 = k1 / sn2; }
         if (gr == gc)     { k0 = k0 + diag_add; if (has_jit) k0 = k0 + jit; }
         if (gr == gc + 1) { k1 = k1 + diag_add; if (has_jit) k1 = k1 + jit; }
@@ -252,9 +253,11 @@ __global__ void band_xbox_kernel(const double *__restrict__ x, int N, int D, dou
     xbox[2 * e + 1] = finite ? hi : NAN;
 }
 
-// One CTA per item.  Tile (r, c) is certainly +0 when the squared distance of the two boxes of x / ell, s, satisfies
-// 0.5 s > 760 + max(0, ln sf2) (with relative slack): every element's distance is at least s (each difference, square and
-// sum rounds monotonically), and exp underflows to +0 below -745.2, so sf2 * exp(-0.5 s) is +0 for all of them.
+// One CTA per item.  Tile (r, c) is certainly +0 when the squared distance of the two boxes of u, s, satisfies
+// 0.5 s > 760 + max(0, ln sf2) (SE) or sqrt(s) > 745.14 (Matern), with relative slack: every element's distance is at
+// least s (each difference, square and sum rounds monotonically), and exp underflows to +0 beyond either point, so K is +0
+// for all of them (the argument is written out next to Band, common.cuh).
+template <int CF>
 __global__ void band_bound_kernel(const double *__restrict__ hyp, int P, int n_ell, int N, int D, const double *__restrict__ xbox,
                                   int *__restrict__ w, int ldw, int *__restrict__ band_out)
 {
@@ -268,10 +271,26 @@ __global__ void band_bound_kernel(const double *__restrict__ hyp, int P, int n_e
     if (tid < n_ell) s_ell[tid] = exp(log(h[tid]));           // as cov_assemble_kernel forms them
     if (tid == 0) {
         const double sf2 = exp(2.0 * log(h[n_ell]));
-        s_thr = (isfinite(sf2) && sf2 > 0.0) ? 760.0 + fmax(0.0, log(sf2)) : NAN;
+        if (CF == 0) s_thr = (isfinite(sf2) && sf2 > 0.0) ? 760.0 + fmax(0.0, log(sf2)) : NAN;
+        else s_thr = (isfinite(sf2) && sf2 > 0.0) ? 745.14 : NAN;
         s_max[0] = s_max[1] = 0;
     }
     __syncthreads();
+    if (CF != 0) {
+        // Matern: the largest s any pair can reach, sum_d (2 max |u_d|)^2, must be finite (else t = inf, K = NaN)
+        if (tid == 0 && s_thr == s_thr) {
+            double smax = 0.0;
+            for (int d = 0; d < D; ++d) {
+                double a = 0.0;
+                for (int r = 0; r < nt1; ++r)
+                    a = fmax(a, fmax(fabs(xbox[2 * (r * D + d)]), fabs(xbox[2 * (r * D + d) + 1])));   // NaN boxes: dense anyway
+                const double g = 2.0 * cov_u<CF>(a, s_ell[0]);
+                smax = __dadd_rn(smax, __dmul_rn(g, g));
+            }
+            if (!isfinite(smax)) s_thr = NAN;
+        }
+        __syncthreads();
+    }
     bool dense = !(s_thr == s_thr);
     for (int d = 0; d < n_ell; ++d) dense = dense || !(isfinite(s_ell[d]) && s_ell[d] > 0.0);
     for (int e = tid; e < nt1 * D; e += blockDim.x) dense = dense || !(xbox[2 * e] == xbox[2 * e]);
@@ -290,14 +309,15 @@ __global__ void band_bound_kernel(const double *__restrict__ hyp, int P, int n_e
                     double s = 0.0;
                     for (int d = 0; d < D; ++d) {
                         const double ell = s_ell[n_ell == 1 ? 0 : d];
-                        const double rlo = xbox[2 * (r * D + d)] / ell, rhi = xbox[2 * (r * D + d) + 1] / ell;
-                        const double clo = xbox[2 * (c * D + d)] / ell, chi = xbox[2 * (c * D + d) + 1] / ell;
+                        const double rlo = cov_u<CF>(xbox[2 * (r * D + d)], ell), rhi = cov_u<CF>(xbox[2 * (r * D + d) + 1], ell);
+                        const double clo = cov_u<CF>(xbox[2 * (c * D + d)], ell), chi = cov_u<CF>(xbox[2 * (c * D + d) + 1], ell);
                         double g = 0.0;
                         if (rlo - chi > g) g = rlo - chi;
                         if (clo - rhi > g) g = clo - rhi;
                         s = __dadd_rn(s, __dmul_rn(g, g));
                     }
-                    maybe = !(0.5 * s * (1.0 - 1e-9) > thr);
+                    if (CF == 0) maybe = !(0.5 * s * (1.0 - 1e-9) > thr);
+                    else maybe = !(sqrt(s) * (1.0 - 1e-9) > thr);
                 }
                 const unsigned hit = __ballot_sync(0xffffffffu, maybe);
                 if (hit) { lo = c0 + __ffs(hit) - 1; break; }
@@ -322,16 +342,22 @@ __global__ void band_bound_kernel(const double *__restrict__ hyp, int P, int n_e
     if (tid == 0) { atomicMax(band_out, s_max[0]); atomicMax(band_out + 1, s_max[1]); }
 }
 
-int launch_band_bound(const double *x, int N, int D, const double *hyp, int P, int n_ell, int B, int *w, int ldw,
+int launch_band_bound(const double *x, int N, int D, const double *hyp, int P, int kind, int B, int *w, int ldw,
                       int *band_out, double *xbox, cudaStream_t s)
 {
+    const int n_ell = kind_n_ell(kind, D);
     if (D > MAX_ELL || n_ell > MAX_ELL) { set_error("D=%d exceeds MAX_ELL=%d", D, MAX_ELL); return GPMC_EINVAL; }
     if (B <= 0) return 0;
     const int nt1 = env_blocks(N);
     if ((size_t)nt1 * sizeof(int) > 48 * 1024) { set_error("band bound: N=%d has too many row blocks", N); return GPMC_EINVAL; }
     prof_begin(KC_ASSEMBLE, s);
     band_xbox_kernel<<<(nt1 * D + 127) / 128, 128, 0, s>>>(x, N, D, xbox);
-    band_bound_kernel<<<B, 256, nt1 * sizeof(int), s>>>(hyp, P, n_ell, N, D, xbox, w, ldw, band_out);
+    switch (kind_cf(kind)) {
+        case 1: band_bound_kernel<1><<<B, 256, nt1 * sizeof(int), s>>>(hyp, P, n_ell, N, D, xbox, w, ldw, band_out); break;
+        case 3: band_bound_kernel<3><<<B, 256, nt1 * sizeof(int), s>>>(hyp, P, n_ell, N, D, xbox, w, ldw, band_out); break;
+        case 5: band_bound_kernel<5><<<B, 256, nt1 * sizeof(int), s>>>(hyp, P, n_ell, N, D, xbox, w, ldw, band_out); break;
+        default: band_bound_kernel<0><<<B, 256, nt1 * sizeof(int), s>>>(hyp, P, n_ell, N, D, xbox, w, ldw, band_out); break;
+    }
     prof_end(KC_ASSEMBLE, s);
     GPMC_LAUNCH_CHECK();
     return 0;
@@ -368,9 +394,29 @@ int launch_band_clear(BatchView A, int N, Band band, int B, cudaStream_t s)
     return 0;
 }
 
-int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P, int n_ell, int flags,
+template <int CF>
+static void cov_assemble_launch(dim3 grid, cudaStream_t s, const double *x, int N, int D, const double *hyp, int P, int n_ell,
+                                int flags, const double *jitter, BatchView A, Envelope env, Band band)
+{
+#define GPMC_ASM_LAUNCH(DT_)                                                                                                     \
+    do {                                                                                                                          \
+        if (flags & GPMC_ASM_PRED) cov_assemble_kernel<DT_, true, CF><<<grid, 256, 0, s>>>(x, N, D, hyp, P, n_ell, flags, jitter, A, env, band);  \
+        else cov_assemble_kernel<DT_, false, CF><<<grid, 256, 0, s>>>(x, N, D, hyp, P, n_ell, flags, jitter, A, env, band);                       \
+    } while (0)
+    switch (D) {
+        case 1: GPMC_ASM_LAUNCH(1); break;
+        case 2: GPMC_ASM_LAUNCH(2); break;
+        case 3: GPMC_ASM_LAUNCH(3); break;
+        case 4: GPMC_ASM_LAUNCH(4); break;
+        default: GPMC_ASM_LAUNCH(0); break;
+    }
+#undef GPMC_ASM_LAUNCH
+}
+
+int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P, int kind, int flags,
                         const double *jitter, BatchView A, int B, cudaStream_t s, Envelope env, Band band)
 {
+    const int n_ell = kind_n_ell(kind, D);
     if (D > MAX_ELL || n_ell > MAX_ELL) { set_error("D=%d exceeds MAX_ELL=%d", D, MAX_ELL); return GPMC_EINVAL; }
     if (B <= 0) return 0;
     static_assert(AT == ENV_ROWS, "one tile row block is one envelope block");
@@ -383,19 +429,12 @@ int launch_cov_assemble(const double *x, int N, int D, const double *hyp, int P,
     prof_begin(KC_ASSEMBLE, s);
     if (env.blk) env_init_kernel<<<B, 128, 0, s>>>(A, env);
     if (band.w) band.width = std::min(band.width, nt - 1);
-#define GPMC_ASM_LAUNCH(DT_)                                                                                                     \
-    do {                                                                                                                          \
-        if (flags & GPMC_ASM_PRED) cov_assemble_kernel<DT_, true><<<grid, 256, 0, s>>>(x, N, D, hyp, P, n_ell, flags, jitter, A, env, band);  \
-        else cov_assemble_kernel<DT_, false><<<grid, 256, 0, s>>>(x, N, D, hyp, P, n_ell, flags, jitter, A, env, band);                       \
-    } while (0)
-    switch (D) {
-        case 1: GPMC_ASM_LAUNCH(1); break;
-        case 2: GPMC_ASM_LAUNCH(2); break;
-        case 3: GPMC_ASM_LAUNCH(3); break;
-        case 4: GPMC_ASM_LAUNCH(4); break;
-        default: GPMC_ASM_LAUNCH(0); break;
+    switch (kind_cf(kind)) {
+        case 1: cov_assemble_launch<1>(grid, s, x, N, D, hyp, P, n_ell, flags, jitter, A, env, band); break;
+        case 3: cov_assemble_launch<3>(grid, s, x, N, D, hyp, P, n_ell, flags, jitter, A, env, band); break;
+        case 5: cov_assemble_launch<5>(grid, s, x, N, D, hyp, P, n_ell, flags, jitter, A, env, band); break;
+        default: cov_assemble_launch<0>(grid, s, x, N, D, hyp, P, n_ell, flags, jitter, A, env, band); break;
     }
-#undef GPMC_ASM_LAUNCH
     prof_end(KC_ASSEMBLE, s);
     GPMC_LAUNCH_CHECK();
     return 0;

@@ -7,7 +7,9 @@
 
 namespace gpmc {
 
-// K[i][j] = sf2 * exp(-0.5 * sum_d ((x_id - z_jd)/ell_d)^2), x[N,D], z[M,D], out[N][ld]; one hyper-parameter row.
+// K[i][j] = cov_k(sf2, sum_d (u(x_id) - u(z_jd))^2) (SE: sf2 * exp(-0.5 * sum_d ((x_id - z_jd)/ell_d)^2)), x[N,D], z[M,D],
+// out[N][ld]; one hyper-parameter row.
+template <int CF>
 __global__ void __launch_bounds__(256)
 cov_cross_kernel(const double *__restrict__ x, const double *__restrict__ z, int N, int M, int D,
                  const double *__restrict__ hyp, int n_ell, double *__restrict__ out, int ld)
@@ -23,10 +25,10 @@ cov_cross_kernel(const double *__restrict__ x, const double *__restrict__ z, int
         double s = 0.0;
         for (int d = 0; d < D; ++d) {
             const double ell = s_ell[n_ell == 1 ? 0 : d];
-            const double df = x[(size_t)i * D + d] / ell - z[(size_t)j * D + d] / ell;
+            const double df = cov_u<CF>(x[(size_t)i * D + d], ell) - cov_u<CF>(z[(size_t)j * D + d], ell);
             s = __dadd_rn(s, __dmul_rn(df, df));
         }
-        out[(size_t)i * ld + j] = sf2 * exp(-0.5 * s);
+        out[(size_t)i * ld + j] = cov_k<CF>(sf2, s);
     }
 }
 
@@ -50,13 +52,19 @@ int gpmc_cov_cross(const double *x_dev, int N, const double *z_dev, int M, int D
                    double *out_dev, int ld, void *stream)
 {
     GPMC_API_LOCK();
-    const int n_ell = (kind == GPMC_KIND_SE_ARD) ? D : 1;
-    if (N <= 0 || M <= 0 || D <= 0 || D > MAX_ELL || P != n_ell + 2 || ld < M) {
+    const int n_ell = kind_n_ell(kind, D);
+    if (N <= 0 || M <= 0 || D <= 0 || D > MAX_ELL || P != n_ell + 2 || kind_cf(kind) < 0 || ld < M) {
         set_error("cov_cross: bad shape N=%d M=%d D=%d P=%d kind=%d ld=%d", N, M, D, P, kind, ld);
         return GPMC_EINVAL;
     }
     dim3 grid((M + 255) / 256 > 64 ? 64 : (M + 255) / 256, N);
-    cov_cross_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x_dev, z_dev, N, M, D, hyp_dev, n_ell, out_dev, ld);
+    cudaStream_t s = (cudaStream_t)stream;
+    switch (kind_cf(kind)) {
+        case 1: cov_cross_kernel<1><<<grid, 256, 0, s>>>(x_dev, z_dev, N, M, D, hyp_dev, n_ell, out_dev, ld); break;
+        case 3: cov_cross_kernel<3><<<grid, 256, 0, s>>>(x_dev, z_dev, N, M, D, hyp_dev, n_ell, out_dev, ld); break;
+        case 5: cov_cross_kernel<5><<<grid, 256, 0, s>>>(x_dev, z_dev, N, M, D, hyp_dev, n_ell, out_dev, ld); break;
+        default: cov_cross_kernel<0><<<grid, 256, 0, s>>>(x_dev, z_dev, N, M, D, hyp_dev, n_ell, out_dev, ld); break;
+    }
     GPMC_LAUNCH_CHECK();
     return 0;
 }

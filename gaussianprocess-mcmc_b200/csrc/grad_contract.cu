@@ -5,6 +5,8 @@
 // its zeros are the assembly's zeros, and the tiles the band bound skipped (K_ij = +0 there) would only add exact zeros.
 //     ell (iso):   K_ij s_ij / ell,  s = |x_i - x_j|^2 / ell^2      ell_d (ARD): K_ij (u_id - u_jd)^2 / ell_d,  u = x / ell
 //     sf:          2 K_ij / sf                                   sn:          2 sn on the diagonal
+//     ell (Matern, d = 1, 3, 5):   sf2 g_d(t) exp(-t) / ell,   g_1 = t, g_3 = t^2, g_5 = t^2 (1 + t) / 3   (t = sqrt(s))
+// Every term but sn's is added only where K_ij != 0, so the tiles the band skips change nothing in either family.
 // Layout: one CTA per (64-row block r, item), 8 warps x 8 rows, a lane owns two adjacent columns of every 64-column tile
 // (W rows are read with 16-byte loads).  Each thread sums its elements tile by tile in column order; the CTA reduces its
 // P partials in a fixed tree and writes them out, and a second kernel sums the row blocks of an item in order -- no
@@ -19,8 +21,8 @@ namespace gpmc {
 constexpr int GT = ENV_ROWS;        // tile edge: one envelope / band row block
 constexpr int GC_THREADS = 256;
 
-// E: partials of the length-scales (1 for iso, D for ARD); ISO: one ell for every input dimension
-template <int E, bool ISO>
+// E: partials of the length-scales (1 for iso, D for ARD); ISO: one ell for every input dimension; CF: covariance family
+template <int E, bool ISO, int CF>
 __global__ void __launch_bounds__(GC_THREADS)
 grad_contract_kernel(const double *__restrict__ x, int N, int Drt, const double *__restrict__ hyp, int P, int n_ell,
                      const double *__restrict__ alpha, int ldv, const double *__restrict__ W, int ldW, long long strideW,
@@ -43,7 +45,7 @@ grad_contract_kernel(const double *__restrict__ x, int N, int Drt, const double 
     const double *ab = alpha + (size_t)b * ldv;
     for (int e = tid; e < GT * D; e += GC_THREADS) {
         const int i = e / D, d = e - i * D;
-        s_ui[d][i] = (i0 + i < N) ? x[(size_t)(i0 + i) * D + d] / s_ell[ISO ? 0 : d] : 0.0;
+        s_ui[d][i] = (i0 + i < N) ? cov_u<CF>(x[(size_t)(i0 + i) * D + d], s_ell[ISO ? 0 : d]) : 0.0;
     }
     if (tid < GT) s_ai[tid] = (i0 + tid < N) ? ab[i0 + tid] : 0.0;
     const double sf2 = s_sf2;
@@ -58,7 +60,7 @@ grad_contract_kernel(const double *__restrict__ x, int N, int Drt, const double 
         __syncthreads();                            // the previous tile's column data has been read
         for (int e = tid; e < GT * D; e += GC_THREADS) {
             const int j = e / D, d = e - j * D;
-            s_uj[d][j] = (j0 + j < N) ? x[(size_t)(j0 + j) * D + d] / s_ell[ISO ? 0 : d] : 0.0;
+            s_uj[d][j] = (j0 + j < N) ? cov_u<CF>(x[(size_t)(j0 + j) * D + d], s_ell[ISO ? 0 : d]) : 0.0;
         }
         if (tid < GT) s_aj[tid] = (j0 + tid < N) ? ab[j0 + tid] : 0.0;
         __syncthreads();
@@ -91,9 +93,14 @@ grad_contract_kernel(const double *__restrict__ x, int N, int Drt, const double 
                         s = __dadd_rn(s, sq[d]);
                     }
                 }
-                const double k = sf2 * exp(-0.5 * s);
+                const double k = cov_k<CF>(sf2, s);
                 if (gjq == gi) acc[E + 1] += ai * ai - wij;           // sn: alpha.alpha - tr W
-                if (k != 0.0) {
+                if (CF != 0 && k != 0.0) {
+                    double cw = ai * s_aj[jl] - wij;
+                    if (gjq < gi) cw = cw + cw;
+                    acc[E] += cw * k;
+                    acc[0] += cw * matern_dk_dell_ell<CF == 0 ? 1 : CF>(sf2, s);
+                } else if (CF == 0 && k != 0.0) {
                     double cf = (ai * s_aj[jl] - wij) * k;
                     if (gjq < gi) cf = cf + cf;                       // (i, j) and (j, i)
                     acc[E] += cf;
@@ -139,12 +146,13 @@ __global__ void grad_finish_kernel(const double *__restrict__ hyp, int P, int n_
     grad[(size_t)b * P + p] = ok ? g : nan("");
 }
 
-int launch_grad_contract(const double *x, int N, int D, const double *hyp, int P, int n_ell, const double *alpha, int ldv,
+int launch_grad_contract(const double *x, int N, int D, const double *hyp, int P, int kind, const double *alpha, int ldv,
                          const double *W, int ldW, long long strideW, const int *band_w, int ldw, const int *info,
                          double *partial, double *grad, int B, cudaStream_t s)
 {
     if (B <= 0) return 0;
-    if (D > MAX_ELL || n_ell > MAX_ELL || P != n_ell + 2 || (n_ell != 1 && n_ell != D)) {
+    const int n_ell = kind_n_ell(kind, D), cf = kind_cf(kind);
+    if (D > MAX_ELL || n_ell > MAX_ELL || P != n_ell + 2 || cf < 0) {
         set_error("grad contraction: D=%d n_ell=%d P=%d", D, n_ell, P);
         return GPMC_EINVAL;
     }
@@ -152,17 +160,20 @@ int launch_grad_contract(const double *x, int N, int D, const double *hyp, int P
     const int nblk = env_blocks(N);
     dim3 grid(nblk, B);
     prof_begin(KC_GRAD, s);
-#define GPMC_GC_LAUNCH(E_, ISO_) \
-    grad_contract_kernel<E_, ISO_><<<grid, GC_THREADS, 0, s>>>(x, N, D, hyp, P, n_ell, alpha, ldv, W, ldW, strideW, band_w, ldw, partial)
-    switch (n_ell) {
-        case 1: GPMC_GC_LAUNCH(1, true); break;
-        case 2: GPMC_GC_LAUNCH(2, false); break;
-        case 3: GPMC_GC_LAUNCH(3, false); break;
-        case 4: GPMC_GC_LAUNCH(4, false); break;
-        case 5: GPMC_GC_LAUNCH(5, false); break;
-        case 6: GPMC_GC_LAUNCH(6, false); break;
-        case 7: GPMC_GC_LAUNCH(7, false); break;
-        default: GPMC_GC_LAUNCH(8, false); break;
+#define GPMC_GC_LAUNCH(E_, ISO_, CF_) \
+    grad_contract_kernel<E_, ISO_, CF_><<<grid, GC_THREADS, 0, s>>>(x, N, D, hyp, P, n_ell, alpha, ldv, W, ldW, strideW, band_w, ldw, partial)
+    if (cf == 1) GPMC_GC_LAUNCH(1, true, 1);
+    else if (cf == 3) GPMC_GC_LAUNCH(1, true, 3);
+    else if (cf == 5) GPMC_GC_LAUNCH(1, true, 5);
+    else switch (n_ell) {
+        case 1: GPMC_GC_LAUNCH(1, true, 0); break;
+        case 2: GPMC_GC_LAUNCH(2, false, 0); break;
+        case 3: GPMC_GC_LAUNCH(3, false, 0); break;
+        case 4: GPMC_GC_LAUNCH(4, false, 0); break;
+        case 5: GPMC_GC_LAUNCH(5, false, 0); break;
+        case 6: GPMC_GC_LAUNCH(6, false, 0); break;
+        case 7: GPMC_GC_LAUNCH(7, false, 0); break;
+        default: GPMC_GC_LAUNCH(8, false, 0); break;
     }
 #undef GPMC_GC_LAUNCH
     grad_finish_kernel<<<B, 32, 0, s>>>(hyp, P, n_ell, info, nblk, partial, grad);

@@ -100,8 +100,8 @@ extern "C" int gpmc_loglik_grad_batched(const double *x_dev, int N, int D, const
 {
     GPMC_API_LOCK();
     cudaStream_t s = (cudaStream_t)stream;
-    const int n_ell = (kind == GPMC_KIND_SE_ARD) ? D : 1;
-    if (N <= 0 || D <= 0 || B < 0 || (kind != GPMC_KIND_SE_ISO && kind != GPMC_KIND_SE_ARD) || P != n_ell + 2) {
+    const int n_ell = kind_n_ell(kind, D);
+    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2 || kind_cf(kind) < 0) {
         set_error("loglik_grad: bad shape N=%d D=%d B=%d P=%d kind=%d", N, D, B, P, kind);
         return GPMC_EINVAL;
     }
@@ -149,7 +149,7 @@ extern "C" int gpmc_loglik_grad_batched(const double *x_dev, int N, int D, const
         int width = -1;
         if (band_on) {
             GPMC_CUDA_CHECK(cudaMemsetAsync(band_dev, 0, 2 * sizeof(int), s));
-            int rc = launch_band_bound(x_dev, N, D, hyp_w, P, n_ell, nb, band_w, l.nblk, band_dev, xbox, s);
+            int rc = launch_band_bound(x_dev, N, D, hyp_w, P, kind, nb, band_w, l.nblk, band_dev, xbox, s);
             if (rc) return rc;
             int bh[2] = {0, 0};
             GPMC_CUDA_CHECK(cudaMemcpyAsync(bh, band_dev, sizeof(bh), cudaMemcpyDeviceToHost, s));
@@ -161,7 +161,7 @@ extern "C" int gpmc_loglik_grad_batched(const double *x_dev, int N, int D, const
             }
         }
         auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
-            int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
+            int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, kind, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
             if (rc) return rc;
             return border_set(V, N, g_w, N, nitems, s);
         };
@@ -174,7 +174,7 @@ extern "C" int gpmc_loglik_grad_batched(const double *x_dev, int N, int D, const
         if ((rc = launch_trmv(A, N, 1, 2, zv, nullptr, nullptr, l.ld, av, nb, s))) return rc;
         BatchView Wv{Wm, (long long)N * l.ld, l.ld, nullptr, nullptr};
         if ((rc = w_sequence(Wv, A, N, nb, width, s))) return rc;
-        if ((rc = launch_grad_contract(x_dev, N, D, hyp_w, P, n_ell, av, l.ld, Wm, l.ld, (long long)N * l.ld,
+        if ((rc = launch_grad_contract(x_dev, N, D, hyp_w, P, kind, av, l.ld, Wm, l.ld, (long long)N * l.ld,
                                        band_on ? band_w : nullptr, l.nblk, info_w, partial, grad_dev + (size_t)s0 * P, nb, s)))
             return rc;
     }

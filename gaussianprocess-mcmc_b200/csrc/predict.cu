@@ -27,6 +27,7 @@ namespace gpmc {
 
 // ------------------------------------------------------------------------------------ predictive path
 // Border rows of sample `item`:  row n = fm (= f - m),  row n + 1 + j = sW * K(x, xs_j)   (sW = 1 / sqrt(sn2))
+template <int CF>
 __global__ void __launch_bounds__(256)
 pred_border_kernel(BatchView A, int n, int D, int M, const double *__restrict__ x, const double *__restrict__ xs,
                    const double *__restrict__ hyp, int P, int n_ell, const double *__restrict__ fm)
@@ -45,13 +46,13 @@ pred_border_kernel(BatchView A, int n, int D, int M, const double *__restrict__ 
     double s = 0.0;
     for (int d = 0; d < D; ++d) {
         const double ell = exp(log(h[n_ell == 1 ? 0 : d]));
-        const double df = x[(size_t)i * D + d] / ell - xs[(size_t)j * D + d] / ell;
+        const double df = cov_u<CF>(x[(size_t)i * D + d], ell) - cov_u<CF>(xs[(size_t)j * D + d], ell);
         s = __dadd_rn(s, __dmul_rn(df, df));
     }
     const double sf2 = exp(2.0 * log(h[n_ell]));
     const double snl = exp(log(h[n_ell + 1]));
     const double sW = 1.0 / sqrt(snl * snl);          // sliceSample.py:259
-    dst[i] = sW * (sf2 * exp(-0.5 * s));              // np.tile(sW, (1, ns)) * Ks, :269
+    dst[i] = sW * cov_k<CF>(sf2, s);              // np.tile(sW, (1, ns)) * Ks, :269
 }
 
 // fmu[item][j] = sW * (V_j . z0),  fs2[item][j] = kss - V_j . V_j   (rows n and n + 1 + j of the factored slot)
@@ -207,8 +208,8 @@ int gpmc_predict_batched(const double *x_dev, int N, int D, const double *xs_dev
 {
     GPMC_API_LOCK();
     cudaStream_t s = (cudaStream_t)stream;
-    const int n_ell = (kind == GPMC_KIND_SE_ARD) ? D : 1;
-    if (N <= 0 || D <= 0 || D > MAX_ELL || M <= 0 || S < 0 || P != n_ell + 2) {
+    const int n_ell = kind_n_ell(kind, D);
+    if (N <= 0 || D <= 0 || D > MAX_ELL || M <= 0 || S < 0 || P != n_ell + 2 || kind_cf(kind) < 0) {
         set_error("predict: bad shape N=%d D=%d M=%d S=%d P=%d kind=%d", N, D, M, S, P, kind);
         return GPMC_EINVAL;
     }
@@ -235,10 +236,16 @@ int gpmc_predict_batched(const double *x_dev, int N, int D, const double *xs_dev
         int *info_w = info_dev + s0;
         BatchView A{mats, (long long)l.mat_elems, l.ld, nullptr, nullptr};
         auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
-            int r = launch_cov_assemble(x_dev, N, D, hyp_w, P, n_ell, GPMC_ASM_PRED | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s);
+            int r = launch_cov_assemble(x_dev, N, D, hyp_w, P, kind, GPMC_ASM_PRED | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s);
             if (r) return r;
             prof_begin(KC_VEC, s);
-            pred_border_kernel<<<dim3((l.ld + 255) / 256, 1 + M, nitems), 256, 0, s>>>(V, N, D, M, x_dev, xs_dev, hyp_w, P, n_ell, fm_w);
+            const dim3 grid((l.ld + 255) / 256, 1 + M, nitems);
+            switch (kind_cf(kind)) {
+                case 1: pred_border_kernel<1><<<grid, 256, 0, s>>>(V, N, D, M, x_dev, xs_dev, hyp_w, P, n_ell, fm_w); break;
+                case 3: pred_border_kernel<3><<<grid, 256, 0, s>>>(V, N, D, M, x_dev, xs_dev, hyp_w, P, n_ell, fm_w); break;
+                case 5: pred_border_kernel<5><<<grid, 256, 0, s>>>(V, N, D, M, x_dev, xs_dev, hyp_w, P, n_ell, fm_w); break;
+                default: pred_border_kernel<0><<<grid, 256, 0, s>>>(V, N, D, M, x_dev, xs_dev, hyp_w, P, n_ell, fm_w); break;
+            }
             prof_end(KC_VEC, s);
             GPMC_LAUNCH_CHECK();
             return 0;
@@ -272,8 +279,8 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
 {
     GPMC_API_LOCK();
     cudaStream_t s = (cudaStream_t)stream;
-    const int n_ell = (kind == GPMC_KIND_SE_ARD) ? D : 1;
-    if (N <= 0 || D <= 0 || D > MAX_ELL || B < 0 || P != n_ell + 2 || max_trips <= 0 || (tape_theta && tape_trips < 1)) {
+    const int n_ell = kind_n_ell(kind, D);
+    if (N <= 0 || D <= 0 || D > MAX_ELL || B < 0 || P != n_ell + 2 || kind_cf(kind) < 0 || max_trips <= 0 || (tape_theta && tape_trips < 1)) {
         set_error("ess_sweep: bad shape N=%d D=%d B=%d P=%d kind=%d max_trips=%d", N, D, B, P, kind, max_trips);
         return GPMC_EINVAL;
     }
@@ -299,7 +306,7 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
         if (ld != N) GPMC_CUDA_CHECK(cudaMemset2DAsync(mats + N, (size_t)ld * 8, 0, (size_t)(ld - N) * 8, (size_t)N * B, s));
         // K = covK.RBF(...).getCovMatrix(x, 'train') (:38-39), L = jitchol(K), nu = L z
         auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
-            return launch_cov_assemble(x_dev, N, D, hyp_dev, P, n_ell, GPMC_ASM_LOWER_ONLY, jit, V, nitems, s);
+            return launch_cov_assemble(x_dev, N, D, hyp_dev, P, kind, GPMC_ASM_LOWER_ONLY, jit, V, nitems, s);
         };
         auto diag = [&](const double *h) { return exp(2.0 * log(h[n_ell])); };
         if ((rc = factor_wave(fill, diag, A, N, B, hyp_dev, P, info_dev, W, jit_dev, map_dev, jitter_policy, 0, s))) return rc;

@@ -100,7 +100,7 @@ static bool debug_on()
 }
 
 struct AuxCtx {
-    const double *x; int N, D, P, n_ell;
+    const double *x; int N, D, P, kind;
     SweepBuffers *w;
     cudaStream_t s;
     int jitter_policy;
@@ -192,11 +192,11 @@ static int aux_fill(const AuxCtx &c, BatchView V1, int nitems, const double *jit
 {
     SweepBuffers &w = *c.w;
     int rc;
-    if ((rc = launch_cov_assemble(c.x, c.N, c.D, w.theta, c.P, c.n_ell, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V1, nitems, c.s))) return rc;
+    if ((rc = launch_cov_assemble(c.x, c.N, c.D, w.theta, c.P, c.kind, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V1, nitems, c.s))) return rc;
     if ((rc = border_set(V1, w.n, w.g, w.ldv, nitems, c.s))) return rc;
     if (g_sds_literal) {
         BatchView Krows{V1.base + (size_t)(w.n + 1) * w.ld, V1.stride, V1.ld, V1.map, V1.count};
-        if ((rc = launch_cov_assemble(c.x, c.N, c.D, w.theta, c.P, c.n_ell, 0, nullptr, Krows, nitems, c.s))) return rc;     // full K, no S
+        if ((rc = launch_cov_assemble(c.x, c.N, c.D, w.theta, c.P, c.kind, 0, nullptr, Krows, nitems, c.s))) return rc;     // full K, no S
     }
     return 0;
 }
@@ -213,7 +213,7 @@ static int aux_form_R(const AuxCtx &c, BatchView V1, BatchView V2, int nitems, b
         return r_sequence(V2, V1, w.n, nitems, w.svec, w.ldv, s);
     }
     // R = K - X X^T with X = K L^-T in rows n+1 .. 2n of V1 (:197-198)
-    if ((rc = launch_cov_assemble(c.x, c.N, c.D, w.theta, c.P, c.n_ell, GPMC_ASM_LOWER_ONLY, nullptr, V2, nitems, s))) return rc;
+    if ((rc = launch_cov_assemble(c.x, c.N, c.D, w.theta, c.P, c.kind, GPMC_ASM_LOWER_ONLY, nullptr, V2, nitems, s))) return rc;
     GemmArgs g{};
     g.C = V2;
     g.A = Operand{V1.base + (size_t)(w.n + 1) * w.ld, V1.stride, V1.ld};
@@ -454,7 +454,7 @@ void sds_loop_stats(long long *rounds, long long *idle_rounds, long long *ladder
 }
 
 static int sds_sweep_resident(const double *x_dev, const double *y_dev, int N, int D, double *F_dev, double *hyp_dev, int B, int P,
-                              int n_ell, const double *scale_dev, const double *prior_k_dev, const double *prior_theta_dev, int iter,
+                              int kind, const double *scale_dev, const double *prior_k_dev, const double *prior_theta_dev, int iter,
                               double my, double lower, double upper, unsigned long long seed, unsigned chain0,
                               const double *tape_z, const double *tape_v, const double *tape_u0, const double *tape_U, int tape_trips,
                               int max_trips, int jitter_policy, int *ntrips_dev, double *loglik_dev, int *status_dev,
@@ -471,7 +471,7 @@ static int sds_sweep_resident(const double *x_dev, const double *y_dev, int N, i
         explicit SchedulePin(int B) { set_schedule_batch(B); }
         ~SchedulePin() { set_schedule_batch(0); }
     } pin(g_sds_pin_schedule ? std::min(cap, B) : 0);
-    AuxCtx ctx{x_dev, N, D, P, n_ell, &w, s, jitter_policy};
+    AuxCtx ctx{x_dev, N, D, P, kind, &w, s, jitter_policy};
     int rc;
     // every slot free, nothing admitted yet
     GPMC_CUDA_CHECK(cudaMemsetAsync(w.chain_of, 0xFF, (size_t)cap * 4, s));
@@ -687,8 +687,8 @@ int gpmc_sds_run(const double *x_dev, const double *y_dev, int N, int D, double 
 {
     GPMC_API_LOCK();
     cudaStream_t s = (cudaStream_t)stream;
-    const int n_ell = (kind == GPMC_KIND_SE_ARD) ? D : 1;
-    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2 || max_trips <= 0 || n_iters < 0 || (hist_f_dev && (thin <= 0 || n_keep <= 0))) {
+    const int n_ell = kind_n_ell(kind, D);
+    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2 || kind_cf(kind) < 0 || max_trips <= 0 || n_iters < 0 || (hist_f_dev && (thin <= 0 || n_keep <= 0))) {
         set_error("sds_run: bad shape N=%d D=%d B=%d P=%d kind=%d max_trips=%d n_iters=%d thin=%d n_keep=%d", N, D, B, P, kind, max_trips,
                   n_iters, thin, n_keep);
         return GPMC_EINVAL;
@@ -709,7 +709,7 @@ int gpmc_sds_run(const double *x_dev, const double *y_dev, int N, int D, double 
     RunSpec run;
     run.n_iters = n_iters; run.hist_hyp = hist_hyp_dev; run.hist_loglik = hist_loglik_dev; run.hist_trips = hist_trips_dev;
     run.hist_f = hist_f_dev; run.thin = thin; run.n_keep = n_keep; run.n_exhausted = n_exhausted_dev;
-    return sds_sweep_resident(x_dev, y_dev, N, D, F_dev, hyp_dev, B, P, n_ell, scale_dev, prior_k_dev, prior_theta_dev, iter_begin,
+    return sds_sweep_resident(x_dev, y_dev, N, D, F_dev, hyp_dev, B, P, kind, scale_dev, prior_k_dev, prior_theta_dev, iter_begin,
                               my, lower, upper, seed, chain0, nullptr, nullptr, nullptr, nullptr, 0, max_trips, jitter_policy,
                               nullptr, nullptr, nullptr, w, s, &run);
 }
@@ -730,8 +730,8 @@ int gpmc_sds_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
 {
     GPMC_API_LOCK();
     cudaStream_t s = (cudaStream_t)stream;
-    const int n_ell = (kind == GPMC_KIND_SE_ARD) ? D : 1;
-    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2 || max_trips <= 0) {
+    const int n_ell = kind_n_ell(kind, D);
+    if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2 || kind_cf(kind) < 0 || max_trips <= 0) {
         set_error("sds_sweep: bad shape N=%d D=%d B=%d P=%d kind=%d max_trips=%d", N, D, B, P, kind, max_trips);
         return GPMC_EINVAL;
     }
@@ -753,11 +753,11 @@ int gpmc_sds_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
         GPMC_CUDA_CHECK(cudaMemset2DAsync(w.buf2 + N, (size_t)w.ld * 8, 0, (size_t)(w.ld - N) * 8, (size_t)(N + 1) * cap, s));
     }
     if (g_sds_mode == 0)
-        return sds_sweep_resident(x_dev, y_dev, N, D, F_dev, hyp_dev, B, P, n_ell, scale_dev, prior_k_dev, prior_theta_dev, iter,
+        return sds_sweep_resident(x_dev, y_dev, N, D, F_dev, hyp_dev, B, P, kind, scale_dev, prior_k_dev, prior_theta_dev, iter,
                                   my, lower, upper, seed, chain0, tape_z, tape_v, tape_u0, tape_U, tape_trips, max_trips,
                                   jitter_policy, ntrips_dev, loglik_dev, status_dev, w, s);
     // ---- wave loop (gpmc_set_tuning(6, 1)): kept for A/B and as the reference the resident loop is tested against
-    AuxCtx ctx{x_dev, N, D, P, n_ell, &w, s, jitter_policy};
+    AuxCtx ctx{x_dev, N, D, P, kind, &w, s, jitter_policy};
     std::vector<int> active;
     for (int c0 = 0; c0 < B; c0 += cap) {
         const int nb = std::min(cap, B - c0);

@@ -2,8 +2,8 @@
 reference uses (``framework.py:158,208`` ``updOpt``, ``demoRegression.py:78,110-115``, and ``plotResult.py:100``, where a
 ``GPR`` is the ``model`` that ``inf_mcmc(f, model)`` reads ``x, y, xs, meanfunc, covfunc, likfunc`` from).
 
-Limited to what the reference needs: a Gaussian likelihood (``likK.Gauss``), a zero mean and ``covK.RBF`` /
-``covK.RBFard``.  The negative log marginal likelihood and its gradient come from ``ops.loglik_grad_batched``
+Limited to a Gaussian likelihood (``likK.Gauss``), a zero mean and ``covK.RBF`` / ``covK.RBFard`` (what the reference
+needs) or ``covK.Matern`` (d = 1, 3, 5).  The negative log marginal likelihood and its gradient come from ``ops.loglik_grad_batched``
 (``gpmc_loglik_grad_batched``: assembly, Cholesky, ``A^-1`` and the gradient contraction on the device); the predictive
 from ``ops.predict_batched``.  Hyper-parameters are kept on pyGPs' log scale (``covfunc.hyp``, ``log(likfunc.sn)``)."""
 import numpy as np
@@ -62,8 +62,8 @@ class GPR(object):
         if mean is not None:
             raise NotImplementedError('GPR: only the zero mean is supported')
         if kernel is not None:
-            if not isinstance(kernel, covK.RBF):
-                raise NotImplementedError('GPR: only covK.RBF / covK.RBFard kernels are supported')
+            if not isinstance(kernel, (covK.RBF, covK.Matern)):
+                raise NotImplementedError('GPR: only covK.RBF / covK.RBFard / covK.Matern kernels are supported')
             self.covfunc = kernel
 
     def setNoise(self, log_sigma=np.log(0.1)):
@@ -79,6 +79,11 @@ class GPR(object):
         self.likRange = likRange
 
     # ------------------------------------------------------------------ hyper-parameters
+    def _kind_kw(self):
+        # an RBF / RBFard row is SE iso / ARD by its width (the ops default); a Matern kernel names its kind
+        kind = getattr(self.covfunc, 'kind', None)
+        return {} if kind is None else {'kind': kind}
+
     def _log_hyp(self):
         return np.concatenate([np.asarray(self.covfunc.hyp, dtype=np.float64), [np.log(self.likfunc.sn)]])
 
@@ -90,7 +95,7 @@ class GPR(object):
     def _nlz_and_grad(self, log_hyp):
         """``nlZ`` and its gradient with respect to the log hyper-parameters (pyGPs' sign and scale)."""
         theta = np.exp(np.asarray(log_hyp, dtype=np.float64))
-        ll, grad, info = ops.loglik_grad_batched(self.x, self.y.reshape(1, -1), theta[None])
+        ll, grad, info = ops.loglik_grad_batched(self.x, self.y.reshape(1, -1), theta[None], **self._kind_kw())
         ll, grad = float(_np(ll)[0]), _np(grad)[0]
         if int(_np(info)[0]) != 0 or not np.isfinite(ll) or not np.all(np.isfinite(grad)):
             return np.inf, np.zeros_like(theta)
@@ -135,7 +140,7 @@ class GPR(object):
         M = self.xs.shape[0]
         theta = np.exp(self._log_hyp())
         m = self.meanfunc.getMean(self.x)
-        fmu, fs2, info = ops.predict_batched(self.x, self.xs, (self.y - m).reshape(1, -1), theta[None])
+        fmu, fs2, info = ops.predict_batched(self.x, self.xs, (self.y - m).reshape(1, -1), theta[None], **self._kind_kw())
         if int(_np(info)[0]) != 0:
             raise np.linalg.LinAlgError('not positive definite, even with jitter.')
         fm = self.meanfunc.getMean(self.xs) + _np(fmu).reshape(M, 1)

@@ -5,7 +5,8 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from ._lib import (KIND_SE_ISO, KIND_SE_ARD, ASM_ADD_S, ASM_LOWER_ONLY, JITTER_NONE, JITTER_PYGPS,
+from ._lib import (KIND_SE_ISO, KIND_SE_ARD, KIND_MATERN1, KIND_MATERN3, KIND_MATERN5, ASM_ADD_S, ASM_LOWER_ONLY,
+                   JITTER_NONE, JITTER_PYGPS,
                    OP_POTRF, OP_LOGLIK, OP_LOGLIK_GRAD, GpmcError)
 
 
@@ -32,6 +33,12 @@ def kind_of(D, P):
     raise ValueError('hyp has %d columns; expected 3 (iso) or D+2=%d (ARD)' % (P, D + 2))
 
 
+def _kind(D, P, kind):
+    """The covariance kind of a call: ``kind`` when given (``KIND_*``; the library rejects a kind that does not fit P),
+    else SE iso or ARD inferred from P by ``kind_of``.  A Matern kind must be named: P = 3 also fits SE iso."""
+    return kind_of(D, P) if kind is None else int(kind)
+
+
 class Workspace(object):
     """Caller-owned device scratch, grown on demand and reused across calls."""
 
@@ -48,7 +55,7 @@ class Workspace(object):
 _default_ws = Workspace()
 
 
-def cov_assemble(x, hyp, add_S=False, lower_only=False, jitter=None, out=None, ld=None):
+def cov_assemble(x, hyp, add_S=False, lower_only=False, jitter=None, out=None, ld=None, kind=None):
     """Batched K (or K+S) for ``hyp[B,P]`` over inputs ``x[N,D]`` -> ``A[B,N,ld]`` (device tensor).
 
     Mirrors ``covK.RBF(np.log(ll), np.log(sf)).getCovMatrix(x, mode='train')`` (+ the S diagonal of
@@ -71,7 +78,7 @@ def cov_assemble(x, hyp, add_S=False, lower_only=False, jitter=None, out=None, l
             out[:, :, N:] = 0.0
     jit = None if jitter is None else _f64_cuda(torch, jitter, 'jitter')
     flags = (ASM_ADD_S if add_S else 0) | (ASM_LOWER_ONLY if lower_only else 0)
-    rc = lib.gpmc_cov_assemble(x.data_ptr(), N, D, hyp.data_ptr(), B, P, kind_of(D, P), flags,
+    rc = lib.gpmc_cov_assemble(x.data_ptr(), N, D, hyp.data_ptr(), B, P, _kind(D, P, kind), flags,
                                None if jit is None else jit.data_ptr(), out.data_ptr(), ld, _stream_ptr(torch))
     _lib.check(rc, 'gpmc_cov_assemble')
     return out
@@ -99,7 +106,7 @@ def potrf_batched(A, jitter_policy=JITTER_NONE, zero_upper=True, n=None, workspa
     return info
 
 
-def loglik_batched(x, g, hyp, jitter_policy=JITTER_PYGPS, workspace=None, max_wave=None):
+def loglik_batched(x, g, hyp, jitter_policy=JITTER_PYGPS, workspace=None, max_wave=None, kind=None):
     """``loglik[b] = log N(g_b; 0, K(hyp_b) + S(hyp_b))`` for device tensors; returns ``(loglik[B], info[B])``.
 
     The metric's unit (``sliceSample.py:136-137,183-190,196,147``), B items in waves."""
@@ -132,13 +139,13 @@ def loglik_batched(x, g, hyp, jitter_policy=JITTER_PYGPS, workspace=None, max_wa
         need = max(one, min(need, (free + have) * 6 // 10))
     ws = wsobj.get(torch, need)
     use_bytes = need if max_wave is not None else ws.numel()       # max_wave: really limit the wave (tests)
-    rc = lib.gpmc_loglik_batched(x.data_ptr(), N, D, g.data_ptr(), hyp.data_ptr(), B, P, kind_of(D, P), jitter_policy,
+    rc = lib.gpmc_loglik_batched(x.data_ptr(), N, D, g.data_ptr(), hyp.data_ptr(), B, P, _kind(D, P, kind), jitter_policy,
                                  out.data_ptr(), info.data_ptr(), ws.data_ptr(), use_bytes, _stream_ptr(torch))
     _lib.check(rc, 'gpmc_loglik_batched')
     return out, info
 
 
-def loglik_grad_batched(x, g, hyp, jitter_policy=JITTER_PYGPS, workspace=None, max_wave=None):
+def loglik_grad_batched(x, g, hyp, jitter_policy=JITTER_PYGPS, workspace=None, max_wave=None, kind=None):
     """``log N(g_b; 0, K(hyp_b) + sn_b^2 I)`` and its gradient with respect to the natural-scale row ``hyp[b] = (ell..,
     sf, sn)``; returns ``(loglik[B], grad[B,P], info[B])`` CUDA tensors (``gpmc_loglik_grad_batched``, include/gpmc.h).
 
@@ -172,14 +179,14 @@ def loglik_grad_batched(x, g, hyp, jitter_policy=JITTER_PYGPS, workspace=None, m
         need = max(one, min(need, (free + have) * 6 // 10))
     ws = wsobj.get(torch, need)
     use_bytes = need if max_wave is not None else ws.numel()
-    rc = lib.gpmc_loglik_grad_batched(x.data_ptr(), N, D, g.data_ptr(), hyp.data_ptr(), B, P, kind_of(D, P), jitter_policy,
+    rc = lib.gpmc_loglik_grad_batched(x.data_ptr(), N, D, g.data_ptr(), hyp.data_ptr(), B, P, _kind(D, P, kind), jitter_policy,
                                       out.data_ptr(), grad.data_ptr(), info.data_ptr(), ws.data_ptr(), use_bytes,
                                       _stream_ptr(torch))
     _lib.check(rc, 'gpmc_loglik_grad_batched')
     return out, grad, info
 
 
-def loglik_host(x, g, hyp, jitter_policy=JITTER_PYGPS):
+def loglik_host(x, g, hyp, jitter_policy=JITTER_PYGPS, kind=None):
     """Same unit for numpy inputs through the library's own pinned staging + stream (the end-to-end call)."""
     _lib.require_cuda()
     lib = _lib.load()
@@ -198,7 +205,7 @@ def loglik_host(x, g, hyp, jitter_policy=JITTER_PYGPS):
     info = np.empty(B, dtype=np.int32)
     if B == 0:
         return out, info
-    rc = lib.gpmc_loglik_host(x.ctypes.data, N, D, g.ctypes.data, hyp.ctypes.data, B, P, kind_of(D, P), jitter_policy,
+    rc = lib.gpmc_loglik_host(x.ctypes.data, N, D, g.ctypes.data, hyp.ctypes.data, B, P, _kind(D, P, kind), jitter_policy,
                               out.ctypes.data, info.ctypes.data)
     _lib.check(rc, 'gpmc_loglik_host')
     return out, info
@@ -225,7 +232,7 @@ class Tape(object):
 
 
 def sds_sweep(x, y, F, Hyp, scale, it, my=None, tape=None, seed=0, chain0=0, max_trips=64, prior_k=None,
-              prior_theta=None, jitter_policy=JITTER_PYGPS, workspace=None, chains_per_wave=None):
+              prior_theta=None, jitter_policy=JITTER_PYGPS, workspace=None, chains_per_wave=None, kind=None):
     """One surrogate-data slice-sampling transition for every chain (``sliceSample.py:76-163``), in place.
 
     ``F[B,N]`` and ``Hyp[B,P]`` are CUDA float64 tensors holding the chains' current ``(f, theta)``; on return
@@ -243,7 +250,7 @@ def sds_sweep(x, y, F, Hyp, scale, it, my=None, tape=None, seed=0, chain0=0, max
     B, P = Hyp.shape
     if F.shape[0] != B:
         raise ValueError('F and Hyp disagree on the number of chains')
-    kind = kind_of(D, P)
+    kind = _kind(D, P, kind)
     if my is None:
         my = float(np.mean(np.asarray(y.cpu() if hasattr(y, 'cpu') else y, dtype=np.float64)))      # sliceSample.py:102
     y = _f64_cuda(torch, y, 'y').reshape(-1)
@@ -292,7 +299,7 @@ def sds_sweep(x, y, F, Hyp, scale, it, my=None, tape=None, seed=0, chain0=0, max
 
 
 def sds_run(x, y, F, Hyp, scale, it0, n_iters, my=None, seed=0, chain0=0, max_trips=64, prior_k=None, prior_theta=None,
-            jitter_policy=JITTER_PYGPS, workspace=None, chains_per_wave=None, keep_f_every=0):
+            jitter_policy=JITTER_PYGPS, workspace=None, chains_per_wave=None, keep_f_every=0, kind=None):
     """``n_iters`` surrogate-data slice-sampling transitions per chain in ONE call (``gpmc_sds_run``): the caller loop of
     ``framework.py:68-75`` for every chain, each chain advancing on its own inside the resident device loop.
 
@@ -310,7 +317,7 @@ def sds_run(x, y, F, Hyp, scale, it0, n_iters, my=None, seed=0, chain0=0, max_tr
     if not (Hyp.is_cuda and Hyp.dtype == torch.float64 and Hyp.is_contiguous() and Hyp.dim() == 2):
         raise ValueError('Hyp must be a contiguous CUDA float64 tensor [B, P]')
     B, P = Hyp.shape
-    kind = kind_of(D, P)
+    kind = _kind(D, P, kind)
     if my is None:
         my = float(np.mean(np.asarray(y.cpu() if hasattr(y, 'cpu') else y, dtype=np.float64)))
     y = _f64_cuda(torch, y, 'y').reshape(-1)
@@ -404,7 +411,7 @@ def trsv_lower(L, rhs, want_lognormal=False):
     return (out[:, :N], quad) if want_lognormal else out[:, :N]
 
 
-def cov_cross(x, z, hyp):
+def cov_cross(x, z, hyp, kind=None):
     """``covK.RBF(...).getCovMatrix(x=x, z=z, mode='cross')`` -> device tensor ``[N, M]`` (``sliceSample.py:263``)."""
     torch = _lib.require_cuda()
     lib = _lib.load()
@@ -417,7 +424,7 @@ def cov_cross(x, z, hyp):
     N, D = x.shape
     M = z.shape[0]
     out = torch.empty((N, M), dtype=torch.float64, device='cuda')
-    rc = lib.gpmc_cov_cross(x.data_ptr(), N, z.data_ptr(), M, D, hyp.data_ptr(), hyp.numel(), kind_of(D, hyp.numel()),
+    rc = lib.gpmc_cov_cross(x.data_ptr(), N, z.data_ptr(), M, D, hyp.data_ptr(), hyp.numel(), _kind(D, hyp.numel(), kind),
                             out.data_ptr(), M, _stream_ptr(torch))
     _lib.check(rc, 'gpmc_cov_cross')
     return out
@@ -440,7 +447,7 @@ def tg2_loglik(y, mu, sn, lower, upper, my=0.0):
     return out
 
 
-def predict_batched(x, xs, fm, hyp, jitter_policy=JITTER_PYGPS, workspace=None):
+def predict_batched(x, xs, fm, hyp, jitter_policy=JITTER_PYGPS, workspace=None, kind=None):
     """``inf_mcmc``'s linear algebra (``sliceSample.py:256-270``) for S stored samples at once.
 
     ``fm[S, N]`` = ``f_s - m`` (centred latent samples), ``hyp[S, P]`` their hyper-parameters, ``xs[M, D]`` test inputs.
@@ -471,7 +478,7 @@ def predict_batched(x, xs, fm, hyp, jitter_policy=JITTER_PYGPS, workspace=None):
     if S == 0 or M == 0:
         return fmu, fs2, info
     ws = (workspace or _default_ws).get(torch, lib.gpmc_predict_workspace_bytes(N, M, S))
-    rc = lib.gpmc_predict_batched(x.data_ptr(), N, D, xs.data_ptr(), M, fm.data_ptr(), hyp.data_ptr(), S, P, kind_of(D, P),
+    rc = lib.gpmc_predict_batched(x.data_ptr(), N, D, xs.data_ptr(), M, fm.data_ptr(), hyp.data_ptr(), S, P, _kind(D, P, kind),
                                   jitter_policy, fmu.data_ptr(), fs2.data_ptr(), info.data_ptr(), ws.data_ptr(), ws.numel(),
                                   _stream_ptr(torch))
     _lib.check(rc, 'gpmc_predict_batched')
@@ -490,7 +497,8 @@ class EssTape(object):
         self.z = None if z is None else np.ascontiguousarray(np.atleast_2d(z), dtype=np.float64)
 
 
-def ess_sweep(x, y, F, Hyp, it=0, my=None, tape=None, seed=0, chain0=0, max_trips=256, jitter_policy=JITTER_PYGPS, workspace=None):
+def ess_sweep(x, y, F, Hyp, it=0, my=None, tape=None, seed=0, chain0=0, max_trips=256, jitter_policy=JITTER_PYGPS, workspace=None,
+              kind=None):
     """One elliptical-slice update of ``F[B,N]`` in place (``sliceSample.py:15-74``) for B chains with ``Hyp[B,P]``.
     Returns ``(ntrips[B], status[B], info[B])`` device tensors."""
     torch = _lib.require_cuda()
@@ -528,7 +536,7 @@ def ess_sweep(x, y, F, Hyp, it=0, my=None, tape=None, seed=0, chain0=0, max_trip
             t_z = torch.tensor(tape.z).cuda()
     ws = (workspace or _default_ws).get(torch, lib.gpmc_ess_workspace_bytes(N, B))
     ptr = lambda t: None if t is None else t.data_ptr()
-    rc = lib.gpmc_ess_sweep(x.data_ptr(), y.data_ptr(), N, D, F.data_ptr(), Hyp.data_ptr(), B, P, kind_of(D, P),
+    rc = lib.gpmc_ess_sweep(x.data_ptr(), y.data_ptr(), N, D, F.data_ptr(), Hyp.data_ptr(), B, P, _kind(D, P, kind),
                             my, 0.0 - my, 100.0 - my, int(seed), int(chain0), int(it),
                             ptr(t_nu), ptr(t_z), ptr(t_u), ptr(t_th), ttrips, int(max_trips), jitter_policy,
                             ntrips.data_ptr(), status.data_ptr(), info.data_ptr(), ws.data_ptr(), ws.numel(), _stream_ptr(torch))

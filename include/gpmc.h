@@ -23,8 +23,10 @@
  *  - the caller owns every buffer including workspace, sized by
  *    gpmc_workspace_bytes().
  *  - hyper-parameter rows are natural scale, hyp[b] = (ell_1..ell_E, sf, sn)
- *    with E = 1 (GPMC_KIND_SE_ISO, the reference's covK.RBF) or E = D
- *    (GPMC_KIND_SE_ARD); P = E + 2.
+ *    with E = 1 (GPMC_KIND_SE_ISO, the reference's covK.RBF, and the Matern
+ *    kinds) or E = D (GPMC_KIND_SE_ARD); P = E + 2.  Every entry point that
+ *    takes `kind` accepts the five kinds below and returns GPMC_EINVAL for any
+ *    other value, or for a P that does not fit the kind.
  *  - threading: like the reference (one Python thread, sliceSample.py uses the
  *    global numpy RNG) the library is meant for one host thread per process and
  *    one process per GPU; it keeps per-process state (side streams and events of
@@ -50,8 +52,16 @@ extern "C" {
 
 #define GPMC_VERSION 100
 
+/* covariance functions (`kind`), with u = x / ell (SE) or u = sqrt(d) x / ell (Matern), s = |u_i - u_j|^2, t = sqrt(s):
+ *   SE:          K = sf2 * exp(-0.5 * s)                            (pyGPs 1.3.4 cov.RBF / cov.RBFard)
+ *   Matern d:    K = sf2 * (f_d(t) * exp(-t)),  f_1 = 1, f_3 = 1 + t, f_5 = 1 + t * (1 + t / 3)
+ *                (pyGPs 1.3.4 cov.Matern(log_ell, d, log_sigma) as restated in oracle/matern_oracle.py; d = 2 nu, isotropic)
+ * sf2 = sf^2; K_ii = sf2 for every kind. */
 #define GPMC_KIND_SE_ISO 0
 #define GPMC_KIND_SE_ARD 1
+#define GPMC_KIND_MATERN1 2
+#define GPMC_KIND_MATERN3 3
+#define GPMC_KIND_MATERN5 4
 
 /* flags of gpmc_cov_assemble */
 #define GPMC_ASM_ADD_S      1   /* add S_ii (sliceSample.py:184-190) on the diagonal */
@@ -87,7 +97,7 @@ size_t gpmc_workspace_bytes(int op, int N, int D, int B);
  * Fused covariance assembly.  Replaces
  *   covK.RBF(np.log(ll), np.log(sf)).getCovMatrix(x, mode='train')   sliceSample.py:104-105,136-137
  *   S build / K+S                                                     sliceSample.py:183-190,207
- * A[b] = sf_b^2 * exp(-0.5 * sum_d ((x_id - x_jd)/ell_bd)^2)  (+ S_ii on the diagonal with
+ * A[b] = sf_b^2 * exp(-0.5 * sum_d ((x_id - x_jd)/ell_bd)^2), or the Matern K of `kind`  (+ S_ii on the diagonal with
  * GPMC_ASM_ADD_S; + jitter_dev[b] when jitter_dev != NULL).  Full symmetric fill unless
  * GPMC_ASM_LOWER_ONLY.  x_dev[N,D]; hyp_dev[B,P]; A_dev[B][N][ld], ld >= N, ld even.
  */
@@ -129,6 +139,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
  *   d loglik / d th_p   = 0.5 sum_ij (alpha_i alpha_j - W_ij) dA_ij/d th_p,   alpha = A^-1 g,  W = A^-1
  *     dA_ij / d ell     = K_ij r2_ij / ell^3              (GPMC_KIND_SE_ISO, r2 = |x_i - x_j|^2)
  *     dA_ij / d ell_d   = K_ij (x_id - x_jd)^2 / ell_d^3  (GPMC_KIND_SE_ARD)
+ *     dA_ij / d ell     = sf2 g_d(t) exp(-t) / ell       (Matern d, t as above; g_1 = t, g_3 = t^2, g_5 = t^2 (1 + t) / 3)
  *     dA_ij / d sf      = 2 K_ij / sf
  *     dA / d sn         = 2 sn I              ->  sn (alpha.alpha - tr W)
  * grad_dev[B,P] is taken with respect to the NATURAL-scale row hyp[b] = (ell.., sf, sn).  An item the jitter ladder
