@@ -15,7 +15,7 @@ KIND_MATERN1, KIND_MATERN3, KIND_MATERN5 = 2, 3, 4
 ASM_ADD_S, ASM_LOWER_ONLY = 1, 2
 JITTER_NONE, JITTER_PYGPS = 0, 1
 INFO_NOT_PD = -1
-OP_POTRF, OP_LOGLIK, OP_SDS, OP_LOGLIK_GRAD = 1, 2, 3, 4
+OP_POTRF, OP_LOGLIK, OP_SDS, OP_LOGLIK_GRAD, OP_MARGINAL = 1, 2, 3, 4, 5
 KC_NAMES = ('assemble', 'gemm_update', 'potf2', 'panel_trsm', 'solve_reduce', 'tri_inverse', 'syrk_R', 'vector_control',
             'band_clear', 'grad_contract')
 
@@ -43,6 +43,9 @@ SIGNATURES = {
     'gpmc_sds_run': (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _i, _i,
                           ctypes.c_double, ctypes.c_double, ctypes.c_double, ctypes.c_ulonglong, ctypes.c_uint, _i, _i,
                           _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _sz, _vp]),
+    'gpmc_marginal_run': (_i, [_vp, _i, _i, _vp, ctypes.c_double, _vp, _i, _i, _i, _vp, _vp, _vp, _i, _i, _i,
+                               ctypes.c_ulonglong, ctypes.c_uint, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'gpmc_marginal_rounds': (_i, [_i, _vp, _vp]),
     'gpmc_aux_workspace_bytes': (_sz, [_i]),
     'gpmc_aux_var_model': (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     'gpmc_trsv_lower_batched': (_i, [_vp, _i, _i, ctypes.c_longlong, _vp, _i, _i, _vp, _vp, _vp]),

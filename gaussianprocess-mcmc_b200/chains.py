@@ -25,10 +25,15 @@ class ChainEnsemble(object):
 
     ``F0[B,N]``/``Hyp0[B,P]`` are the GLOBAL initial states (every rank passes the same arrays, or only its shard
     with ``sharded_input=True``); ``sweep(it)`` advances every local chain by one transition and returns the gathered
-    ``(Hyp[B,P], loglik[B], ntrips[B])`` as numpy arrays on every rank."""
+    ``(Hyp[B,P], loglik[B], ntrips[B])`` as numpy arrays on every rank.
+
+    ``likelihood='gauss'``: the chains sample the hyper-parameters of GP regression with a Gaussian likelihood, the
+    latent f integrated out (``ops.marginal_run``; ``F0`` may be None, loglik is ``log N(y - mean(y); 0, K + S)``, and
+    ``burn_in`` is the iteration up to which the noise stays frozen).  ``'tg2'`` (default) is the surrogate-data slice
+    sampler of the reference's truncated-Gaussian model."""
 
     def __init__(self, x, y, F0, Hyp0, scale, seed=0, max_trips=64, sweeper=None, gather_f=False, sharded_input=False,
-                 distributed=True, strict=False, kind=None):
+                 distributed=True, strict=False, kind=None, likelihood='tg2', burn_in=500):
         self.x = np.asarray(x, dtype=np.float64)
         if self.x.ndim == 1:
             self.x = self.x.reshape(-1, 1)
@@ -37,6 +42,9 @@ class ChainEnsemble(object):
         self.scale = np.asarray(scale, dtype=np.float64).reshape(-1)
         self.seed, self.max_trips, self.gather_f = int(seed), int(max_trips), gather_f
         self.kind = kind                   # covariance kind (ops.KIND_*); None: SE iso / ARD from the width of Hyp0
+        if likelihood not in ('tg2', 'gauss'):
+            raise ValueError("likelihood must be 'tg2' or 'gauss'")
+        self.likelihood, self.burn_in = likelihood, int(burn_in)
         # A chain whose slice does not close within ``max_trips`` proposals keeps its state and is reported with
         # status 1 (the reference's ``while True`` would loop on, or raise LinAlgError out of jitchol when the
         # factorisation at the current state is the reason).  ``strict`` turns that into an exception; otherwise the
@@ -53,7 +61,7 @@ class ChainEnsemble(object):
                 self.dist, self.rank, self.world = dist, dist.get_rank(), dist.get_world_size()
         except ImportError:
             pass
-        F0 = np.asarray(F0, dtype=np.float64)
+        F0 = None if F0 is None and likelihood == 'gauss' else np.asarray(F0, dtype=np.float64)
         Hyp0 = np.asarray(Hyp0, dtype=np.float64)
         if sharded_input:
             self.n_local = Hyp0.shape[0]
@@ -68,10 +76,10 @@ class ChainEnsemble(object):
             self.n_local = self.hi - self.lo
             self._counts = [shard_bounds(self.n_chains, self.world, r)[1] - shard_bounds(self.n_chains, self.world, r)[0]
                             for r in range(self.world)]
-            F0, Hyp0 = F0[self.lo:self.hi], Hyp0[self.lo:self.hi]
+            F0, Hyp0 = (None if F0 is None else F0[self.lo:self.hi]), Hyp0[self.lo:self.hi]
         self.P = Hyp0.shape[1]
         # the sweeper is the device path; tests of the host logic inject their own (gloo, no GPU)
-        self._sweeper = sweeper or _DeviceSweeper(self)
+        self._sweeper = sweeper or (_MarginalSweeper(self) if likelihood == 'gauss' else _DeviceSweeper(self))
         self._sweeper.load(F0, Hyp0)
 
     def _all_counts(self, n_local):
@@ -262,3 +270,34 @@ class _DeviceSweeper(object):
 
     def state(self):
         return self.F.cpu().numpy(), self.H.cpu().numpy()
+
+
+class _MarginalSweeper(_DeviceSweeper):
+    """``likelihood='gauss'``: holds the shard's hyper-parameters in HBM and advances them with ``gpmc_marginal_run``."""
+
+    def load(self, F0, Hyp0):
+        super().load(np.zeros((Hyp0.shape[0], 0)) if F0 is None else F0, Hyp0)
+
+    def _call(self, it0, n_iters):
+        e = self.ens
+        torch = self.torch
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        out = ops.marginal_run(self.x, self.y, self.H, self.scale, it0, n_iters, m=e.my, burn_in=e.burn_in, seed=e.seed,
+                               chain0=e.lo, max_trips=e.max_trips, kind=e.kind)
+        e1.record()
+        e1.synchronize()
+        self.last_busy_ms = e0.elapsed_time(e1)
+        return out
+
+    def sweep(self, it):
+        hh, ll, nt, exh = self._call(it, 1)
+        return self.H, ll[:, 0], nt[:, 0], (exh != 0).to(self.torch.int32)
+
+    def run(self, it0, n_iters, thin_f=0, thin_phase=0):
+        if thin_f:
+            raise ValueError("likelihood='gauss' has no latent f to keep")
+        hh, ll, nt, exh = self._call(it0, n_iters)
+        # transitions that kept their state: budget used up, or every transition of a chain that cannot start
+        n_exh = int(exh.clamp(min=0).sum().item()) + n_iters * int((exh < 0).sum().item())
+        return hh, ll, nt, None, n_exh

@@ -273,6 +273,8 @@ size_t gpmc_workspace_bytes(int op, int N, int D, int B)
         return l.fixed_bytes + wave * l.per_item_bytes;
     }
     if (op == GPMC_OP_LOGLIK_GRAD) return loglik_grad_workspace_bytes(N, D, B);
+    // the sampler's arrays (sized for P = D + 2, the widest row) and the log-likelihood unit's recommended workspace
+    if (op == GPMC_OP_MARGINAL) return marginal_state_bytes(N, D + 2, B) + gpmc_workspace_bytes(GPMC_OP_LOGLIK, N, D, B);
     return 0;
 }
 
@@ -361,12 +363,12 @@ int gpmc_potrf_batched(double *A_dev, int N, int ld, int B, int *info_dev, int j
     return 0;
 }
 
-int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, const double *hyp_dev, int B, int P,
-                        int kind, int jitter_policy, double *loglik_dev, int *info_dev, void *ws_dev, size_t ws_bytes,
-                        void *stream)
+}  // extern "C"
+
+namespace gpmc {
+int loglik_batched(const double *x_dev, int N, int D, const double *g_dev, int ldg, const double *hyp_dev, int B, int P, int kind,
+                   int jitter_policy, double *loglik_dev, int *info_dev, void *ws_dev, size_t ws_bytes, cudaStream_t s)
 {
-    GPMC_API_LOCK();
-    cudaStream_t s = (cudaStream_t)stream;
     const int n_ell = kind_n_ell(kind, D);
     if (N <= 0 || D <= 0 || B < 0 || P != n_ell + 2 || kind_cf(kind) < 0) { set_error("loglik: bad shape N=%d D=%d B=%d P=%d kind=%d", N, D, B, P, kind); return GPMC_EINVAL; }
     if (B == 0) return 0;
@@ -423,12 +425,12 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
                     const Envelope env{env_all + (size_t)s0 * nblk, nblk, N, bh[0]};
                     const Band band{w_all + (size_t)s0 * nblk, nblk, bh[1], 0};
                     const double *hyp_w = hyp_dev + (size_t)s0 * P;
-                    const double *g_w = g_dev + (size_t)s0 * N;
+                    const double *g_w = g_dev + (size_t)s0 * ldg;
                     int *info_w = info_dev + s0;
                     auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
                         int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, kind, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
                         if (rc) return rc;
-                        return border_set(V, N, g_w, N, nitems, s);
+                        return border_set(V, N, g_w, ldg, nitems, s);
                     };
                     auto diag = [&](const double *h) { return host_diag_value(h, n_ell); };
                     rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, Wsc, jit_dev, map_dev, jitter_policy, 1, s, potrf_fuse_compact(), env);
@@ -450,7 +452,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
     for (int s0 = 0; s0 < B; s0 += wave) {
         const int nb = std::min(wave, B - s0);
         const double *hyp_w = hyp_dev + (size_t)s0 * P;
-        const double *g_w = g_dev + (size_t)s0 * N;
+        const double *g_w = g_dev + (size_t)s0 * ldg;
         int *info_w = info_dev + s0;
         BatchView A{mats, (long long)l.mat_elems, l.ld, nullptr, nullptr};
         const int fuse = potrf_fuse_auto(N, nb, 1);
@@ -495,7 +497,7 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
         auto fill = [&](BatchView V, int nitems, const double *jit) -> int {
             int rc = launch_cov_assemble(x_dev, N, D, hyp_w, P, kind, GPMC_ASM_ADD_S | GPMC_ASM_LOWER_ONLY, jit, V, nitems, s, env, band);
             if (rc) return rc;
-            return border_set(V, N, g_w, N, nitems, s);
+            return border_set(V, N, g_w, ldg, nitems, s);
         };
         auto diag = [&](const double *h) { return host_diag_value(h, n_ell); };
         rc = factor_wave(fill, diag, A, N, nb, hyp_w, P, info_w, W, jit_dev, map_dev, jitter_policy, 1, s, fuse, env);
@@ -505,6 +507,19 @@ int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, 
         if (rc) return rc;
     }
     return 0;
+}
+
+}  // namespace gpmc
+
+extern "C" {
+
+int gpmc_loglik_batched(const double *x_dev, int N, int D, const double *g_dev, const double *hyp_dev, int B, int P,
+                        int kind, int jitter_policy, double *loglik_dev, int *info_dev, void *ws_dev, size_t ws_bytes,
+                        void *stream)
+{
+    GPMC_API_LOCK();
+    return loglik_batched(x_dev, N, D, g_dev, N, hyp_dev, B, P, kind, jitter_policy, loglik_dev, info_dev, ws_dev, ws_bytes,
+                          (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------------------ host-buffer path

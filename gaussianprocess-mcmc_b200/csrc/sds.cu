@@ -11,40 +11,11 @@
 // keyed by (seed, global chain id), so results do not depend on how chains are sharded over GPUs.
 #include "common.cuh"
 #include "sds.cuh"
+#include "slice_common.cuh"
 #include "tg2.cuh"
 #include "../../include/gpmc.h"
 
 namespace gpmc {
-
-// ------------------------------------------------------------------------------------- Philox4x32-10
-__device__ __forceinline__ void philox_round(unsigned &c0, unsigned &c1, unsigned &c2, unsigned &c3, unsigned k0, unsigned k1)
-{
-    const unsigned long long p0 = 0xD2511F53ull * c0, p1 = 0xCD9E8D57ull * c2;
-    const unsigned h0 = (unsigned)(p0 >> 32), l0 = (unsigned)p0, h1 = (unsigned)(p1 >> 32), l1 = (unsigned)p1;
-    c0 = h1 ^ c1 ^ k0; c1 = l1; c2 = h0 ^ c3 ^ k1; c3 = l0;
-}
-__device__ void philox4x32(unsigned long long seed, unsigned c0, unsigned c1, unsigned c2, unsigned c3, unsigned out[4])
-{
-    unsigned k0 = (unsigned)seed, k1 = (unsigned)(seed >> 32);
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        philox_round(c0, c1, c2, c3, k0, k1);
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
-}
-// two uniforms on (0,1) with 53 random bits each, from one Philox block
-__device__ __forceinline__ void philox_uniform2(unsigned long long seed, unsigned chain, unsigned sweep, unsigned stream,
-                                                unsigned idx, double &u0, double &u1)
-{
-    unsigned o[4];
-    philox4x32(seed, chain, sweep, stream, idx, o);
-    const unsigned long long a = ((unsigned long long)o[0] << 32 | o[1]) >> 11;
-    const unsigned long long b = ((unsigned long long)o[2] << 32 | o[3]) >> 11;
-    u0 = ((double)a + 0.5) * (1.0 / 9007199254740992.0);
-    u1 = ((double)b + 0.5) * (1.0 / 9007199254740992.0);
-}
-enum { STREAM_Z = 0, STREAM_BRACKET = 1, STREAM_TRIP = 2 };
 
 // --------------------------------------------------------------------------------- scalar formulas
 // S_ii of aux_var_model (sliceSample.py:184-190) for the SE kernel, whose diagonal is sf2 everywhere.
@@ -55,24 +26,6 @@ __device__ __forceinline__ double s_diag_value(double sf, double sn)
     const double v_1 = 1.0 / (sn * sn) + K_ii_inv;
     double Sii = 1.0 / (v_1 - K_ii_inv);
     return (Sii < 0.0) ? 0.0 : Sii;
-}
-
-// log_gamma (sliceSample.py:209-232): Gamma log-pdf for every entry, inverse-Gamma for the last (noise).
-__device__ double log_prior_entry(double x, double k, double theta, bool inverse_gamma)
-{
-    if (!inverse_gamma) return (k - 1.0) * log(x) - x / theta - k * log(theta) - log(tgamma(k));       // :224
-    return log(pow(theta, k)) - log(tgamma(k)) + (-k - 1.0) * log(x) + (-theta / x);                   // :229
-}
-
-// head + prior[sf] + prior[ell_0..] + G (+ prior[sn] after burn-in): the summation order of :127-129,150-152
-__device__ double density_sum(double head, const double *hyp, const double *pk, const double *pth, int P, double G, int iter)
-{
-    const int n_ell = P - 2;
-    double acc = head + log_prior_entry(hyp[n_ell], pk[n_ell], pth[n_ell], false);
-    for (int d = 0; d < n_ell; ++d) acc = acc + log_prior_entry(hyp[d], pk[d], pth[d], false);
-    acc = acc + G;
-    if (iter >= 500) acc += log_prior_entry(hyp[P - 1], pk[P - 1], pth[P - 1], true);
-    return acc;
 }
 
 // ------------------------------------------------------------------------------------------ kernels
@@ -155,7 +108,7 @@ __global__ void __launch_bounds__(256) sds_threshold_kernel(SdsState st)
     if (threadIdx.x == 0) {
         st.cur_llk[c] = llk;
         const int it = st.iter_of ? st.iter_of[c] : st.iter;
-        st.threshold[c] = density_sum(st.log_u0[c] + llk, hyp, st.prior_k, st.prior_theta, P, st.G[c], it);            // :127-129
+        st.threshold[c] = density_sum(st.log_u0[c] + llk, hyp, st.prior_k, st.prior_theta, P, st.G[c], it, 500);            // :127-129
         st.curG[c] = st.G[c];
         if (st.chain_of) {
             st.phase[c] = SDS_PHASE_ACTIVE;
@@ -219,7 +172,7 @@ __global__ void __launch_bounds__(256) sds_accept_kernel(SdsState st)
     const int it = st.iter_of ? st.iter_of[c] : st.iter;          // (read before the block barriers inside tg2_loglik_block:
     const double llk = tg2_loglik_block(st.y, st.my, fp, st.n, th[P - 1], st.lower, st.upper, red);   // thread 0 advances it below)  :142-143
     if (threadIdx.x == 0) {
-        const double proposal = density_sum(llk, th, st.prior_k, st.prior_theta, P, st.G[c], it);                     // :149-152
+        const double proposal = density_sum(llk, th, st.prior_k, st.prior_theta, P, st.G[c], it, 500);                     // :149-152
         const bool ok = (proposal > st.threshold[c]) && isfinite(proposal);                                         // :154
         st.ntrips[c] += 1;
         st.last_proposal[c] = proposal;

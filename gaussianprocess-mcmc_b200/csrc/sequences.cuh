@@ -62,6 +62,11 @@ int r_sequence(BatchView Rm, BatchView U, int n, int B, const double *svec, long
 
 // gpmc_workspace_bytes(GPMC_OP_LOGLIK_GRAD, ...) (loglik_grad.cu)
 size_t loglik_grad_workspace_bytes(int N, int D, int B);
+// the sampler's own arrays inside a gpmc_marginal_run workspace (marginal.cu); the log-likelihood unit gets the rest
+size_t marginal_state_bytes(int N, int P, int B);
+// gpmc_loglik_batched with the right-hand side of item b at g_dev + b * ldg (ldg = 0: one row shared by every item) (capi.cu)
+int loglik_batched(const double *x_dev, int N, int D, const double *g_dev, int ldg, const double *hyp_dev, int B, int P, int kind,
+                   int jitter_policy, double *loglik_dev, int *info_dev, void *ws_dev, size_t ws_bytes, cudaStream_t s);
 
 // small helpers
 int fill_int(int *p, int v, int n, cudaStream_t s);

@@ -51,6 +51,7 @@ class GPR(object):
         self.likRange = None
         self.method = 'BFGS'
         self.optim_result = None
+        self.hyp_samples = None
 
     # ------------------------------------------------------------------ model set-up (pyGPs names)
     def setData(self, x, y):
@@ -131,21 +132,51 @@ class GPR(object):
         self._set_log_hyp(best.x)
         return self.getPosterior()
 
+    # ------------------------------------------------------------------ fully Bayesian hyper-parameters
+    def sampleHyp(self, n_iters, n_chains=8, scale=None, burn=0, thin=1, seed=0, max_trips=64):
+        """Posterior samples of the hyper-parameters instead of one type-II ML point: ``n_chains`` slice-sampling chains
+        (``ops.marginal_run``: the latent f integrated out, the hyper-priors of ``sliceSample.py:124-125``, every prior
+        from the first iteration) start at the current hyper-parameters and run ``n_iters`` transitions each.  The
+        samples after the first ``burn`` of every chain, every ``thin``-th, are kept as natural-scale rows
+        ``(ell.., sf, sn)`` in ``hyp_samples`` and returned.  ``scale``: the slice widths (default: the current theta)."""
+        theta = np.exp(self._log_hyp())
+        scale = theta if scale is None else np.asarray(scale, dtype=np.float64)
+        import torch
+        H = torch.tensor(np.tile(theta, (int(n_chains), 1))).cuda()
+        hh, _, _, _ = ops.marginal_run(self.x, self.y.reshape(-1), H, scale, 0, int(n_iters), m=0.0, burn_in=0, seed=seed,
+                                       max_trips=max_trips, **self._kind_kw())
+        self.hyp_samples = _np(hh)[:, int(burn)::int(thin), :].reshape(-1, theta.shape[0]).copy()
+        return self.hyp_samples
+
     # ------------------------------------------------------------------ prediction
-    def predict(self, xs, ys=None):
+    def predict(self, xs, ys=None, samples=None):
         """``(ym, ys2, fm, fs2, lp)`` as columns ``[M, 1]``: latent mean / variance (clamped at 0, as pyGPs does),
-        ``ym = fm``, ``ys2 = fs2 + sn^2``, ``lp = log N(ys; ym, ys2)`` (``ys`` zero when omitted, as pyGPs evaluates it)."""
+        ``ym = fm``, ``ys2 = fs2 + sn^2``, ``lp = log N(ys; ym, ys2)`` (``ys`` zero when omitted, as pyGPs evaluates it).
+
+        ``samples[S, P]`` (natural-scale rows, e.g. ``hyp_samples``): the predictive of the mixture over them, from ONE
+        ``ops.predict_batched`` call -- ``fm`` the mean of the per-sample means, ``fs2`` the mean of ``fs2 + fmu^2`` minus
+        ``fm^2``, ``ys2 = fs2 +`` the mean of ``sn^2``."""
         xs = np.asarray(xs, dtype=np.float64)
         self.xs = xs.reshape(-1, 1) if xs.ndim == 1 else xs
         M = self.xs.shape[0]
-        theta = np.exp(self._log_hyp())
+        theta = np.exp(self._log_hyp())[None] if samples is None else np.atleast_2d(np.asarray(samples, dtype=np.float64))
+        S = theta.shape[0]
         m = self.meanfunc.getMean(self.x)
-        fmu, fs2, info = ops.predict_batched(self.x, self.xs, (self.y - m).reshape(1, -1), theta[None], **self._kind_kw())
-        if int(_np(info)[0]) != 0:
+        fm_rows = np.tile((self.y - m).reshape(1, -1), (S, 1))
+        fmu, fs2, info = ops.predict_batched(self.x, self.xs, fm_rows, theta, **self._kind_kw())
+        if np.any(_np(info) != 0):
             raise np.linalg.LinAlgError('not positive definite, even with jitter.')
-        fm = self.meanfunc.getMean(self.xs) + _np(fmu).reshape(M, 1)
-        fs2 = np.maximum(_np(fs2).reshape(M, 1), 0)
-        ym, ys2 = fm, fs2 + self.likfunc.sn ** 2
+        fmu = _np(fmu).reshape(S, M)
+        fs2 = np.maximum(_np(fs2).reshape(S, M), 0)
+        if samples is None:
+            fm = self.meanfunc.getMean(self.xs) + fmu.reshape(M, 1)
+            fs2 = fs2.reshape(M, 1)
+            ym, ys2 = fm, fs2 + self.likfunc.sn ** 2
+        else:
+            mu = fmu.mean(axis=0)
+            fm = self.meanfunc.getMean(self.xs) + mu.reshape(M, 1)
+            fs2 = ((fs2 + fmu ** 2).mean(axis=0) - mu ** 2).reshape(M, 1)
+            ym, ys2 = fm, fs2 + np.mean(theta[:, -1] ** 2)
         yy = np.zeros((M, 1)) if ys is None else np.asarray(ys, dtype=np.float64).reshape(M, 1)
         lp = -(yy - ym) ** 2 / (2 * ys2) - 0.5 * np.log(2 * np.pi * ys2)
         if ys is not None:

@@ -7,7 +7,7 @@ import numpy as np
 from . import _lib
 from ._lib import (KIND_SE_ISO, KIND_SE_ARD, KIND_MATERN1, KIND_MATERN3, KIND_MATERN5, ASM_ADD_S, ASM_LOWER_ONLY,
                    JITTER_NONE, JITTER_PYGPS,
-                   OP_POTRF, OP_LOGLIK, OP_LOGLIK_GRAD, GpmcError)
+                   OP_POTRF, OP_LOGLIK, OP_LOGLIK_GRAD, OP_MARGINAL, GpmcError)
 
 
 def _stream_ptr(torch):
@@ -355,6 +355,94 @@ def sds_run(x, y, F, Hyp, scale, it0, n_iters, my=None, seed=0, chain0=0, max_tr
                           n_exh.data_ptr(), ws.data_ptr(), ws_bytes, _stream_ptr(torch))
     _lib.check(rc, 'gpmc_sds_run')
     return hist_hyp, hist_ll, hist_trips, hist_f, int(n_exh.item())
+
+
+class MarginalTape(object):
+    """Explicit randomness of ``n_iters`` marginal slice-sampling transitions for B chains (``sliceSample.py:110,127,132``):
+    ``v[B, n_iters, P]``, ``u0[B, n_iters]``, ``U[B, n_iters, T, P]``, all U(0,1)."""
+
+    def __init__(self, v, u0, U):
+        self.v = np.ascontiguousarray(v, dtype=np.float64)
+        self.u0 = np.ascontiguousarray(u0, dtype=np.float64)
+        self.U = np.ascontiguousarray(U, dtype=np.float64)
+
+
+def marginal_run(x, y, Hyp, scale, it0, n_iters, m=None, burn_in=500, seed=0, chain0=0, max_trips=64, prior_k=None,
+                 prior_theta=None, tape=None, kind=None, jitter_policy=JITTER_PYGPS, workspace=None):
+    """``n_iters`` slice-sampling transitions of the hyper-parameters of every chain under a Gaussian likelihood, the latent
+    f integrated out (``gpmc_marginal_run``): the target is ``N(y - m; 0, K + S) * priors``, one banded log-likelihood
+    evaluation per proposal.  ``m=None`` is ``mean(y)`` (``sliceSample.py:102``).
+
+    ``Hyp[B,P]`` (CUDA float64) holds the state on entry and the final state on return.  Returns device tensors
+    ``(hist_hyp[B, n_iters, P], hist_loglik[B, n_iters], hist_trips[B, n_iters], exhausted[B])``; ``exhausted[b]`` counts
+    the transitions that used up ``max_trips`` (-1: the chain's starting log-likelihood is not finite, state kept)."""
+    torch = _lib.require_cuda()
+    lib = _lib.load()
+    x = _f64_cuda(torch, x, 'x')
+    if x.dim() == 1:
+        x = x.reshape(-1, 1)
+    N, D = x.shape
+    if not (Hyp.is_cuda and Hyp.dtype == torch.float64 and Hyp.is_contiguous() and Hyp.dim() == 2):
+        raise ValueError('Hyp must be a contiguous CUDA float64 tensor [B, P]')
+    B, P = Hyp.shape
+    kind = _kind(D, P, kind)
+    if m is None:
+        m = float(np.mean(np.asarray(y.cpu() if hasattr(y, 'cpu') else y, dtype=np.float64)))
+    y = _f64_cuda(torch, y, 'y').reshape(-1)
+    if y.numel() != N:
+        raise ValueError('y must have N=%d entries' % N)
+    k, th = prior_constants(P - 2)
+    k = _f64_cuda(torch, k if prior_k is None else prior_k, 'prior_k').reshape(-1)
+    th = _f64_cuda(torch, th if prior_theta is None else prior_theta, 'prior_theta').reshape(-1)
+    scale = _f64_cuda(torch, scale, 'scale').reshape(-1)
+    if scale.numel() != P or k.numel() != P or th.numel() != P:
+        raise ValueError('scale and the prior constants must have P=%d entries' % P)
+    n_iters = int(n_iters)
+    hist_hyp = torch.zeros((B, max(n_iters, 0), P), dtype=torch.float64, device='cuda')
+    hist_ll = torch.zeros((B, max(n_iters, 0)), dtype=torch.float64, device='cuda')
+    hist_trips = torch.zeros((B, max(n_iters, 0)), dtype=torch.int32, device='cuda')
+    exhausted = torch.zeros((B,), dtype=torch.int32, device='cuda')
+    tv = tu = tU = None
+    ttrips = 0
+    if tape is not None:
+        if tape.v.shape != (B, n_iters, P) or tape.u0.shape != (B, n_iters) or tape.U.ndim != 4 or \
+                tape.U.shape[:2] != (B, n_iters) or tape.U.shape[3] != P:
+            raise ValueError('tape shapes do not match B=%d n_iters=%d P=%d' % (B, n_iters, P))
+        tv, tu, tU = (torch.tensor(a).cuda() for a in (tape.v, tape.u0, tape.U))
+        ttrips = tape.U.shape[2]
+    ws_bytes = 0
+    ws = None
+    if B > 0 and n_iters > 0:
+        wsobj = workspace or _default_ws
+        need = lib.gpmc_workspace_bytes(OP_MARGINAL, N, D, B)
+        have = 0 if wsobj.buf is None else wsobj.buf.numel()
+        if have < need:
+            # growing: never ask for more than 60 % of what is free (as loglik_batched)
+            free, _ = torch.cuda.mem_get_info()
+            one = lib.gpmc_workspace_bytes(OP_MARGINAL, N, D, B) - lib.gpmc_workspace_bytes(OP_LOGLIK, N, D, B) + \
+                lib.gpmc_workspace_bytes(OP_LOGLIK, N, D, 1)
+            need = max(one, min(need, (free + have) * 6 // 10))
+        ws = wsobj.get(torch, need)
+        ws_bytes = ws.numel()
+    ptr = lambda t: None if t is None else t.data_ptr()
+    rc = lib.gpmc_marginal_run(x.data_ptr(), N, D, y.data_ptr(), float(m), Hyp.data_ptr(), B, P, kind,
+                               scale.data_ptr(), k.data_ptr(), th.data_ptr(), int(it0), n_iters, int(burn_in), int(seed),
+                               int(chain0), ptr(tv), ptr(tu), ptr(tU), ttrips, int(max_trips), jitter_policy,
+                               hist_hyp.data_ptr(), hist_ll.data_ptr(), hist_trips.data_ptr(), exhausted.data_ptr(),
+                               ptr(ws), ws_bytes, _stream_ptr(torch))
+    _lib.check(rc, 'gpmc_marginal_run')
+    return hist_hyp, hist_ll, hist_trips, exhausted
+
+
+def marginal_rounds():
+    """``(active[R], ms[R])`` of the rounds of the last ``marginal_run``: chains evaluated per round and host wall time."""
+    lib = _lib.load()
+    n = lib.gpmc_marginal_rounds(0, None, None)
+    act = np.zeros(n, dtype=np.int32)
+    ms = np.zeros(n, dtype=np.float64)
+    if n:
+        lib.gpmc_marginal_rounds(n, act.ctypes.data, ms.ctypes.data)
+    return act, ms
 
 
 def _pad_matrix(torch, A, ld):

@@ -83,6 +83,7 @@ extern "C" {
 #define GPMC_OP_LOGLIK  2
 #define GPMC_OP_SDS     3
 #define GPMC_OP_LOGLIK_GRAD 4
+#define GPMC_OP_MARGINAL 5
 
 int gpmc_version(void);
 /* panel width (block-column width) of the blocked Cholesky this build was compiled with: 64 or 128 */
@@ -208,6 +209,55 @@ int gpmc_sds_run(const double *x_dev, const double *y_dev, int N, int D, double 
                  int thin, int n_keep, int *n_exhausted_dev, void *ws_dev, size_t ws_bytes, void *stream);
 
 /*
+ * Slice sampling of the hyper-parameters of GP regression with a Gaussian likelihood, the latent f integrated out: B
+ * independent chains with target  p(theta | y) ~ N(y - m; 0, K_theta + S_theta) * prod_p prior_p(theta_p),  i.e. the
+ * log-likelihood unit of gpmc_loglik_batched (y - m as every item's right-hand side) plus the hyper-priors of
+ * gpmc_sds_sweep (log_gamma, sliceSample.py:209-232).  Each transition is the reference's hyper-rectangle slice sampler
+ * (sliceSample.py:110-163) without f, g and the truncated-Gaussian term:
+ *   bracket (:110-112)   v ~ U(0, scale)^P, hyp_min = max(hyp - v, 0), hyp_max = hyp_min + scale
+ *   threshold (:127-129) log u0 + prior[sf] + prior[ell..] + G_cur (+ prior[sn] once iter >= burn_in); G_cur is the
+ *                        log-likelihood at the chain's current theta, carried from the accepted proposal (evaluated once per
+ *                        call, for every chain, in the first round)
+ *   shrink loop (:131-163) theta' = hyp_min + (hyp_max - hyp_min) U; while iter < burn_in theta'_sn = hyp_sn and the sn prior
+ *                        is left out of both sides (the reference's rule with burn_in = 500; 0 turns it off); G' =
+ *                        loglik(theta'); accept if 0 + priors + G' > threshold and finite, else shrink every dimension
+ *                        toward hyp.  A factorisation that fails even with the jitter ladder gives G' = NaN: rejected.
+ *   x_dev[N,D], y_dev[N], m    data and the constant mean (the reference's mean(y), :102)
+ *   hyp_dev[B,P]               state on entry, final state on return (natural scale, as every other entry point)
+ *   scale_dev[P], prior_k_dev[P], prior_theta_dev[P]   as gpmc_sds_sweep
+ *   iter_begin, n_iters        every chain runs its transitions iter_begin .. iter_begin + n_iters - 1 back to back
+ *   randomness                 Philox4x32-10 keyed by (seed, chain0 + chain, iteration) on the streams of gpmc_sds_run (a
+ *                              chain draws the v, u0 and U gpmc_sds_run would), or, with all three tapes given,
+ *                              tape_v[B, n_iters, P], tape_u0[B, n_iters], tape_U[B, n_iters, tape_trips, P] (U(0,1));
+ *                              the trip budget is then min(max_trips, tape_trips)
+ *   max_trips                  a transition that uses it up keeps the chain's state and is counted in exhausted_dev[b]
+ *   history (any may be NULL)  hist_hyp_dev[B, n_iters, P], hist_loglik_dev[B, n_iters] (G of the sample),
+ *                              hist_trips_dev[B, n_iters]; exhausted_dev[B] (may be NULL): transitions that used up the
+ *                              budget, or -1 for a chain whose log-likelihood at its starting state is not finite (it keeps
+ *                              that state for the whole call, its history repeats it with 0 trips, and it costs nothing)
+ * Every chain stays in flight: a round proposes for every chain still inside a transition, evaluates those proposals in
+ * one gpmc_loglik_batched-style call (waves, compact band layout and jitter ladder unchanged), accepts or shrinks, and
+ * starts the next transition of every chain that finished one.  The host reads the active count once per round, so launch
+ * sizes, and the results, repeat bit for bit.  Returns when every chain has finished; gpmc_loglik_layout then reports the
+ * layout of the last round.  Workspace: gpmc_workspace_bytes(GPMC_OP_MARGINAL, N, D, B) (the sampler's O(B P) arrays plus
+ * the log-likelihood unit's; a smaller one runs the rounds in more waves).  GPMC_EINVAL for an unknown kind, a P that does
+ * not fit it, n_iters < 0, iter_begin < 0, burn_in < 0, max_trips <= 0, an unknown jitter policy, a tape that is not all
+ * three arrays with tape_trips >= 1 (or none with tape_trips = 0), and missing inputs; B = 0 or n_iters = 0 return 0.
+ */
+int gpmc_marginal_run(const double *x_dev, int N, int D, const double *y_dev, double m,
+                      double *hyp_dev, int B, int P, int kind,
+                      const double *scale_dev, const double *prior_k_dev, const double *prior_theta_dev,
+                      int iter_begin, int n_iters, int burn_in, unsigned long long seed, unsigned chain0,
+                      const double *tape_v, const double *tape_u0, const double *tape_U, int tape_trips,
+                      int max_trips, int jitter_policy,
+                      double *hist_hyp_dev, double *hist_loglik_dev, int *hist_trips_dev, int *exhausted_dev,
+                      void *ws_dev, size_t ws_bytes, void *stream);
+/* Rounds of the last gpmc_marginal_run on this process: returns their number; the first `capacity` of them give the
+ * chains evaluated in the round (active_out) and its host wall time in ms, which ends in a synchronisation (ms_out).
+ * Either pointer may be NULL. */
+int gpmc_marginal_rounds(int capacity, int *active_out, double *ms_out);
+
+/*
  * aux_var_model(f, K, sn, g) for one caller-supplied K (sliceSample.py:165-207).  K_dev[N][ld] (ld % 16 == 0, pad
  * columns zero), S_dev[ld] = diag of S (sliceSample.py:184-190; entries beyond N zero), g_dev[ld].  Outputs
  * L_dev = chol(K+S) (:196), m_dev[ld] = R S^-1 g (:204), C_dev = chol(R + 1e-11 I) (:205), both N x ld lower with
@@ -323,7 +373,8 @@ int gpmc_ess_sweep(const double *x_dev, const double *y_dev, int N, int D, doubl
 int gpmc_set_tuning(int key, int value);
 
 /* Layout the last gpmc_loglik_batched / gpmc_loglik_host call used: *band_W = 0 for the dense layout, else the row width
- * of the compact band layout (key 17); *waves = the number of waves the call's items were factored in. */
+ * of the compact band layout (key 17); *waves = the number of waves the call's items were factored in.  After
+ * gpmc_marginal_run: the layout of its last round. */
 int gpmc_loglik_layout(int *band_W, int *waves);
 
 /* FP64 micro-benchmarks used by bench.py to put a measured peak beside the roofline:
